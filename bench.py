@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Throughput of the token-sparsification hot path inside DynamicViT DeiT-S/16, keep rate 0.7, 224 px.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl d2s|reference] [--batch B] [--legs a,b,...]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl d2s|reference] [--batch B] [--legs a,b,...] [--dump-outputs DIR]
 
 A "step" is one inference pass of the pruned model over one batch of synthetic images (BASELINE.json configs[1]: batch 1024
 per GPU, bf16).  N > 1 = one process per GPU (torchrun); the batch dimension is sharded with no data-path collective (weak
@@ -24,6 +24,11 @@ scaling: every rank owns its own 1024 images).  Rank 0 prints ONE JSON line.
   gpu_eager_baseline  the oracle's restatement of the reference forward executed by torch eager on the same GPU in bf16
   cpu_baseline   the CPU restatement of the reference forward (oracle/), timed on this box's host cores
   --impl reference   times that CPU forward alone (the reference is pure PyTorch; see DESIGN.md section 7)
+
+--steps K is the number of timed steps of every leg that times the project's own path (value, e2e, train, arch_base, variant_b).
+--dump-outputs DIR writes what the timed path computed in its last step (rank 0): the logits and the kept-token indices of every
+stage, as DIR/<name>.npy in float32.  Weights and inputs are seeded, so two builds run with the same arguments can be compared
+output for output.  bench.py writes nothing into the repository tree (it may be read-only).
 """
 import argparse
 import json
@@ -33,6 +38,7 @@ import subprocess
 import sys
 import time
 
+sys.dont_write_bytecode = True   # no __pycache__ in the repository tree for the modules only bench.py imports
 ROOT = os.path.dirname(os.path.abspath(__file__))
 for _p in (ROOT, os.path.join(ROOT, "tests", "golden")):
     if _p not in sys.path:
@@ -48,6 +54,7 @@ TRAIN_GFLOP_PER_IMG = 36.8                              # SURVEY.md 8d: 3 x 9.2 
 ALL_LEGS = ("parity", "infer", "e2e", "h2d", "train", "kernels", "ptopk", "sweep", "base", "variant_b", "eager", "cpu")
 W_SEED = 61                                             # seeded weights (tests/golden/fixtures.py): well-spread predictor scores
 L2_BYTES = 126e6
+DUMP_BYTES = 64 << 20                                   # --dump-outputs: at most this much in all
 
 
 def parse():
@@ -58,14 +65,23 @@ def parse():
     ap.add_argument("--impl", default="d2s", choices=["d2s", "reference"])
     ap.add_argument("--batch", type=int, default=1024, help="images per GPU per step")
     ap.add_argument("--train-batch", type=int, default=256, help="images per GPU per training step (BASELINE configs[2])")
-    ap.add_argument("--train-steps", type=int, default=10)
+    ap.add_argument("--train-steps", type=int, default=None, help="timed training steps (default: --steps)")
     ap.add_argument("--cpu-batch", type=int, default=8, help="images per CPU step (BASELINE configs[0])")
     ap.add_argument("--no-graph", action="store_true")
     ap.add_argument("--teacher-stream", type=int, default=1, help="training leg: run the frozen teacher on a second stream (1) or inline (0)")
     ap.add_argument("--torch-adamw", action="store_true", help="training leg: torch.optim.AdamW(capturable) instead of runner.FlatAdamW")
     ap.add_argument("--skip-cpu", action="store_true", help="omit the cpu_baseline leg (debugging only)")
     ap.add_argument("--legs", default=",".join(ALL_LEGS), help="comma-separated subset of: " + ", ".join(ALL_LEGS))
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the timed path's outputs of its last step (rank 0) as DIR/<name>.npy, float32")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "d2s":
+        ap.error("--dump-outputs writes the outputs of the d2s arm")
+    if args.train_steps is None:
+        args.train_steps = args.steps
+    return args
 
 
 def peaks():
@@ -220,6 +236,21 @@ def time_graphed(calls, torch, launches=24, replays=5):
 def nsets_for(bytes_per_call):
     """How many rotating argument sets make the working set larger than twice the L2 (at most 8, at least 1)."""
     return int(max(1, min(8, -(-2 * L2_BYTES // max(1.0, float(bytes_per_call))))))
+
+
+def dump_outputs(out_dir, arrays):
+    """Write each batch-major array as out_dir/<name>.npy in float32 (the indices are small integers: exact).  Above DUMP_BYTES
+    in all, the same fixed, seeded sample of rows (images) is taken from every array."""
+    import numpy as np
+    arrays = {k: v.detach().float().cpu().numpy() for k, v in arrays.items()}
+    rows = next(iter(arrays.values())).shape[0]
+    row_bytes = sum(a[0].nbytes for a in arrays.values())
+    if rows * row_bytes > DUMP_BYTES:
+        keep = np.sort(np.random.RandomState(0).choice(rows, DUMP_BYTES // row_bytes, replace=False))
+        arrays = {k: a[keep] for k, a in arrays.items()}
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(out_dir, k + ".npy"), a)
 
 
 def row(kernel, shape, ms, algo_bytes, launches_per_step=None, flops=None):
@@ -577,7 +608,7 @@ def train_leg(pkg, args, dev, rank, world, torch, dist, pk):
     return out
 
 
-def base_leg(pkg, dev, torch, pk, no_graph=False):
+def base_leg(pkg, dev, torch, pk, K, no_graph=False):
     """DeiT-B widths (D = 768, 12 heads, hidden 3072; dynamic_vit.py:1301-1303) through the same inference path: attention on
     the tcgen05 kernel, proj / fc2 + residual + LayerNorm as the CTA-pair GEMM with the row kept in two 384-column halves,
     fc1 + GELU as the CTA-pair GEMM; qkv stays the library GEMM and the hidden activations make an HBM round trip (the
@@ -597,7 +628,6 @@ def base_leg(pkg, dev, torch, pk, no_graph=False):
         runner.replay()
     torch.cuda.synchronize()
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-    K = 10
     e0.record()
     for _ in range(K):
         runner.replay()
@@ -617,7 +647,7 @@ def base_leg(pkg, dev, torch, pk, no_graph=False):
     return res
 
 
-def variant_b_leg(pkg, dev, torch, no_graph=False):
+def variant_b_leg(pkg, dev, torch, K, no_graph=False):
     """Dense2Sparse (Variant B, dynamic_vit.py:814-1015): one pruning stage at block 3, keep ratio 0.7, top-k selection, the
     large LayerNorm predictor, CLS-attention rows collected in every block.  Inference at batch 1024 (CUDA graph) and the
     reference's training loop (train.py:40-66: student + teacher with CLS attention, MaskLoss + BackboneLoss, AdamW) at batch
@@ -634,7 +664,6 @@ def variant_b_leg(pkg, dev, torch, no_graph=False):
         runner.replay()
     torch.cuda.synchronize()
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-    K = 10
     e0.record()
     for _ in range(K):
         runner.replay()
@@ -772,6 +801,8 @@ def run_gpu(args):
     model = pkg.variant_a.DefaultVisionTransformerDiffPruning(pruning_loc=LOCS, token_ratio=RATIOS, distill=True, **DEIT_S)
     sd = seeded_weights(model)
     runner = pkg.runner.InferenceRunner(model, B, dev, dtype=torch.bfloat16, use_graph=not args.no_graph, warmup=2)
+    # the captured forward's kept-index tensors, which every replay rewrites (an eager forward rebinds model.kept_token_indices)
+    graph_kept = list(runner.model.kept_token_indices)
     line = {"metric": METRIC, "unit": UNIT, "n_gpus": world, "steps": K, "warmup": W, "higher_is_better": True, "scaling": "weak",
             "vs_baseline": None, "dtype": "bf16", "data": "synthetic"}
 
@@ -808,6 +839,9 @@ def run_gpu(args):
     total_ms = float(ms.item())
     value = world * B * K / (total_ms / 1e3)
     logits_ok = bool(torch.isfinite(runner.logits.float()).all())
+    if args.dump_outputs and rank == 0:
+        kept = graph_kept if runner.graph is not None else runner.model.kept_token_indices
+        dump_outputs(args.dump_outputs, {"logits": runner.logits, **{f"kept_token_indices_{s}": k for s, k in enumerate(kept)}})
 
     # ---- e2e: pinned host images -> device -> forward -> host logits, every step -----------------------
     e2e = None
@@ -915,9 +949,9 @@ def run_gpu(args):
     if "sweep" in legs:
         line["sweep"] = sweep_leg(pkg.ops, dev, torch, pk)
     if "base" in legs and rank == 0:
-        line["arch_base"] = base_leg(pkg, dev, torch, pk, args.no_graph)
+        line["arch_base"] = base_leg(pkg, dev, torch, pk, K, args.no_graph)
     if "variant_b" in legs and rank == 0:
-        line["variant_b"] = variant_b_leg(pkg, dev, torch, args.no_graph)
+        line["variant_b"] = variant_b_leg(pkg, dev, torch, K, args.no_graph)
         torch.cuda.empty_cache()
     if "eager" in legs:
         line["gpu_eager_baseline"] = gpu_eager_leg(sd, dev, B, torch)

@@ -58,7 +58,42 @@ def sd_checksum(sd):
     return [s, a]
 
 
-def save_npz(name, arrays, meta):
+# A golden tensor of more than SAMPLE_ABOVE elements is stored as SAMPLE_N of its elements (flat indices from sample_index),
+# with its shape and its largest magnitude in meta["sampled"]: every golden file stays under 1 MB.
+SAMPLE_ABOVE, SAMPLE_N = 16384, 8192
+
+
+def sample_index(numel):
+    """Sorted flat indices of the stored elements of a sampled golden tensor.  numpy's legacy RandomState keeps its stream
+    fixed across numpy versions, so the indices are a pure function of `numel`."""
+    return torch.from_numpy(np.sort(np.random.RandomState(numel).choice(numel, SAMPLE_N, replace=False)))
+
+
+def sample_arrays(arrays, meta):
+    """Replace every tensor above SAMPLE_ABOVE elements by its sample; record what golden_view needs in meta["sampled"].
+    Used for the model goldens (save_npz(..., sample=True)), the only ones that would exceed 1 MB whole."""
+    out = dict(arrays)
+    for k, v in arrays.items():
+        if torch.is_tensor(v) and v.numel() > SAMPLE_ABOVE:
+            out[k] = v.reshape(-1)[sample_index(v.numel())]
+            meta.setdefault("sampled", {})[k] = dict(shape=list(v.shape), absmax=float(v.abs().max()))
+    return out
+
+
+def golden_view(arrays, meta, key, t):
+    """(t, golden, max |golden|) for comparing a computed tensor `t` with golden `key`: a sampled golden is compared on the
+    same elements of t, against the largest magnitude of the whole golden tensor."""
+    s = meta.get("sampled", {}).get(key)
+    if s is None:
+        ref = arrays[key]
+        return t, ref, float(ref.abs().max())
+    assert list(t.shape) == s["shape"], (key, tuple(t.shape), s["shape"])
+    return t.reshape(-1)[sample_index(t.numel()).to(t.device)], arrays[key], s["absmax"]
+
+
+def save_npz(name, arrays, meta, sample=False):
+    if sample:
+        arrays = sample_arrays(arrays, meta)
     out = {k: (v.detach().cpu().numpy() if torch.is_tensor(v) else np.asarray(v)) for k, v in arrays.items()}
     out["__meta__"] = np.frombuffer(json.dumps(meta).encode(), dtype=np.uint8)
     np.savez_compressed(os.path.join(HERE, name), **out)

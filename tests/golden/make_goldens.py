@@ -273,7 +273,7 @@ def model_goldens():
     # calls alternate: (x, now_policy), (prev_decision, keep_policy)
     for s in range(len(locs)):
         A[f"A_eval_kept{s}"] = rec_idx[2 * s + 1]
-    fx.save_npz("golden_models.npz", A, meta)
+    fx.save_npz("golden_models.npz", A, meta, sample=True)
     print("golden_models.npz:", len(A), "arrays")
 
 

@@ -1,8 +1,7 @@
-"""Load the UNMODIFIED reference hot-path modules from /root/reference (this container only).
+"""Load the UNMODIFIED reference hot-path modules from a checkout of marc345/Dense2Sparse-ViT (REF_ROOT).
 
-Test/fixture infrastructure: used by make_goldens.py and by the optional
-"live reference" CPU tests.  /root/reference does not exist on the GPU box, so
-nothing under `-m gpu`, smoke() or bench.py may import this module.
+Golden-generation infrastructure: used by make_goldens.py and make_loss_goldens.py only.  The tests, smoke()
+and bench.py read the stored goldens and never import this module: the reference is not part of this repository.
 
 The reference needs six timm names (vit_models/dynamic_vit.py:30-32,
 vit_models/default_dynamic_vit.py:30-32); timm is not installed, so a stub

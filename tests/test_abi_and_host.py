@@ -131,32 +131,83 @@ def test_state_dict_names_follow_reference(d2s):
     assert "score_predictor.0.out_conv.6.bn.running_mean" in set(s.state_dict())
 
 
+# The hot-path attribute surface of the reference's modules (SURVEY.md 8b): what patch.install() must replace, and nothing else.
+_REFERENCE_SURFACE = {
+    "peturbed_topk": ["PerturbedTopK.__call__"],
+    "default_dynamic_vit": ["batch_index_select", "Attention.softmax_with_policy", "Attention.forward", "Block.forward",
+                            "PatchEmbed.forward", "PredictorLG.forward", "DefaultVisionTransformerDiffPruning.forward",
+                            "DefaultVisionTransformerTeacher.forward"],
+    "dynamic_vit": ["batch_index_select", "PerturbedTopK", "Attention.softmax_with_policy", "Attention.forward", "Block.forward",
+                    "PatchEmbed.forward", "PredictorLG.forward", "VisionTransformerDiffPruning.forward",
+                    "VisionTransformerDiffPruning.forward_cls_attn", "VisionTransformerTeacher.forward",
+                    "VisionTransformerTeacher.forward_cls_attention"],
+}
+
+
+def _reference_stand_ins(d2s):
+    """Module objects named like the reference's vit_models modules, carrying the surface above plus attributes install() must
+    leave alone (Mlp, helpers).  Every original is a distinct function that fails if it runs; dynamic_vit.PerturbedTopK is the
+    class of peturbed_topk, as the reference imports it.  The Variant A model class builds like the reference's (same
+    constructor, same submodules), so a patched forward runs on real tensors."""
+    import types
+
+    def original():
+        def f(*a, **k):
+            raise AssertionError("the reference's own code ran: install() did not replace it")
+        return f
+
+    mods = {}
+    for name, surface in _REFERENCE_SURFACE.items():
+        mod = types.ModuleType("vit_models." + name)
+        mod.untouched_helper = original()
+        mod.Mlp = type("Mlp", (), {"__module__": mod.__name__, "forward": original()})
+        for entry in surface:
+            owner, _, attr = entry.rpartition(".")
+            if not owner:
+                setattr(mod, attr, mods["peturbed_topk"].PerturbedTopK if attr == "PerturbedTopK" else original())
+                continue
+            if not hasattr(mod, owner):
+                base = (d2s.variant_a.DefaultVisionTransformerDiffPruning,) if owner == "DefaultVisionTransformerDiffPruning" else ()
+                setattr(mod, owner, type(owner, base, {"__module__": mod.__name__, "untouched": original()}))
+            setattr(getattr(mod, owner), attr, original())
+        mods[name] = mod
+    return mods
+
+
+def _attribute_snapshot(mods):
+    """(module, attribute) and (module, Class.attribute) -> object, for the classes each module defines."""
+    snap = {}
+    for name, mod in mods.items():
+        for attr, val in vars(mod).items():
+            snap[(name, attr)] = val
+            if isinstance(val, type) and val.__module__ == mod.__name__:
+                for cattr, cval in vars(val).items():
+                    snap[(name, f"{attr}.{cattr}")] = cval
+    return snap
+
+
 def test_patch_install_swaps_reference_surface(d2s):
-    """In the build container the real reference is importable: install() must replace exactly the
-    hot-path attribute surface of SURVEY.md 8b and uninstall() must restore it."""
-    sys.path.insert(0, os.path.join(ROOT, "tests", "golden"))
-    import refload
-    if not refload.reference_available():
-        pytest.skip("/root/reference not present (GPU box)")
-    ns = refload.load_reference()
-    orig_a = ns.ddvit.DefaultVisionTransformerDiffPruning.forward
-    orig_sel = ns.ddvit.batch_index_select
-    orig_b = ns.dvit.Attention.softmax_with_policy
-    d2s.patch.install(dvit=ns.dvit, ddvit=ns.ddvit, ptopk=ns.ptopk)
+    """install() must replace exactly the hot-path attribute surface of SURVEY.md 8b and uninstall() must restore it."""
+    mods = _reference_stand_ins(d2s)
+    before = _attribute_snapshot(mods)
+    d2s.patch.install(ddvit=mods["default_dynamic_vit"], dvit=mods["dynamic_vit"], ptopk=mods["peturbed_topk"])
     try:
-        assert ns.ddvit.batch_index_select is d2s.ops.batch_index_select
-        assert ns.ddvit.DefaultVisionTransformerDiffPruning.forward is not orig_a
-        assert ns.dvit.Attention.softmax_with_policy is not orig_b
-        m = ns.ddvit.DefaultVisionTransformerDiffPruning(patch_size=16, embed_dim=64, depth=2, num_heads=2,
-                                                         pruning_loc=[1], token_ratio=[0.7], distill=True).eval()
+        after = _attribute_snapshot(mods)
+        assert set(after) == set(before)
+        changed = {k for k in before if after[k] is not before[k]}
+        assert changed == {(name, entry) for name, surface in _REFERENCE_SURFACE.items() for entry in surface}
+        ddvit, dvit = mods["default_dynamic_vit"], mods["dynamic_vit"]
+        assert ddvit.batch_index_select is d2s.ops.batch_index_select and dvit.batch_index_select is d2s.ops.batch_index_select
+        assert dvit.PerturbedTopK is d2s.perturbed_topk.PerturbedTopK
+        m = ddvit.DefaultVisionTransformerDiffPruning(patch_size=16, embed_dim=64, depth=2, num_heads=2,
+                                                      pruning_loc=[1], token_ratio=[0.7], distill=True).eval()
         with pytest.raises(RuntimeError, match="no CPU fallback|CUDA"):   # patched forward reaches the kernels
             with torch.no_grad():
                 m(torch.randn(1, 3, 224, 224))
     finally:
         d2s.patch.uninstall()
-    assert ns.ddvit.batch_index_select is orig_sel
-    assert ns.ddvit.DefaultVisionTransformerDiffPruning.forward is orig_a
-    assert ns.dvit.Attention.softmax_with_policy is orig_b
+    restored = _attribute_snapshot(mods)
+    assert set(restored) == set(before) and all(restored[k] is before[k] for k in before)
 
 
 # ---- multi-rank path on CPU (gloo, world_size 2) ----------------------------------------------------
