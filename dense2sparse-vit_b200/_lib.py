@@ -76,6 +76,12 @@ SIGNATURES = {
     "d2s_mlp_residual_ln_bf16": [_p, _p, _p, _p, _p, _p, _p, _p, _f, _i, _i, _i, _i, _i, _p, _p, _p],
     "d2s_mlp_lnin_residual_ln_bf16": [_p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _f, _i, _i, _i, _i, _i, _p, _p, _p, _p],
     "d2s_add_layernorm": [_p, _p, _p, _p, _i, _i, _i, _i, ctypes.c_longlong, ctypes.c_longlong, _f, _i, _p, _p, _p],
+    "d2s_threshold_select_varlen_f32": [_p, _p, _i, _i, _f, _p, _p, _p, _p],
+    "d2s_score_tail_b_varlen": [_p, _p, _i, _i, _i, _i, _p, _p, _f, _p, _p, _i, _p, _p, _p],
+    "d2s_pool_concat_varlen_inplace": [_p, _p, _i, _i, _i, _i, _p],
+    "d2s_attn_varlen_fwd": [_p, _p, _i, _i, _i, _i, _i, _f, _p, _p, _p],
+    "d2s_gather_layernorm_varlen": [_p, _p, _p, _p, _p, _i, _i, _i, _i, _i, _f, _p, _p, _p],
+    "d2s_gather_layernorm_stats_varlen": [_p, _p, _p, _i, _i, _i, _i, _f, _p, _p, _p],
 }
 INFO_SYMBOLS = ["d2s_last_error", "d2s_version", "d2s_launch_count"]
 ALL_SYMBOLS = sorted(list(SIGNATURES) + INFO_SYMBOLS)

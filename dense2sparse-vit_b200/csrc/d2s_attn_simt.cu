@@ -468,10 +468,12 @@ constexpr int kAttnWarps = kAttnThreads / 32;
 constexpr int kQR = 4;       // query rows per warp pass
 constexpr int kAttnEPL = 8;  // T <= 256
 
-template <typename T_, int HD>
+// kVar: variable-length form (d2s_attn_varlen_fwd): image b has Tv = lens[b] valid tokens of its T (padded) rows; rows and cls_row
+// columns Tv..T-1 are written as zeros (no policy)
+template <typename T_, int HD, bool kVar = false>
 __global__ void __launch_bounds__(kAttnThreads)
 attn_simt_fwd_kernel(const T_* __restrict__ qkv, const float* __restrict__ policy, int T, int H, float scale, float eps,
-                     T_* __restrict__ out, float* __restrict__ cls_row, int rows_per_cta) {
+                     T_* __restrict__ out, float* __restrict__ cls_row, int rows_per_cta, const int* __restrict__ lens) {
   extern __shared__ float sm[];
   float* Ks = sm;                                  // T x (HD+1)
   float* Vs = Ks + (size_t)T * (HD + 1);           // T x HD
@@ -484,7 +486,8 @@ attn_simt_fwd_kernel(const T_* __restrict__ qkv, const float* __restrict__ polic
   const T_* q_base = qkv + (size_t)b * T * tok_stride + (size_t)h * HD;
   const T_* k_base = q_base + (size_t)H * HD;
   const T_* v_base = q_base + (size_t)2 * H * HD;
-  for (int idx = threadIdx.x; idx < T * HD; idx += kAttnThreads) {
+  const int Tv = kVar ? min(max(lens[b], 0), T) : T;
+  for (int idx = threadIdx.x; idx < Tv * HD; idx += kAttnThreads) {
     const int j = idx / HD, d = idx % HD;
     Ks[j * (HD + 1) + d] = ld_as_float(k_base, (size_t)j * tok_stride + d);
     Vs[j * HD + d] = ld_as_float(v_base, (size_t)j * tok_stride + d);
@@ -496,11 +499,17 @@ attn_simt_fwd_kernel(const T_* __restrict__ qkv, const float* __restrict__ polic
   float* my_q = qs + warp * kQR * HD;
   float* my_p = ps + (size_t)warp * kQR * T;
   const int row_begin = blockIdx.x * rows_per_cta;
-  const int row_end = min(T, row_begin + rows_per_cta);
+  const int row_end = min(Tv, row_begin + rows_per_cta);
+  if (kVar) {   // pad rows of this CTA's row range and the CLS row's pad columns: zeros
+    for (int idx = threadIdx.x; idx < (min(T, row_begin + rows_per_cta) - max(row_begin, Tv)) * HD; idx += kAttnThreads)
+      st_from_float(out, ((size_t)b * T + max(row_begin, Tv) + idx / HD) * (size_t)(H * HD) + (size_t)h * HD + idx % HD, 0.f);
+    if (cls_row && blockIdx.x == 0)
+      for (int j = Tv + threadIdx.x; j < T; j += kAttnThreads) cls_row[(size_t)bh * T + j] = 0.f;
+  }
   for (int i0 = row_begin + warp * kQR; i0 < row_end; i0 += kAttnWarps * kQR) {
 #pragma unroll
     for (int r = 0; r < kQR; ++r) {
-      const int i = min(i0 + r, T - 1);
+      const int i = min(i0 + r, Tv - 1);
       for (int d = lane; d < HD; d += 32) my_q[r * HD + d] = ld_as_float(q_base, (size_t)i * tok_stride + d) * scale;
     }
     __syncwarp();
@@ -516,7 +525,7 @@ attn_simt_fwd_kernel(const T_* __restrict__ qkv, const float* __restrict__ polic
 #pragma unroll
       for (int e = 0; e < kAttnEPL; ++e) {
         const int j = lane + 32 * e;
-        if (j < T) {
+        if (j < Tv) {
           const float kv = Ks[j * (HD + 1) + d];
 #pragma unroll
           for (int r = 0; r < kQR; ++r) s[r][e] = fmaf(qd[r], kv, s[r][e]);
@@ -528,14 +537,14 @@ attn_simt_fwd_kernel(const T_* __restrict__ qkv, const float* __restrict__ polic
       const int i = i0 + r;
       float m = -INFINITY;
 #pragma unroll
-      for (int e = 0; e < kAttnEPL; ++e) if (lane + 32 * e < T) m = fmaxf(m, s[r][e]);
+      for (int e = 0; e < kAttnEPL; ++e) if (lane + 32 * e < Tv) m = fmaxf(m, s[r][e]);
       m = warp_max(m);
       float sum = 0.f;
 #pragma unroll
       for (int e = 0; e < kAttnEPL; ++e) {
         const int j = lane + 32 * e;
         float a = 0.f;
-        if (j < T) a = expf(s[r][e] - m) * ((j == i) ? 1.0f : pol_s[j]);
+        if (j < Tv) a = expf(s[r][e] - m) * ((j == i) ? 1.0f : pol_s[j]);
         s[r][e] = a;
         sum += a;
       }
@@ -544,7 +553,7 @@ attn_simt_fwd_kernel(const T_* __restrict__ qkv, const float* __restrict__ polic
 #pragma unroll
       for (int e = 0; e < kAttnEPL; ++e) {
         const int j = lane + 32 * e;
-        if (j < T) {
+        if (j < Tv) {
           const float p = (s[r][e] + c) / den;
           my_p[r * T + j] = p;
           if (cls_row && i == 0) cls_row[(size_t)bh * T + j] = p;
@@ -557,7 +566,7 @@ attn_simt_fwd_kernel(const T_* __restrict__ qkv, const float* __restrict__ polic
     for (int r = 0; r < kQR; ++r)
 #pragma unroll
       for (int q = 0; q < HD / 32; ++q) o[r][q] = 0.f;
-    for (int j = 0; j < T; ++j) {
+    for (int j = 0; j < Tv; ++j) {
       float vv[HD / 32];
 #pragma unroll
       for (int q = 0; q < HD / 32; ++q) vv[q] = Vs[j * HD + lane + 32 * q];
@@ -583,13 +592,13 @@ attn_simt_fwd_kernel(const T_* __restrict__ qkv, const float* __restrict__ polic
 
 template <typename T_, int HD>
 static int launch_attn_simt(const void* qkv, const float* policy, int B, int T, int H, float scale, float eps, void* out,
-                            float* cls_row, cudaStream_t stream) {
+                            float* cls_row, cudaStream_t stream, const int* lens) {
   const size_t smem = sizeof(float) * ((size_t)T * (HD + 1) + (size_t)T * HD + ((T + 3) & ~3) +
                                        (size_t)kAttnWarps * kQR * HD + (size_t)kAttnWarps * kQR * T);
   D2S_REQUIRE(smem <= 227 * 1024, D2S_ERR_ARG, "attn(simt): T=%d needs %zu B of shared memory", T, smem);
-  auto kern = attn_simt_fwd_kernel<T_, HD>;
-  static SmemOptIn opt;  // one per template instantiation
-  cudaError_t e = opt_in_smem(opt, kern, 227 * 1024);
+  auto kern = lens ? attn_simt_fwd_kernel<T_, HD, true> : attn_simt_fwd_kernel<T_, HD>;
+  static SmemOptIn opt[2];  // one per kernel instantiation
+  cudaError_t e = opt_in_smem(opt[lens ? 1 : 0], kern, 227 * 1024);
   D2S_REQUIRE(e == cudaSuccess, D2S_ERR_CUDA, "attn(simt): cudaFuncSetAttribute: %s", cudaGetErrorString(e));
   // enough CTAs to fill the machine: split the query rows when B*H is small
   int chunks = ceil_div(2 * kNumSMs, B * H);
@@ -597,21 +606,21 @@ static int launch_attn_simt(const void* qkv, const float* policy, int B, int T, 
   chunks = chunks < 1 ? 1 : (chunks > max_chunks ? max_chunks : chunks);
   const int rows_per_cta = ceil_div(ceil_div(T, chunks), kQR) * kQR;
   dim3 grid(ceil_div(T, rows_per_cta), B * H);
-  kern<<<grid, kAttnThreads, smem, stream>>>((const T_*)qkv, policy, T, H, scale, eps, (T_*)out, cls_row, rows_per_cta);
+  kern<<<grid, kAttnThreads, smem, stream>>>((const T_*)qkv, policy, T, H, scale, eps, (T_*)out, cls_row, rows_per_cta, lens);
   count_launch();
-  return check_launch("d2s_attn_policy_fwd(simt)");
+  return check_launch(lens ? "d2s_attn_varlen_fwd(simt)" : "d2s_attn_policy_fwd(simt)");
 }
 
 int attn_simt_dispatch(const void* qkv, const float* policy, int dtype, int B, int T, int H, int hd, float scale,
-                       float eps, void* out, float* cls_row, cudaStream_t stream) {
+                       float eps, void* out, float* cls_row, cudaStream_t stream, const int* lens) {
   D2S_REQUIRE(hd == 64 || hd == 32, D2S_ERR_ARG, "attn(simt): hd=%d unsupported (32 or 64)", hd);
   D2S_REQUIRE(T >= 1 && T <= 32 * kAttnEPL, D2S_ERR_ARG, "attn(simt): T=%d outside [1,%d]", T, 32 * kAttnEPL);
   if (dtype == D2S_F32) {
-    return hd == 64 ? launch_attn_simt<float, 64>(qkv, policy, B, T, H, scale, eps, out, cls_row, stream)
-                    : launch_attn_simt<float, 32>(qkv, policy, B, T, H, scale, eps, out, cls_row, stream);
+    return hd == 64 ? launch_attn_simt<float, 64>(qkv, policy, B, T, H, scale, eps, out, cls_row, stream, lens)
+                    : launch_attn_simt<float, 32>(qkv, policy, B, T, H, scale, eps, out, cls_row, stream, lens);
   }
-  return hd == 64 ? launch_attn_simt<__nv_bfloat16, 64>(qkv, policy, B, T, H, scale, eps, out, cls_row, stream)
-                  : launch_attn_simt<__nv_bfloat16, 32>(qkv, policy, B, T, H, scale, eps, out, cls_row, stream);
+  return hd == 64 ? launch_attn_simt<__nv_bfloat16, 64>(qkv, policy, B, T, H, scale, eps, out, cls_row, stream, lens)
+                  : launch_attn_simt<__nv_bfloat16, 32>(qkv, policy, B, T, H, scale, eps, out, cls_row, stream, lens);
 }
 
 }  // namespace d2s

@@ -57,19 +57,23 @@ __device__ __forceinline__ float row_lanes_sum(float v) {
 
 // kLPR lanes per row (16: two rows per warp; 32 for wide rows -- at 12 vectors per lane the 1536-wide predictor LayerNorm ran at
 // 2.6 TB/s), kVPL 16-byte vectors per lane (D <= kLPR * kVPL * elems-per-vector)
-template <typename T_, int kVPL, int kLPR>
+// kVar: variable-length gather (d2s_gather_layernorm_varlen): output token t >= 1 of image b is a pad row when t - 1 >= cnt[b]; it
+// is processed as a zero row (its index is not read) and written as zeros, out_norm included.
+template <typename T_, int kVPL, int kLPR, bool kVar = false>
 __global__ void __launch_bounds__(kLnThreads)
 add_layernorm_kernel(const T_* __restrict__ x, const T_* __restrict__ y, const T_* __restrict__ gamma,
                      const T_* __restrict__ beta, long long rows, int T, int D, long long x_stride_b, long long x_stride_t,
                      float eps, int norm_row0, T_* __restrict__ out_sum, T_* __restrict__ out_norm,
-                     const int64_t* __restrict__ gather_idx, const T_* __restrict__ cls_row, float2* __restrict__ stats) {
+                     const int64_t* __restrict__ gather_idx, const T_* __restrict__ cls_row, float2* __restrict__ stats,
+                     const int* __restrict__ cnt) {
   constexpr int VE = LnVec<T_>::kElems;
   const int sub = threadIdx.x & (kLPR - 1);
   const long long row = (long long)blockIdx.x * (kLnThreads / kLPR) + threadIdx.x / kLPR;
-  const bool row_ok = row < rows;
   const int nvec = D / VE;
-  const long long b = row_ok ? row / T : 0;
-  const int t = row_ok ? (int)(row - b * T) : 0;
+  const long long b = row < rows ? row / T : 0;
+  const int t = row < rows ? (int)(row - b * T) : 0;
+  const bool pad = kVar && row < rows && t > 0 && t - 1 >= cnt[b];
+  const bool row_ok = row < rows && !pad;   // a row whose input is read
   // gather mode (d2s_gather_layernorm): output token 0 is the CLS row, token t >= 1 is input token idx[b, t-1] + 1
   const long long src_t = (gather_idx && row_ok && t > 0) ? gather_idx[b * (T - 1) + (t - 1)] + 1 : (long long)t;
   // assemble mode (d2s_assemble_layernorm, cls_row != NULL): token 0 is the class token, token t >= 1 is patch t-1 of x, and
@@ -99,7 +103,7 @@ add_layernorm_kernel(const T_* __restrict__ x, const T_* __restrict__ y, const T
       for (int q = 0; q < VE; ++q) v[k][q] = 0.f;
     }
   }
-  if (out_sum && row_ok) {
+  if (out_sum && (row_ok || pad)) {
 #pragma unroll
     for (int k = 0; k < kVPL; ++k) {
       const int vi = sub + kLPR * k;
@@ -122,8 +126,8 @@ add_layernorm_kernel(const T_* __restrict__ x, const T_* __restrict__ y, const T
   const float rstd = rsqrtf(row_lanes_sum<kLPR>(var) / (float)D + eps);
   // per-row (mean, rstd) for a consumer that applies the LayerNorm itself (the qkv GEMM on its resident input rows); out_norm may
   // then be NULL.  For bf16 both forms use h = fma(fma(x, rstd, -mean * rstd), gamma, beta), so they give the same bits.
-  if (stats != nullptr && row_ok && sub == 0) stats[row] = make_float2(mean, rstd);
-  if (!row_ok || t < norm_row0 || out_norm == nullptr) return;
+  if (stats != nullptr && (row_ok || pad) && sub == 0) stats[row] = make_float2(mean, rstd);
+  if (!(row_ok || pad) || t < norm_row0 || out_norm == nullptr) return;
   const float shift = -mean * rstd;
   T_* hr = out_norm + (b * (T - norm_row0) + (t - norm_row0)) * (long long)D;
 #pragma unroll
@@ -135,7 +139,7 @@ add_layernorm_kernel(const T_* __restrict__ x, const T_* __restrict__ y, const T
       LnVec<T_>::unpack(*reinterpret_cast<const int4*>(beta + (size_t)vi * VE), bt);
 #pragma unroll
       for (int q = 0; q < VE; ++q)     // bf16: the form the GEMM kernels use (same bits as the on-the-fly norm); fp32: the more accurate one
-        o[q] = sizeof(T_) == 2 ? fmaf(fmaf(v[k][q], rstd, shift), g[q], bt[q]) : fmaf((v[k][q] - mean) * rstd, g[q], bt[q]);
+        o[q] = pad ? 0.f : sizeof(T_) == 2 ? fmaf(fmaf(v[k][q], rstd, shift), g[q], bt[q]) : fmaf((v[k][q] - mean) * rstd, g[q], bt[q]);
       *reinterpret_cast<int4*>(hr + (size_t)vi * VE) = LnVec<T_>::pack(o);
     }
   }
@@ -157,25 +161,26 @@ __global__ void apply_ln_stats_kernel(const __nv_bfloat16* __restrict__ x, const
         __float2bfloat16_rn(fmaf(fmaf(__bfloat162float(xr[c]), st.y, shift), __bfloat162float(gamma[c]), __bfloat162float(beta[c])));
 }
 
-template <typename T_>
+template <typename T_, bool kVar = false>
 static int launch_ln(const void* x, const void* y, const void* gamma, const void* beta, int B, int T, int D,
                      long long sb, long long st, float eps, int norm_row0, void* out_sum, void* out_norm, cudaStream_t stream,
-                     const int64_t* gather_idx = nullptr, const void* cls_row = nullptr, float* stats = nullptr) {
+                     const int64_t* gather_idx = nullptr, const void* cls_row = nullptr, float* stats = nullptr,
+                     const int* cnt = nullptr) {
   constexpr int VE = LnVec<T_>::kElems;
   const long long rows = (long long)B * T;
   const int nvec = D / VE;
   const int vpl = ceil_div(nvec, 16);
 #define D2S_LN_LAUNCH(V, L)                                                                                            \
-  add_layernorm_kernel<T_, V, L><<<(unsigned)((rows + kLnThreads / L - 1) / (kLnThreads / L)), kLnThreads, 0, stream>>>(  \
+  add_layernorm_kernel<T_, V, L, kVar><<<(unsigned)((rows + kLnThreads / L - 1) / (kLnThreads / L)), kLnThreads, 0, stream>>>(  \
       (const T_*)x, (const T_*)y, (const T_*)gamma, (const T_*)beta, rows, T, D, sb, st, eps, norm_row0, (T_*)out_sum,     \
-      (T_*)out_norm, gather_idx, (const T_*)cls_row, reinterpret_cast<float2*>(stats))
+      (T_*)out_norm, gather_idx, (const T_*)cls_row, reinterpret_cast<float2*>(stats), cnt)
   if (vpl <= 2) D2S_LN_LAUNCH(2, 16);
   else if (vpl <= 3) D2S_LN_LAUNCH(3, 16);
   else if (vpl <= 6) D2S_LN_LAUNCH(3, 32);
   else D2S_LN_LAUNCH(6, 32);
 #undef D2S_LN_LAUNCH
   count_launch();
-  return check_launch("d2s_add_layernorm");
+  return check_launch(kVar ? "d2s_gather_layernorm_varlen" : "d2s_add_layernorm");
 }
 
 }  // namespace d2s
@@ -262,6 +267,42 @@ extern "C" int d2s_gather_layernorm_stats(const void* x, const int64_t* idx, int
   if (B == 0) return D2S_OK;
   return launch_ln<__nv_bfloat16>(x, nullptr, x, x, B, K + 1, D, (long long)T_in * D, D, eps, 0, out_sum, nullptr, (cudaStream_t)stream,
                                   K ? idx : nullptr, nullptr, stats);
+}
+
+/* Variable-length forms of the two gathers above (threshold inference): idx (B,Kmax) holds image b's count[b] kept spatial indices
+ * followed by padding (never read); output rows 1 + count[b] .. Kmax of out_sum / out_norm are zeros, stats of those rows are the
+ * (mean, rstd) of a zero row. */
+extern "C" int d2s_gather_layernorm_varlen(const void* x, const int64_t* idx, const int* count, const void* gamma, const void* beta,
+                                           int dtype, int B, int T_in, int D, int Kmax, float eps, void* out_sum, void* out_norm,
+                                           d2s_stream_t stream) {
+  D2S_REQUIRE(x && (idx || Kmax == 0) && count && gamma && beta && out_sum && out_norm, D2S_ERR_ARG, "gather_layernorm_varlen: null pointer");
+  D2S_REQUIRE(dtype == D2S_F32 || dtype == D2S_BF16, D2S_ERR_ARG, "gather_layernorm_varlen: dtype %d unsupported", dtype);
+  D2S_REQUIRE(B >= 0 && T_in >= 1 && D >= 1 && Kmax >= 0 && Kmax <= T_in - 1, D2S_ERR_ARG,
+              "gather_layernorm_varlen: bad shape B=%d T_in=%d D=%d Kmax=%d", B, T_in, D, Kmax);
+  const int ve = dtype == D2S_BF16 ? 8 : 4;
+  D2S_REQUIRE(D % ve == 0 && D / ve <= 16 * 12, D2S_ERR_ARG, "gather_layernorm_varlen: D=%d must be a multiple of %d and at most %d",
+              D, ve, 16 * 12 * ve);
+  D2S_REQUIRE(aligned16(x) && aligned16(gamma) && aligned16(beta) && aligned16(out_sum) && aligned16(out_norm), D2S_ERR_ALIGN,
+              "gather_layernorm_varlen: pointers must be 16-byte aligned");
+  if (B == 0) return D2S_OK;
+  const long long sb = (long long)T_in * D, st = D;
+  return dtype == D2S_BF16
+             ? launch_ln<__nv_bfloat16, true>(x, nullptr, gamma, beta, B, Kmax + 1, D, sb, st, eps, 0, out_sum, out_norm,
+                                              (cudaStream_t)stream, Kmax ? idx : nullptr, nullptr, nullptr, count)
+             : launch_ln<float, true>(x, nullptr, gamma, beta, B, Kmax + 1, D, sb, st, eps, 0, out_sum, out_norm, (cudaStream_t)stream,
+                                      Kmax ? idx : nullptr, nullptr, nullptr, count);
+}
+
+extern "C" int d2s_gather_layernorm_stats_varlen(const void* x, const int64_t* idx, const int* count, int B, int T_in, int D, int Kmax,
+                                                 float eps, void* out_sum, float* stats, d2s_stream_t stream) {
+  D2S_REQUIRE(x && (idx || Kmax == 0) && count && out_sum && stats, D2S_ERR_ARG, "gather_layernorm_stats_varlen: null pointer");
+  D2S_REQUIRE(B >= 0 && T_in >= 1 && D >= 8 && Kmax >= 0 && Kmax <= T_in - 1 && D % 8 == 0 && D / 8 <= 16 * 12, D2S_ERR_ARG,
+              "gather_layernorm_stats_varlen: bad shape B=%d T_in=%d D=%d Kmax=%d", B, T_in, D, Kmax);
+  D2S_REQUIRE(aligned16(x) && aligned16(out_sum) && (reinterpret_cast<uintptr_t>(stats) & 7u) == 0, D2S_ERR_ALIGN,
+              "gather_layernorm_stats_varlen: x / out_sum must be 16-byte aligned, stats 8-byte aligned");
+  if (B == 0) return D2S_OK;
+  return launch_ln<__nv_bfloat16, true>(x, nullptr, x, x, B, Kmax + 1, D, (long long)T_in * D, D, eps, 0, out_sum, nullptr,
+                                        (cudaStream_t)stream, Kmax ? idx : nullptr, nullptr, stats, count);
 }
 
 extern "C" int d2s_assemble_layernorm_stats(const void* patches, const void* cls, const void* pos, int B, int N, int D, float eps,

@@ -155,12 +155,15 @@ pool_act_kernel(const T_* __restrict__ z, const float* __restrict__ policy, int 
 // In-place form for Variant B (dynamic_vit.py:538-545): z (B,N,C) already activated; the upper half of every token
 // row is REPLACED by the image's mean over tokens of that upper half, i.e. z becomes cat(local, global.expand) without
 // a second tensor.  grid = B; phase 1 reduces, phase 2 broadcasts.
-template <typename T_>
+// kVar (d2s_pool_concat_varlen_inplace): image b has Nv = nv[b] valid rows of its N (padded) rows; the mean runs over those and
+// is written into those; pad rows are neither read nor written.
+template <typename T_, bool kVar = false>
 __global__ void __launch_bounds__(kPoolThreads)
-pool_concat_inplace_kernel(T_* __restrict__ z, int N, int C) {
+pool_concat_inplace_kernel(T_* __restrict__ z, int N, int C, const int* __restrict__ nv) {
   constexpr int VE = PVec<T_>::kElems;
   extern __shared__ float red[];  // groups x (C/2), then the pooled row at red[0 .. C/2)
   const int b = blockIdx.x;
+  const int Nv = kVar ? min(max(nv[b], 0), N) : N;
   const int hvec = C / VE / 2, half = C / 2;
   const int groups = kPoolThreads / hvec;   // host guarantees hvec <= kPoolThreads
   const int v = threadIdx.x % hvec, g = threadIdx.x / hvec;
@@ -168,7 +171,7 @@ pool_concat_inplace_kernel(T_* __restrict__ z, int N, int C) {
 #pragma unroll
   for (int q = 0; q < 8; ++q) acc[q] = 0.f;
   if (g < groups) {
-    for (int n = g; n < N; n += groups) {
+    for (int n = g; n < Nv; n += groups) {
       float x[8];
       PVec<T_>::unpack(*reinterpret_cast<const int4*>(z + ((size_t)b * N + n) * C + half + (size_t)v * VE), x);
 #pragma unroll
@@ -181,7 +184,7 @@ pool_concat_inplace_kernel(T_* __restrict__ z, int N, int C) {
   for (int c = threadIdx.x; c < half; c += kPoolThreads) {
     float s = 0.f;
     for (int gg = 0; gg < groups; ++gg) s += red[(size_t)gg * half + c];
-    red[(size_t)groups * half + c] = PVec<T_>::round(s / (float)N);   // torch.mean rounds to the tensor dtype
+    red[(size_t)groups * half + c] = PVec<T_>::round(s / (float)Nv);  // torch.mean rounds to the tensor dtype
   }
   __syncthreads();
   if (g < groups) {
@@ -189,7 +192,7 @@ pool_concat_inplace_kernel(T_* __restrict__ z, int N, int C) {
 #pragma unroll
     for (int q = 0; q < VE; ++q) m[q] = red[(size_t)groups * half + (size_t)v * VE + q];
     const int4 packed = PVec<T_>::pack(m);
-    for (int n = g; n < N; n += groups)
+    for (int n = g; n < Nv; n += groups)
       *reinterpret_cast<int4*>(z + ((size_t)b * N + n) * C + half + (size_t)v * VE) = packed;
   }
 }
@@ -498,11 +501,30 @@ extern "C" int d2s_pool_concat_inplace(void* z, int dtype, int B, int N, int C, 
   const size_t smem = ((size_t)groups + 1) * (C / 2) * sizeof(float);
   D2S_REQUIRE(smem <= 48 * 1024, D2S_ERR_ARG, "pool_concat_inplace: C=%d needs %zu B of shared memory", C, smem);
   if (dtype == D2S_BF16)
-    pool_concat_inplace_kernel<__nv_bfloat16><<<B, kPoolThreads, smem, (cudaStream_t)stream>>>((__nv_bfloat16*)z, N, C);
+    pool_concat_inplace_kernel<__nv_bfloat16><<<B, kPoolThreads, smem, (cudaStream_t)stream>>>((__nv_bfloat16*)z, N, C, nullptr);
   else
-    pool_concat_inplace_kernel<float><<<B, kPoolThreads, smem, (cudaStream_t)stream>>>((float*)z, N, C);
+    pool_concat_inplace_kernel<float><<<B, kPoolThreads, smem, (cudaStream_t)stream>>>((float*)z, N, C, nullptr);
   count_launch();
   return check_launch("d2s_pool_concat_inplace");
+}
+
+extern "C" int d2s_pool_concat_varlen_inplace(void* z, const int* n, int dtype, int B, int Nmax, int C, d2s_stream_t stream) {
+  D2S_REQUIRE(z && n, D2S_ERR_ARG, "pool_concat_varlen_inplace: null pointer");
+  D2S_REQUIRE(dtype == D2S_F32 || dtype == D2S_BF16, D2S_ERR_ARG, "pool_concat_varlen_inplace: dtype %d unsupported", dtype);
+  const int ve = dtype == D2S_BF16 ? 8 : 4;
+  D2S_REQUIRE(B >= 0 && Nmax >= 1 && C >= 2 * ve && C % (2 * ve) == 0 && C / ve / 2 <= kPoolThreads, D2S_ERR_ARG,
+              "pool_concat_varlen_inplace: bad shape B=%d Nmax=%d C=%d", B, Nmax, C);
+  D2S_REQUIRE(aligned16(z), D2S_ERR_ALIGN, "pool_concat_varlen_inplace: z must be 16-byte aligned");
+  if (B == 0) return D2S_OK;
+  const int groups = kPoolThreads / (C / ve / 2);
+  const size_t smem = ((size_t)groups + 1) * (C / 2) * sizeof(float);
+  D2S_REQUIRE(smem <= 48 * 1024, D2S_ERR_ARG, "pool_concat_varlen_inplace: C=%d needs %zu B of shared memory", C, smem);
+  if (dtype == D2S_BF16)
+    pool_concat_inplace_kernel<__nv_bfloat16, true><<<B, kPoolThreads, smem, (cudaStream_t)stream>>>((__nv_bfloat16*)z, Nmax, C, n);
+  else
+    pool_concat_inplace_kernel<float, true><<<B, kPoolThreads, smem, (cudaStream_t)stream>>>((float*)z, Nmax, C, n);
+  count_launch();
+  return check_launch("d2s_pool_concat_varlen_inplace");
 }
 
 extern "C" int d2s_bias_act(void* u, const void* bias, int dtype, long long rows, int N, int C, int act, d2s_stream_t stream) {

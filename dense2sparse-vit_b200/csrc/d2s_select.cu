@@ -131,28 +131,38 @@ select_topk_kernel(const float* __restrict__ score, int N, int K, int order,
 // torch's CPU cumsum (acc_type<float> = double), the oracle's arithmetic -- and every token reads the prefix at its own rank.
 // Outputs: mask (B,N) uint8 0/1 (a torch.bool tensor's storage), count (B) int32 = kept tokens per image, kept (B,N) int64 =
 // the kept token indices in ascending order followed by -1 padding (the index list a varlen gather consumes); NULL to skip.
+// kVar (d2s_threshold_select_varlen_f32): image b selects among its first nv[b] scores of the N-wide row (the rest is never read);
+// mask / kept entries past nv[b] are 0 / -1.
+template <bool kVar>
 __global__ void __launch_bounds__(kSelThreads)
 threshold_select_kernel(const float* __restrict__ score, int N, float threshold, uint8_t* __restrict__ mask,
-                        int* __restrict__ count, int64_t* __restrict__ kept) {
+                        int* __restrict__ count, int64_t* __restrict__ kept, const int* __restrict__ nv) {
   __shared__ SelSmem s;
   __shared__ float sorted_s[kSelMaxN];
   __shared__ int total_s;
   const int b = blockIdx.x, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  const int Nv = kVar ? min(max(nv[b], 0), N) : N;   // valid scores of this image; N is the row pitch
+  if (kVar) {
+    for (int i = Nv + tid; i < N; i += kSelThreads) {
+      if (mask) mask[(size_t)b * N + i] = 0;
+      if (kept) kept[(size_t)b * N + i] = -1;
+    }
+  }
   float myv[kSelEPT];
   uint32_t mykey[kSelEPT];
 #pragma unroll
   for (int e = 0; e < kSelEPT; ++e) {
     const int i = e * kSelThreads + tid;
-    myv[e] = (i < N) ? score[(size_t)b * N + i] : 0.f;
+    myv[e] = (i < Nv) ? score[(size_t)b * N + i] : 0.f;
     mykey[e] = float_to_ordered(myv[e]);
-    if (i < N) s.key[i] = mykey[e];
+    if (i < Nv) s.key[i] = mykey[e];
   }
   __syncthreads();
   int rank[kSelEPT];
 #pragma unroll
   for (int e = 0; e < kSelEPT; ++e) rank[e] = 0;
-  const int nchunks = (N + kSelThreads - 1) / kSelThreads;
-  for (int j = 0; j < N; ++j) {
+  const int nchunks = (Nv + kSelThreads - 1) / kSelThreads;
+  for (int j = 0; j < Nv; ++j) {
     const uint32_t kj = s.key[j];  // broadcast read
 #pragma unroll
     for (int e = 0; e < kSelEPT; ++e)
@@ -160,11 +170,11 @@ threshold_select_kernel(const float* __restrict__ score, int N, float threshold,
   }
 #pragma unroll
   for (int e = 0; e < kSelEPT; ++e)
-    if (e * kSelThreads + tid < N) sorted_s[rank[e]] = myv[e];
+    if (e * kSelThreads + tid < Nv) sorted_s[rank[e]] = myv[e];
   __syncthreads();
   if (tid == 0) {
     double acc = 0.0;
-    for (int r = 0; r < N; ++r) {
+    for (int r = 0; r < Nv; ++r) {
       acc += (double)sorted_s[r];
       sorted_s[r] = (float)acc;
     }
@@ -174,8 +184,8 @@ threshold_select_kernel(const float* __restrict__ score, int N, float threshold,
 #pragma unroll
   for (int e = 0; e < kSelEPT; ++e) {
     const int i = e * kSelThreads + tid;
-    const bool keep = (i < N) && (sorted_s[rank[e]] > threshold);
-    if (i < N && mask) mask[(size_t)b * N + i] = keep ? 1 : 0;
+    const bool keep = (i < Nv) && (sorted_s[rank[e]] > threshold);
+    if (i < Nv && mask) mask[(size_t)b * N + i] = keep ? 1 : 0;
     ball[e] = __ballot_sync(0xffffffffu, keep);
     if (lane == 0) s.warp_cnt[e][warp] = __popc(ball[e]);
   }
@@ -192,7 +202,7 @@ threshold_select_kernel(const float* __restrict__ score, int N, float threshold,
 #pragma unroll
   for (int e = 0; e < kSelEPT; ++e) {
     const int i = e * kSelThreads + tid;
-    if (i >= N) continue;
+    if (i >= Nv) continue;
     int before = 0;
     for (int ee = 0; ee <= e; ++ee) {
       const int wend = (ee == e) ? warp : kSelWarps;
@@ -347,12 +357,14 @@ score_tail_a_kernel(const T_* __restrict__ hidden, int N, int C, const float* __
                      prev_kept ? prev_kept + (size_t)b * K : nullptr);
 }
 
-template <typename T_>
+// kVar (d2s_score_tail_b_varlen): image b has nv[b] valid rows of its N (padded) rows; the softmax runs over those only, pad rows
+// are never read, their scores are -inf and their probabilities 0 (no selection)
+template <typename T_, bool kVar = false>
 __global__ void __launch_bounds__(kSelThreads)
 score_tail_b_kernel(const T_* __restrict__ hidden, int N, int C, const float* __restrict__ ln_w,
                     const float* __restrict__ ln_b, float ln_eps, const float* __restrict__ W,
                     const float* __restrict__ bias_p, int prob_mode, int K, float* __restrict__ scores, float* __restrict__ probs,
-                    int64_t* __restrict__ kept, int64_t* __restrict__ dropped) {
+                    int64_t* __restrict__ kept, int64_t* __restrict__ dropped, const int* __restrict__ nv) {
   __shared__ SelSmem s;
   extern __shared__ float w_s[];  // gw[c] = ln_w[c]*W[c] (or W[c]),  then scalar sum(ln_b*W)
   const int b = blockIdx.x;
@@ -368,10 +380,11 @@ score_tail_b_kernel(const T_* __restrict__ hidden, int N, int C, const float* __
   // Phase 1 (four lanes per token row, see score_tail_a_kernel): raw scores into shared memory.
   const int quad = threadIdx.x >> 2, q4 = threadIdx.x & 3;
   const int nchunk = C / VE;
+  const int Nv = kVar ? min(max(nv[b], 0), N) : N;   // valid rows of this image; N is the row pitch
   float* sc_s = reinterpret_cast<float*>(s.key);   // scores live in the key array until they are turned into keys
-  for (int n0 = 0; n0 < N; n0 += kSelThreads / 4) {
+  for (int n0 = 0; n0 < Nv; n0 += kSelThreads / 4) {
     const int n = n0 + quad;
-    const T_* row = hidden + ((size_t)b * N + min(n, N - 1)) * C;
+    const T_* row = hidden + ((size_t)b * N + min(n, Nv - 1)) * C;
     float mean = 0.f, rstd = 1.f;
     if (ln_w) {
       float sum = 0.f;
@@ -402,7 +415,7 @@ score_tail_b_kernel(const T_* __restrict__ hidden, int N, int C, const float* __
     var += __shfl_xor_sync(0xffffffffu, var, 2);
     dot += __shfl_xor_sync(0xffffffffu, dot, 2);
     if (ln_w) rstd = rsqrtf(var / (float)C + ln_eps);
-    if (n < N && q4 == 0) {
+    if (n < Nv && q4 == 0) {
       const float val = dot * rstd + beta_dot + bias;
       sc_s[n] = val;
       scores[(size_t)b * N + n] = val;
@@ -414,7 +427,7 @@ score_tail_b_kernel(const T_* __restrict__ hidden, int N, int C, const float* __
 #pragma unroll
   for (int e = 0; e < kMaxPerThread; ++e) {
     const int n = e * kSelThreads + threadIdx.x;
-    sc[e] = (n < N) ? sc_s[n] : -INFINITY;
+    sc[e] = (n < Nv) ? sc_s[n] : -INFINITY;
     lmax = fmaxf(lmax, sc[e]);
   }
   __syncthreads();   // every score has been read before the key array is overwritten below
@@ -425,7 +438,7 @@ score_tail_b_kernel(const T_* __restrict__ hidden, int N, int C, const float* __
 #pragma unroll
     for (int e = 0; e < kMaxPerThread; ++e) {
       const int n = e * kSelThreads + threadIdx.x;
-      pr[e] = (n < N) ? expf(sc[e] - gmax) : 0.f;
+      pr[e] = (n < Nv) ? expf(sc[e] - gmax) : 0.f;
       lsum += pr[e];
     }
     const float gsum = block_reduce_sum(lsum, s);
@@ -438,9 +451,12 @@ score_tail_b_kernel(const T_* __restrict__ hidden, int N, int C, const float* __
 #pragma unroll
   for (int e = 0; e < kMaxPerThread; ++e) {
     const int n = e * kSelThreads + threadIdx.x;
-    if (n < N) {
+    if (n < Nv) {
       probs[(size_t)b * N + n] = pr[e];
       s.key[n] = float_to_ordered(pr[e]);
+    } else if (kVar && n < N) {
+      probs[(size_t)b * N + n] = 0.f;
+      scores[(size_t)b * N + n] = -INFINITY;
     }
   }
   if (kept == nullptr) return;
@@ -509,9 +525,19 @@ extern "C" int d2s_threshold_select_f32(const float* score, int B, int N, float 
   D2S_REQUIRE(score && (mask || kept || count), D2S_ERR_ARG, "threshold_select: null pointer");
   D2S_REQUIRE(B >= 0 && N >= 1 && N <= kSelMaxN, D2S_ERR_ARG, "threshold_select: N=%d outside [1,%d]", N, kSelMaxN);
   if (B == 0) return D2S_OK;
-  threshold_select_kernel<<<B, kSelThreads, 0, (cudaStream_t)stream>>>(score, N, threshold, mask, count, kept);
+  threshold_select_kernel<false><<<B, kSelThreads, 0, (cudaStream_t)stream>>>(score, N, threshold, mask, count, kept, nullptr);
   count_launch();
   return check_launch("d2s_threshold_select_f32");
+}
+
+extern "C" int d2s_threshold_select_varlen_f32(const float* score, const int* n, int B, int Nmax, float threshold, uint8_t* mask,
+                                              int* count, int64_t* kept, d2s_stream_t stream) {
+  D2S_REQUIRE(score && n && (mask || kept || count), D2S_ERR_ARG, "threshold_select_varlen: null pointer");
+  D2S_REQUIRE(B >= 0 && Nmax >= 1 && Nmax <= kSelMaxN, D2S_ERR_ARG, "threshold_select_varlen: Nmax=%d outside [1,%d]", Nmax, kSelMaxN);
+  if (B == 0) return D2S_OK;
+  threshold_select_kernel<true><<<B, kSelThreads, 0, (cudaStream_t)stream>>>(score, Nmax, threshold, mask, count, kept, n);
+  count_launch();
+  return check_launch("d2s_threshold_select_varlen_f32");
 }
 
 static int check_tail(const void* hidden, int dtype, int B, int N, int C, int K) {
@@ -559,12 +585,33 @@ extern "C" int d2s_score_tail_b(const void* hidden, int dtype, int B, int N, int
   const size_t smem = (size_t)C * sizeof(float);
   if (dtype == D2S_F32)
     score_tail_b_kernel<float><<<B, kSelThreads, smem, (cudaStream_t)stream>>>(
-        (const float*)hidden, N, C, ln_w, ln_b, ln_eps, W, bias, prob_mode, K, scores, probs, kept, dropped);
+        (const float*)hidden, N, C, ln_w, ln_b, ln_eps, W, bias, prob_mode, K, scores, probs, kept, dropped, nullptr);
   else
     score_tail_b_kernel<__nv_bfloat16><<<B, kSelThreads, smem, (cudaStream_t)stream>>>(
-        (const __nv_bfloat16*)hidden, N, C, ln_w, ln_b, ln_eps, W, bias, prob_mode, K, scores, probs, kept, dropped);
+        (const __nv_bfloat16*)hidden, N, C, ln_w, ln_b, ln_eps, W, bias, prob_mode, K, scores, probs, kept, dropped, nullptr);
   count_launch();
   return check_launch("d2s_score_tail_b");
+}
+
+extern "C" int d2s_score_tail_b_varlen(const void* hidden, const int* n, int dtype, int B, int Nmax, int C, const float* ln_w,
+                                       const float* ln_b, float ln_eps, const float* W, const float* bias, int prob_mode, float* scores,
+                                       float* probs, d2s_stream_t stream) {
+  D2S_REQUIRE(n, D2S_ERR_ARG, "score_tail_b_varlen: null n");
+  int rc = check_tail(hidden, dtype, B, Nmax, C, 0);
+  if (rc) return rc;
+  D2S_REQUIRE(W && scores && probs, D2S_ERR_ARG, "score_tail_b_varlen: null W/scores/probs");
+  D2S_REQUIRE((ln_w == nullptr) == (ln_b == nullptr), D2S_ERR_ARG, "score_tail_b_varlen: ln_w and ln_b must both be set or both NULL");
+  D2S_REQUIRE(prob_mode == D2S_PROB_SOFTMAX || prob_mode == D2S_PROB_SIGMOID, D2S_ERR_ARG, "score_tail_b_varlen: bad prob_mode");
+  if (B == 0) return D2S_OK;
+  const size_t smem = (size_t)C * sizeof(float);
+  if (dtype == D2S_F32)
+    score_tail_b_kernel<float, true><<<B, kSelThreads, smem, (cudaStream_t)stream>>>(
+        (const float*)hidden, Nmax, C, ln_w, ln_b, ln_eps, W, bias, prob_mode, 0, scores, probs, nullptr, nullptr, n);
+  else
+    score_tail_b_kernel<__nv_bfloat16, true><<<B, kSelThreads, smem, (cudaStream_t)stream>>>(
+        (const __nv_bfloat16*)hidden, Nmax, C, ln_w, ln_b, ln_eps, W, bias, prob_mode, 0, scores, probs, nullptr, nullptr, n);
+  count_launch();
+  return check_launch("d2s_score_tail_b_varlen");
 }
 
 extern "C" int d2s_gumbel_decision_f32(const float* logp, const float* gumbel, const float* prev, int64_t n,

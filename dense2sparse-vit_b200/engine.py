@@ -113,8 +113,9 @@ def _qkv_pair_ok(lin, x):
             and lin.out_features % 192 == 0 and lin.out_features % 256 != 0)
 
 
-def attention_pre_proj(m, x, policy=None, return_cls_attn=False):
-    """Attention.forward up to (not including) the output projection (dynamic_vit.py:216-231): (o (B,T,C), cls_attn)."""
+def attention_pre_proj(m, x, policy=None, return_cls_attn=False, lens=None):
+    """Attention.forward up to (not including) the output projection (dynamic_vit.py:216-231): (o (B,T,C), cls_attn).
+    lens (B) int32: a padded batch (image b = its first lens[b] tokens), run by the variable-length attention kernel."""
     B, T, C = x.shape
     H = m.num_heads
     lin = m.qkv
@@ -133,6 +134,12 @@ def attention_pre_proj(m, x, policy=None, return_cls_attn=False):
         qkv = ops.linear_act(x, lin.weight, lin.bias, ops.ACT_NONE)
     else:
         qkv = ops.linear_train(lin, x)
+    if lens is not None:
+        if _needs_grad(qkv) or not qkv.is_cuda or not _attn_kernel_ok(qkv, H) or policy is not None:
+            raise RuntimeError("variable-length attention: inference only, no policy, CUDA qkv of a shape the d2s attention kernels "
+                               f"take (bf16 with head dim 64 or fp32 with head dim 32 / 64, T <= 256); got {tuple(qkv.shape)} {qkv.dtype}")
+        o, cls_attn = ops.attention_core(qkv, H, scale=m.scale, want_cls_row=return_cls_attn, lengths=lens)
+        return o, (cls_attn.to(qkv.dtype) if cls_attn is not None else None)
     if _needs_grad(qkv, policy) and qkv.is_cuda and qkv.dtype == torch.bfloat16 and T <= 256 and _TRAIN_ATTN:
         # training, bf16: the tcgen05 flash forward / backward pair on the packed tensor (T <= 208, hd 64), else per-head GEMMs
         # on a head-major copy around the padded-row policy softmax
@@ -279,13 +286,17 @@ class _Stream:
     """Residual stream of the model-level inference loops: x plus a pending branch (x + branch is the value the reference
     holds in `x`).  The branch is either a tensor y or a deferred Linear `lin = (a, module)` (attn.proj / mlp.fc2), so
     that the next consumer can run it as ONE kernel with the residual add and its LayerNorm (ops.linear_residual_ln).
-    Falls back to plain Block.forward when the fused path does not apply."""
+    Falls back to plain Block.forward when the fused path does not apply.
+    Padded batches (threshold inference): `lens` (B) int32 on the device counts each image's valid tokens (CLS included) of the
+    stream's T rows, None when every image has all T.  Rows lens[b].. are pad rows: the variable-length gather writes them as zeros,
+    later kernels keep them finite and no valid row depends on them (attention masks them; everything else works row by row)."""
 
     def __init__(self, x, asm=None):
         # asm = (patches, cls_token, pos_embed): the token assembly itself is deferred, so that it runs fused with the first
         # block's norm1 (ops.assemble_layernorm); any other access to .x materialises it with the plain assembly kernel
         self._x, self._asm = x, asm
         self.y, self.lin, self.mlp, self.gidx = None, None, None, None
+        self.gcount, self.lens = None, None
 
     @property
     def x(self):
@@ -309,13 +320,18 @@ class _Stream:
             return torch.Size((B, N + 1, D))
         return self._x.shape
 
-    def gather(self, x, kept):
+    def gather(self, x, kept, counts=None):
         """The pruning stage's kept-token gather (default_dynamic_vit.py:464-468, dynamic_vit.py:907-912), deferred so that it
-        runs fused with the next block's norm1 (ops.gather_layernorm)."""
+        runs fused with the next block's norm1 (ops.gather_layernorm).  counts (B) int32: image b keeps kept[b, :counts[b]] (the
+        threshold inference, dynamic_vit.py:954-960); the stream becomes a padded batch of lengths counts + 1."""
         self.x, self.y, self.lin, self.mlp, self.gidx = x, None, None, None, kept
+        self.gcount, self.lens = counts, (None if counts is None else counts + 1)
 
     def _flush_gather(self):
         if self.gidx is not None:
+            if self.gcount is not None:
+                raise RuntimeError("the variable-length gather runs fused with the next block's norm1 (ops.gather_layernorm): "
+                                   "the block after a threshold stage must take the fused inference path")
             self.x, self.gidx = ops.gather_tokens(self.x, self.gidx, prepend_cls=True), None
 
     def _flush_lin(self):
@@ -346,11 +362,11 @@ class _Stream:
             return self._x, h
         if self.gidx is not None:
             if row0 == 0 and self.x.dtype in (torch.float32, torch.bfloat16):
-                (x, kept), self.gidx = (self.x, self.gidx), None
+                (x, kept, counts), self.gidx, self.gcount = (self.x, self.gidx, self.gcount), None, None
                 if lazy and x.dtype == torch.bfloat16:
-                    self.x, st = ops.gather_layernorm(x, kept, norm.weight, norm.bias, norm.eps, want_stats=True)
+                    self.x, st = ops.gather_layernorm(x, kept, norm.weight, norm.bias, norm.eps, want_stats=True, counts=counts)
                     return self.x, _LazyNorm(self.x, st, norm)
-                self.x, h = ops.gather_layernorm(x, kept, norm.weight, norm.bias, norm.eps)
+                self.x, h = ops.gather_layernorm(x, kept, norm.weight, norm.bias, norm.eps, counts=counts)
                 return self.x, h
             self._flush_gather()
         if self.mlp is not None:
@@ -416,7 +432,7 @@ class _Stream:
             lazy1 = (_LAZY_NORM1 and _is_plain_ln(blk.norm1) and blk.norm1.weight.dtype == torch.bfloat16
                      and _qkv_pair_ok(blk.attn.qkv, self._probe()))
             _, h = self._sum_norm(blk.norm1, lazy=lazy1)
-            o, cls_attn = attention_pre_proj(blk.attn, h, policy, return_cls_attn)
+            o, cls_attn = attention_pre_proj(blk.attn, h, policy, return_cls_attn, lens=self.lens)
             self.lin = (o, blk.attn.proj)
             # norm2 is only ever read by this block's MLP: when that MLP runs as the one kernel, hand it the statistics
             lazy = (_LAZY_NORM2 and _mlp_is_plain(blk.mlp, o) and _mlp_fused_ok(blk.mlp, o, o) and o.shape[-1] == 384
@@ -427,6 +443,9 @@ class _Stream:
             else:
                 self.y = blk.mlp(_norm_value(h))
             return cls_attn
+        if self.lens is not None:
+            raise RuntimeError("a padded (variable-length) batch runs on the fused inference path only: CUDA, float32 / bfloat16, "
+                               "plain LayerNorms, no stochastic depth or active dropout")
         if _train_fusable(blk, self.x, self.y):
             return self._block_train(blk, policy, return_cls_attn)
         out = block_forward(blk, self.value(), policy, return_cls_attn)
@@ -680,6 +699,26 @@ def predictor_b_forward(m, x, policy=None, current_sigma=0.0005, cls_attn=None, 
     return scores, probs, kept, dropped
 
 
+def predictor_b_varlen(m, x, n):
+    """Variant B's PredictorLG.forward at inference (dynamic_vit.py:536-554) over a padded batch: x (B,Nmax,D) spatial tokens of
+    which image b has n[b] (int32, device).  The mean pool and the softmax run over each image's valid rows only (the varlen pool
+    and tail kernels); every other layer works row by row.  Returns (scores, keep probabilities) (B,Nmax); pad entries are -inf / 0."""
+    if not m.topk_selection:
+        raise RuntimeError("PredictorLG is only defined for topk_selection=True (dynamic_vit.py:537)")
+    h = ops.pool_concat_varlen_(_seq_forward(m.in_conv, x).contiguous(), n)
+    body, norm, lin = _predictor_b_tail_parts(m)
+    h = _seq_forward(body, h)
+    if not _tail_ok(h):
+        raise RuntimeError(f"predictor width {h.shape[-1]} is outside the d2s tail kernel (multiples of 8 in [8, 1024])")
+    prob_mode = ops.PROB_SOFTMAX if m.loss_type in ["kl_div", "mse"] else ops.PROB_SIGMOID
+    if isinstance(norm, torch.nn.LayerNorm):
+        ln_w, ln_b, ln_eps = norm.weight, norm.bias, norm.eps
+    else:  # BatchNormLayer (eval: a per-channel affine map, row by row): normalise upstream, the kernel then skips its LayerNorm
+        h, ln_w, ln_b, ln_eps = norm(h), None, None, 0.0
+    scores, probs = ops.score_tail_b_varlen(h, n, ln_w, ln_b, lin.weight, lin.bias, ln_eps, prob_mode)
+    return scores.to(x.dtype), probs.to(x.dtype)
+
+
 # ---- model forwards ------------------------------------------------------------------------------------
 def _embed_stream(model, img):
     """The residual stream after patch embedding; on the inference path the token assembly is left pending (fused with the first
@@ -779,6 +818,13 @@ def variant_a_forward(model, img):
 
 def variant_b_forward(model, img, stacked_cls_attn_weights=None):
     """VisionTransformerDiffPruning.forward (dynamic_vit.py:814-1015)."""
+    if (model.patch_score_threshold is not None and not model.training
+            and (_THRESHOLD_INFERENCE or getattr(model, "d2s_threshold_inference", False))):
+        # OPT-IN.  The reference's inference branch of this mode cannot run (dynamic_vit.py:936 reads `score`, which is only
+        # assigned in a comment at :933, and :947 indexes with a float mask).  What it evidently intends -- the same cumulative-score
+        # threshold on pred_score, then a variable-length removal of the dropped tokens, batch size 1 by design
+        # (mask_predictor.py:249-254) -- is the equal-count case of the padded-batch forward (forward_varlen)
+        return _variant_b_threshold_eval(model, img, ragged=False)
     st = _embed_stream(model, img)
     B, T0, D = st.shape
     dt, dev = st._probe().dtype, st._probe().device
@@ -834,27 +880,6 @@ def variant_b_forward(model, img, stacked_cls_attn_weights=None):
                 model.dropped_token_indices.append(~spatial_mask.unsqueeze(-1).repeat(1, 1, D).flatten())
                 keep_mask = torch.cat((torch.ones(B, 1, dtype=dt, device=dev), spatial_mask), dim=1).float()
                 st.block(blk, policy=keep_mask.unsqueeze(-1))
-            elif _THRESHOLD_INFERENCE or getattr(model, "d2s_threshold_inference", False):
-                # OPT-IN.  The reference's inference branch of this mode cannot run (dynamic_vit.py:936 reads `score`, which
-                # is only assigned in a comment at :933, and :947 indexes with a float mask).  What it evidently intends -- the
-                # same cumulative-score threshold on pred_score, then a variable-length removal of the dropped tokens, batch
-                # size 1 by design (mask_predictor.py:249-254) -- runs here as: prefix-sum select kernel -> kept index list,
-                # one host read of the kept count (the output shape depends on it, as in the reference's boolean indexing),
-                # gather of CLS + kept tokens fused with the block's norm1.
-                x = st.value()
-                pred_logits, pred_score = predictor_b_forward(pred, x[:, 1:])
-                spatial_mask, kept_count, kept_pad = ops.threshold_select(pred_score.detach(), thr, want_indices=True)
-                counts = kept_count.tolist()
-                if len(set(counts)) != 1:
-                    raise RuntimeError(f"patch_score_threshold inference: images keep different token counts {counts}; like the "
-                                       "reference's x.flatten()[mask].reshape(B, -1, D) this mode is for batch size 1")
-                model.keep_ratios = kept_count.to(torch.float32) / N
-                model.min_keep_ratio = model.avg_keep_ratio = model.max_keep_ratio = counts[0] / N
-                kept = kept_pad[:, :counts[0]].contiguous()
-                model.kept_token_indices.append(kept)
-                model.pred_logits.append(pred_logits)
-                st.gather(x, kept)
-                st.block(blk)
             else:
                 # the reference's inference branch of this mode reads an undefined name (dynamic_vit.py:936)
                 raise NotImplementedError("patch_score_threshold inference is undefined in the reference "
@@ -874,6 +899,64 @@ def variant_b_forward(model, img, stacked_cls_attn_weights=None):
         return x, features, model.pred_logits, model.kept_token_indices
     logits = model.head(model.pre_logits(st.cls_normed(model.norm)))
     return logits, model.cls_attns, model.pred_logits, model.kept_token_indices
+
+
+def _variant_b_threshold_eval(model, img, ragged):
+    """Inference of the dynamic keep-ratio mode (what dynamic_vit.py:935-960 intends) over a padded batch: at each pruning stage
+    the predictor scores the valid tokens, the prefix-sum select kernel picks each image's kept set (ascending, -1 padded), ONE host
+    read of the per-image counts sizes the next stage (Tmax = 1 + max count), and the gather of CLS + kept tokens runs fused with
+    the block's norm1; the stream then carries per-image lengths that the attention kernel honours.  The pruning block and the
+    later ones run without a policy.  ragged=False: forward()'s dense outputs, which need equal counts (batch size 1).
+    Returns (logits, cls_attns, pred_logits, kept): cls_attns of the blocks that are not pruning stages (B,H,Tmax_i-1), zero past
+    an image's tokens; pred_logits (B,Nmax_s), -inf past them; kept (B,Kmax_s) int64 stage-relative ascending, -1 padded."""
+    thr = model.patch_score_threshold
+    st = _embed_stream(model, img)
+    B, T0, _ = st.shape
+    N = T0 - 1
+    model.num_kept_tokens = []
+    model.cls_attns = []
+    model.pred_logits = []
+    model.kept_token_indices = []
+    model.dropped_token_indices = []
+    n = None                                       # valid spatial tokens per image (B) int32 on the device
+    p_count = 0
+    for i, blk in enumerate(model.blocks):
+        if i in model.pruning_loc:
+            x = st.value()
+            if n is None:
+                n = torch.full((B,), x.shape[1] - 1, dtype=torch.int32, device=x.device)
+            pred_logits, pred_score = predictor_b_varlen(model.score_predictor[p_count], x[:, 1:], n)
+            _, count, kept = ops.threshold_select(pred_score.detach(), thr, want_indices=True, lengths=n)
+            counts = count.tolist()                # the stage's one host read: the output shape depends on it
+            if not ragged and len(set(counts)) != 1:
+                raise RuntimeError(f"patch_score_threshold inference: images keep different token counts {counts}; like the "
+                                   "reference's x.flatten()[mask].reshape(B, -1, D) forward() is for batch size 1 here -- "
+                                   "model.forward_varlen(x) runs such a batch (padded outputs)")
+            model.keep_ratios = count.to(torch.float32) / N
+            model.min_keep_ratio, model.max_keep_ratio = min(counts) / N, max(counts) / N
+            model.avg_keep_ratio = sum(counts) / len(counts) / N
+            kept = kept[:, :max(counts)].contiguous()
+            model.kept_token_indices.append(kept)
+            model.pred_logits.append(pred_logits)
+            st.gather(x, kept, count)
+            n = count
+            st.block(blk)
+            p_count += 1
+        else:
+            cls_attn = st.block(blk, return_cls_attn=True)
+            model.cls_attns.append(cls_attn[:, :, 1:])
+    logits = model.head(model.pre_logits(st.cls_normed(model.norm)))
+    return logits, model.cls_attns, model.pred_logits, model.kept_token_indices
+
+
+def variant_b_forward_varlen(model, img):
+    """VisionTransformerDiffPruning.forward_varlen: the dynamic keep-ratio inference of a whole batch in which images keep
+    different token counts (padded outputs, see _variant_b_threshold_eval)."""
+    if model.training:
+        raise ValueError("forward_varlen is an inference path: call model.eval() first (training uses the keep-mask policy)")
+    if model.patch_score_threshold is None:
+        raise ValueError("forward_varlen runs the dynamic keep-ratio mode: the model has no patch_score_threshold")
+    return _variant_b_threshold_eval(model, img, ragged=True)
 
 
 def variant_b_forward_cls_attn(model, img):

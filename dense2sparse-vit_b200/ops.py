@@ -86,18 +86,50 @@ def select_topk(score: torch.Tensor, k: int, order: int = ORDER_INDEX_ASC, want_
     return kept, dropped
 
 
-def threshold_select(score, threshold, want_indices=False):
+def _lengths(lengths, B, what):
+    """Per-image valid lengths of a padded (B, n_max, ...) tensor as the int32 device vector the varlen kernels read."""
+    _check_cuda(lengths)
+    if lengths.dim() != 1 or lengths.shape[0] != B:
+        raise ValueError(f"{what}: lengths must be a (B={B},) vector, got shape {tuple(lengths.shape)}")
+    return lengths.to(torch.int32).contiguous()
+
+
+def threshold_select(score, threshold, want_indices=False, lengths=None):
     """Dynamic keep-ratio selection (vit_models/dynamic_vit.py:880-890, :935-945): tokens whose cumulative ascending-sorted
     score mass exceeds `threshold` are kept.  score (B,N) -> (mask (B,N) bool, count (B) int32[, kept (B,N) int64: the kept
-    indices in ascending order, then -1 padding])."""
+    indices in ascending order, then -1 padding]).
+    lengths (B) int: image b selects among its first lengths[b] scores only (a padded batch); entries past it are never read,
+    their mask is False and their kept entry -1."""
     _check_cuda(score)
     s = _f32c(score)
     B, N = s.shape
     mask = torch.empty(B, N, dtype=torch.bool, device=s.device)
     count = torch.empty(B, dtype=torch.int32, device=s.device)
     kept = torch.empty(B, N, dtype=torch.int64, device=s.device) if want_indices else None
-    _call("d2s_threshold_select_f32", _ptr(s), B, N, float(threshold), _ptr(mask), _ptr(count), _ptr(kept), _stream(s))
+    if lengths is None:
+        _call("d2s_threshold_select_f32", _ptr(s), B, N, float(threshold), _ptr(mask), _ptr(count), _ptr(kept), _stream(s))
+    else:
+        n = _lengths(lengths, B, "threshold_select")
+        _call("d2s_threshold_select_varlen_f32", _ptr(s), _ptr(n), B, N, float(threshold), _ptr(mask), _ptr(count), _ptr(kept),
+              _stream(s))
     return (mask, count, kept) if want_indices else (mask, count)
+
+
+def score_tail_b_varlen(hidden, lengths, ln_weight, ln_bias, weight, bias, ln_eps=1e-5, prob_mode=PROB_SOFTMAX):
+    """score_tail_b without selection over a padded batch: image b's rows are hidden[b, :lengths[b]].  The softmax runs over
+    those rows only; pad rows are never read, their scores are -inf and their probabilities 0.  Returns (scores, probs) (B,N)."""
+    _check_cuda(hidden, weight)
+    h = _as_kernel_float(hidden.detach()).contiguous()
+    B, N, C = h.shape
+    n = _lengths(lengths, B, "score_tail_b_varlen")
+    lw, lb = _f32c(ln_weight), _f32c(ln_bias)
+    w = _f32c(weight).reshape(-1)
+    bz = _f32c(bias).reshape(-1) if bias is not None else None
+    scores = torch.empty(B, N, dtype=torch.float32, device=h.device)
+    probs = torch.empty(B, N, dtype=torch.float32, device=h.device)
+    _call("d2s_score_tail_b_varlen", _ptr(h), _ptr(n), _dtype_code(h), B, N, C, _ptr(lw), _ptr(lb), float(ln_eps), _ptr(w),
+          _ptr(bz), prob_mode, _ptr(scores), _ptr(probs), _stream(h))
+    return scores, probs
 
 
 def score_tail_a(hidden, weight, bias, k=0, gumbel=None, prev=None, act_input=ACT_NONE, want_prev_kept=False):
@@ -782,19 +814,28 @@ def attention_train(qkv, num_heads, policy=None, scale=None, eps=1e-6, want_cls_
     return _AttentionTrain.apply(qkv, policy, num_heads, float(scale), float(eps), bool(want_cls_row))
 
 
-def attention_core(qkv, num_heads, policy=None, scale=None, eps=1e-6, want_cls_row=False):
+def attention_core(qkv, num_heads, policy=None, scale=None, eps=1e-6, want_cls_row=False, lengths=None):
     """Fused inference attention: packed qkv (B,T,3*H*hd) straight from the qkv Linear -> (out (B,T,H*hd),
     cls_row (B,H,T) fp32 | None).  bf16 runs the tcgen05/TMEM kernel, fp32 the SIMT parity kernel.
-    No autograd: the training path uses softmax_with_policy around library GEMMs."""
+    No autograd: the training path uses softmax_with_policy around library GEMMs.
+    lengths (B) int: a padded batch, image b is its first lengths[b] tokens (keys and queries); out rows and cls_row columns
+    past it are zeros.  No policy in that form."""
     _check_cuda(qkv, policy)
     q = qkv.detach().contiguous()
     B, T, C3 = q.shape
     D = C3 // 3
     hd = D // num_heads
     scale = hd ** -0.5 if scale is None else scale
-    pol = _f32c(policy.reshape(B, T)) if policy is not None else None
     out = torch.empty(B, T, D, dtype=q.dtype, device=q.device)
     cls_row = torch.empty(B, num_heads, T, dtype=torch.float32, device=q.device) if want_cls_row else None
+    if lengths is not None:
+        if policy is not None:
+            raise ValueError("attention_core: the variable-length form takes no policy")
+        n = _lengths(lengths, B, "attention_core")
+        _call("d2s_attn_varlen_fwd", _ptr(q), _ptr(n), _dtype_code(q), B, T, num_heads, hd, float(scale), _ptr(out), _ptr(cls_row),
+              _stream(q))
+        return out, cls_row
+    pol = _f32c(policy.reshape(B, T)) if policy is not None else None
     _call("d2s_attn_policy_fwd", _ptr(q), _ptr(pol), _dtype_code(q), B, T, num_heads, hd, float(scale), float(eps),
               _ptr(out), _ptr(cls_row), None, _stream(q))
     return out, cls_row
@@ -839,28 +880,38 @@ def layernorm_from_stats(x, stats, weight, bias, rows_per_image=1):
     return out
 
 
-def gather_layernorm(x, kept, weight, bias, eps, want_stats=False):
+def gather_layernorm(x, kept, weight, bias, eps, want_stats=False, counts=None):
     """(xg, LayerNorm(xg)) with xg = [CLS, x[:, kept + 1]]: the kept-token gather of the pruning stage fused with the next
     block's norm1 (vit_models/default_dynamic_vit.py:464-468, dynamic_vit.py:907-912 + :263).  Inference only.
-    want_stats (bf16): (xg, stats (B*(K+1), 2) f32 = per-row (mean, rstd)) instead; the consumer applies the LayerNorm."""
-    _check_cuda(x, kept, weight, bias)
+    want_stats (bf16): (xg, stats (B*(K+1), 2) f32 = per-row (mean, rstd)) instead; the consumer applies the LayerNorm.
+    counts (B) int: a variable-length gather, image b keeps kept[b, :counts[b]] (the rest of the row is padding, never read);
+    output rows 1 + counts[b] .. K are zeros (both outputs), their stats those of a zero row."""
+    _check_cuda(x, kept, weight, bias, counts)
     if kept.dtype != torch.int64:
         raise TypeError("indices must be int64")
     xc, ic = x.detach().contiguous(), kept.contiguous()
     B, T, D = xc.shape
     K = ic.shape[1]
+    n = None if counts is None else _lengths(counts, B, "gather_layernorm")
     if want_stats:
         if xc.dtype != torch.bfloat16:
             raise TypeError("gather_layernorm(want_stats=True) is a bf16 path")
         out_sum = torch.empty(B, K + 1, D, dtype=xc.dtype, device=xc.device)
         stats = torch.empty(B * (K + 1), 2, dtype=torch.float32, device=xc.device)
-        if B:
+        if B and n is None:
             _call("d2s_gather_layernorm_stats", _ptr(xc), _ptr(ic), B, T, D, K, float(eps), _ptr(out_sum), _ptr(stats), _stream(xc))
+        elif B:
+            _call("d2s_gather_layernorm_stats_varlen", _ptr(xc), _ptr(ic), _ptr(n), B, T, D, K, float(eps), _ptr(out_sum), _ptr(stats),
+                  _stream(xc))
         return out_sum, stats
     w, b = weight.detach().to(xc.dtype).contiguous(), bias.detach().to(xc.dtype).contiguous()
     out_sum = torch.empty(B, K + 1, D, dtype=xc.dtype, device=xc.device)
     out_norm = torch.empty_like(out_sum)
-    _call("d2s_gather_layernorm", _ptr(xc), _ptr(ic), _ptr(w), _ptr(b), _dtype_code(xc), B, T, D, K, float(eps),
+    if n is None:
+        _call("d2s_gather_layernorm", _ptr(xc), _ptr(ic), _ptr(w), _ptr(b), _dtype_code(xc), B, T, D, K, float(eps),
+              _ptr(out_sum), _ptr(out_norm), _stream(xc))
+    else:
+        _call("d2s_gather_layernorm_varlen", _ptr(xc), _ptr(ic), _ptr(n), _ptr(w), _ptr(b), _dtype_code(xc), B, T, D, K, float(eps),
               _ptr(out_sum), _ptr(out_norm), _stream(xc))
     return out_sum, out_norm
 
@@ -1072,6 +1123,18 @@ def pool_concat_(z):
         raise ValueError("pool_concat_ works in place on a contiguous tensor")
     B, N, C = z.shape
     _call("d2s_pool_concat_inplace", _ptr(z), _dtype_code(z), B, N, C, _stream(z))
+    return z
+
+
+def pool_concat_varlen_(z, lengths):
+    """pool_concat_ over a padded batch: image b's mean runs over z[b, :lengths[b]] and is written into those rows only; pad
+    rows are neither read nor written."""
+    _check_cuda(z)
+    if not z.is_contiguous():
+        raise ValueError("pool_concat_varlen_ works in place on a contiguous tensor")
+    B, N, C = z.shape
+    n = _lengths(lengths, B, "pool_concat_varlen_")
+    _call("d2s_pool_concat_varlen_inplace", _ptr(z), _ptr(n), _dtype_code(z), B, N, C, _stream(z))
     return z
 
 

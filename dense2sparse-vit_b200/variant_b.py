@@ -113,6 +113,13 @@ class VisionTransformerDiffPruning(_VitBackbone):
     def forward_cls_attn(self, x):
         return engine.variant_b_forward_cls_attn(self, x)
 
+    def forward_varlen(self, x):
+        """Dynamic keep-ratio inference (patch_score_threshold set, eval mode) of a batch whose images keep different token counts:
+        (logits (B, classes), cls_attns, pred_logits, kept) in forward()'s eval order, ragged entries padded -- kept[s] (B,Kmax_s)
+        int64 stage-relative ascending with -1, pred_logits[s] (B,Nmax_s) with -inf, cls_attns[i] (B,H,Tmax_i-1) with zeros.
+        Sets keep_ratios (per image) and min / avg / max_keep_ratio of the last stage."""
+        return engine.variant_b_forward_varlen(self, x)
+
 
 class VisionTransformerTeacher(_VitBackbone):
     """dynamic_vit.py:1036-1176: unpruned ViT returning (logits, tokens, cls_attn (B,depth,H,T))."""

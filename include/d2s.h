@@ -62,6 +62,41 @@ int d2s_select_topk_f32(const float* score, int B, int N, int K, int order,
 int d2s_threshold_select_f32(const float* score, int B, int N, float threshold, uint8_t* mask, int* count, int64_t* kept,
                              d2s_stream_t stream);
 
+/* ---- variable-length (padded) form of the dynamic keep-ratio inference ----------------------------------------------------
+ * The inference branch of the threshold mode (dynamic_vit.py:935-960: threshold select, then x.flatten()[mask].reshape(B, -1, D))
+ * keeps a different number of tokens per image.  Batched, a stage's tokens are PADDED: x (B,Tmax,D) plus a device length per
+ * image (len (B) int32, CLS included); rows len[b]..Tmax-1 are pad rows, written as zeros by the varlen gather and finite (but
+ * otherwise unspecified) after it; no valid output depends on them.  Lengths are read on the device (one value per image, clamped
+ * to [0, Tmax]); the kernels are the dense ones compiled with the per-image length.
+ *
+ * d2s_threshold_select_varlen_f32: d2s_threshold_select_f32 on each image's prefix score[b, :n[b]] (score (B,Nmax) f32, n (B)
+ * int32); entries past n[b] are never read, their mask is 0 and their kept entry -1.  Replaces dynamic_vit.py:935-945. */
+int d2s_threshold_select_varlen_f32(const float* score, const int* n, int B, int Nmax, float threshold, uint8_t* mask, int* count,
+                                    int64_t* kept, d2s_stream_t stream);
+/* d2s_score_tail_b_varlen: the Variant B tail of d2s_score_tail_b without selection (dynamic_vit.py:547-554) over the first n[b]
+ * rows of hidden (B,Nmax,C); the softmax runs over those rows only; pad rows are never read, their scores are -inf and their
+ * probabilities 0. */
+int d2s_score_tail_b_varlen(const void* hidden, const int* n, int dtype, int B, int Nmax, int C, const float* ln_w, const float* ln_b,
+                            float ln_eps, const float* W, const float* bias, int prob_mode, float* scores, float* probs,
+                            d2s_stream_t stream);
+/* d2s_pool_concat_varlen_inplace: d2s_pool_concat_inplace with the mean over each image's first n[b] rows (dynamic_vit.py:539-545
+ * with padding), written into those rows; pad rows are neither read nor written. */
+int d2s_pool_concat_varlen_inplace(void* z, const int* n, int dtype, int B, int Nmax, int C, d2s_stream_t stream);
+/* d2s_attn_varlen_fwd: Attention.forward's core (dynamic_vit.py:218-234) over the first len[b] tokens of every image, no policy:
+ * qkv (B,Tmax,3,H,hd), out (B,Tmax,H*hd), cls_row (B,H,Tmax) f32 or NULL; out rows and cls_row columns >= len[b] are zeros.
+ * BF16: the tcgen05 kernel of d2s_attn_policy_fwd (hd == 64), F32: its SIMT parity kernel (hd in {32,64}).  Tmax <= 256; the kernel
+ * template is chosen from Tmax.  Valid rows are bit-identical to d2s_attn_policy_fwd run on the image alone when len[b] and Tmax
+ * are on the same side of 128. */
+int d2s_attn_varlen_fwd(const void* qkv, const int* len, int dtype, int B, int Tmax, int H, int hd, float scale, void* out,
+                        float* cls_row, d2s_stream_t stream);
+/* d2s_gather_layernorm_varlen / d2s_gather_layernorm_stats_varlen: d2s_gather_layernorm / _stats (dynamic_vit.py:954-960 + the next
+ * block's norm1) with idx (B,Kmax) holding image b's count[b] kept spatial indices, then padding that is never read (-1 from the
+ * select); output rows 1 + count[b] .. Kmax are zeros (out_sum and out_norm), their stats the (mean, rstd) of a zero row. */
+int d2s_gather_layernorm_varlen(const void* x, const int64_t* idx, const int* count, const void* gamma, const void* beta, int dtype,
+                                int B, int T_in, int D, int Kmax, float eps, void* out_sum, void* out_norm, d2s_stream_t stream);
+int d2s_gather_layernorm_stats_varlen(const void* x, const int64_t* idx, const int* count, int B, int T_in, int D, int Kmax, float eps,
+                                      void* out_sum, float* stats, d2s_stream_t stream);
+
 /* ---- (1b) fused predictor tails -----------------------------------------------------------------
  * Variant A tail: Linear(C,2)+LogSoftmax (default_dynamic_vit.py:319-320), then either
  *   eval : top-K of logp[:,:,0] in descending-score order (default_dynamic_vit.py:461-463)  -> kept
