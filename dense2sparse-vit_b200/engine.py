@@ -33,6 +33,7 @@ _QKV_PAIR = os.environ.get("D2S_QKV_PAIR", "1") != "0"     # A/B switch: inferen
 _PRED_FUSED = os.environ.get("D2S_PRED_FUSED", "1") != "0"  # A/B switch: second half of the Variant A predictor + selection as one tcgen05 kernel (inference, D = 384)
 _POOL_TRAIN = os.environ.get("D2S_POOL_TRAIN", "1") != "0"  # A/B switch: the predictors' local/global split as one kernel each way
 _THRESHOLD_INFERENCE = os.environ.get("D2S_THRESHOLD_INFERENCE", "0") == "1"   # opt-in: what dynamic_vit.py:935-949 intends
+_LONG_ATTN = os.environ.get("D2S_LONG_ATTN", "1") != "0"    # A/B switch: bf16 inference attention beyond 256 tokens on the key-blocked kernel
 INIT_N = 14 * 14  # the reference hard-codes 196 spatial tokens (dynamic_vit.py:828, default_dynamic_vit.py:446)
 
 
@@ -54,10 +55,13 @@ def _ln_rows_ok(x):
 
 
 def _attn_kernel_ok(qkv, H):
-    """Shapes of d2s_attn_policy_fwd: bf16 -> tcgen05 kernel (hd 64), fp32 -> SIMT kernel (hd 32 / 64); T <= 256."""
+    """Shapes of the fused attention kernels: bf16 -> tcgen05 kernel (hd 64), fp32 -> SIMT kernel (hd 32 / 64), T <= 256; and bf16,
+    hd 64, 256 < T <= 2048 -> the key-blocked tcgen05 kernel (d2s_attn_long_fwd) unless D2S_LONG_ATTN=0."""
     hd = qkv.shape[-1] // 3 // H
-    if qkv.shape[1] > 256 or qkv.shape[-1] != 3 * H * hd:
+    if qkv.shape[-1] != 3 * H * hd:
         return False
+    if qkv.shape[1] > 256:
+        return _LONG_ATTN and qkv.dtype == torch.bfloat16 and hd == 64 and qkv.shape[1] <= ops.LONG_ATTN_MAX_T
     return (qkv.dtype == torch.bfloat16 and hd == 64) or (qkv.dtype == torch.float32 and hd in (32, 64))
 
 
@@ -137,7 +141,7 @@ def attention_pre_proj(m, x, policy=None, return_cls_attn=False, lens=None):
     if lens is not None:
         if _needs_grad(qkv) or not qkv.is_cuda or not _attn_kernel_ok(qkv, H) or policy is not None:
             raise RuntimeError("variable-length attention: inference only, no policy, CUDA qkv of a shape the d2s attention kernels "
-                               f"take (bf16 with head dim 64 or fp32 with head dim 32 / 64, T <= 256); got {tuple(qkv.shape)} {qkv.dtype}")
+                               f"take (bf16 with head dim 64 and T <= 2048, or fp32 with head dim 32 / 64 and T <= 256); got {tuple(qkv.shape)} {qkv.dtype}")
         o, cls_attn = ops.attention_core(qkv, H, scale=m.scale, want_cls_row=return_cls_attn, lengths=lens)
         return o, (cls_attn.to(qkv.dtype) if cls_attn is not None else None)
     if _needs_grad(qkv, policy) and qkv.is_cuda and qkv.dtype == torch.bfloat16 and T <= 256 and _TRAIN_ATTN:

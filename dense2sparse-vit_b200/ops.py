@@ -819,8 +819,11 @@ def attention_core(qkv, num_heads, policy=None, scale=None, eps=1e-6, want_cls_r
     cls_row (B,H,T) fp32 | None).  bf16 runs the tcgen05/TMEM kernel, fp32 the SIMT parity kernel.
     No autograd: the training path uses softmax_with_policy around library GEMMs.
     lengths (B) int: a padded batch, image b is its first lengths[b] tokens (keys and queries); out rows and cls_row columns
-    past it are zeros.  No policy in that form."""
+    past it are zeros.  No policy in that form.
+    bf16 inputs with T > 256 run the key-blocked kernel of attention_long."""
     _check_cuda(qkv, policy)
+    if qkv.dtype == torch.bfloat16 and qkv.shape[1] > LONG_ATTN_MIN_T:
+        return attention_long(qkv, num_heads, policy=policy, scale=scale, eps=eps, want_cls_row=want_cls_row, lengths=lengths)
     q = qkv.detach().contiguous()
     B, T, C3 = q.shape
     D = C3 // 3
@@ -838,6 +841,34 @@ def attention_core(qkv, num_heads, policy=None, scale=None, eps=1e-6, want_cls_r
     pol = _f32c(policy.reshape(B, T)) if policy is not None else None
     _call("d2s_attn_policy_fwd", _ptr(q), _ptr(pol), _dtype_code(q), B, T, num_heads, hd, float(scale), float(eps),
               _ptr(out), _ptr(cls_row), None, _stream(q))
+    return out, cls_row
+
+
+LONG_ATTN_MIN_T = 256     # attention_core hands bf16 sequences longer than this to attention_long
+LONG_ATTN_MAX_T = 2048
+
+
+def attention_long(qkv, num_heads, policy=None, scale=None, eps=1e-6, want_cls_row=False, lengths=None):
+    """Fused inference attention for any 1 <= T <= 2048 (384 / 512-pixel inputs): the key-blocked tcgen05 kernel
+    (d2s_attn_long_fwd), with the semantics of attention_core -- policy softmax (vit_models/dynamic_vit.py:195-214), CLS row,
+    and the variable-length form (lengths (B) int, no policy).  bf16 packed qkv (B,T,3*H*64) -> (out (B,T,H*64) bf16,
+    cls_row (B,H,T) fp32 | None).  No autograd."""
+    _check_cuda(qkv, policy)
+    if qkv.dtype != torch.bfloat16:
+        raise TypeError(f"attention_long: bf16 qkv only, got {qkv.dtype}")
+    q = qkv.detach().contiguous()
+    B, T, C3 = q.shape
+    D = C3 // 3
+    hd = D // num_heads
+    scale = hd ** -0.5 if scale is None else scale
+    if lengths is not None and policy is not None:
+        raise ValueError("attention_long: the variable-length form takes no policy")
+    out = torch.empty(B, T, D, dtype=q.dtype, device=q.device)
+    cls_row = torch.empty(B, num_heads, T, dtype=torch.float32, device=q.device) if want_cls_row else None
+    n = _lengths(lengths, B, "attention_long") if lengths is not None else None
+    pol = _f32c(policy.reshape(B, T)) if policy is not None else None
+    _call("d2s_attn_long_fwd", _ptr(q), _ptr(pol), _ptr(n), B, T, num_heads, hd, float(scale), float(eps), _ptr(out),
+          _ptr(cls_row), _stream(q))
     return out, cls_row
 
 

@@ -234,6 +234,15 @@ int d2s_adamw_flat_f32(float* p, const float* g, float* m, float* v, void* shado
  * 100 binades, so the result does not depend on where a row's maximum sits. */
 int d2s_attn_policy_fwd(const void* qkv, const float* policy, int dtype, int B, int T, int H, int hd,
                         float scale, float eps, void* out, float* cls_row, float* stats, d2s_stream_t stream);
+/* d2s_attn_long_fwd: the same attention core (dynamic_vit.py:195-214 softmax_with_policy, :218-234 Attention.forward) for
+ * sequences beyond 256 tokens (384 / 512-pixel inputs): bf16 only, hd == 64, 1 <= T <= 2048, key-blocked tcgen05/TMEM kernel
+ * (128-row query tiles x 128-column key blocks, K / V streamed, no (B,H,T,T) tensor, no global scratch).
+ * qkv (B,T,3,H,64), out (B,T,H*64), cls_row (B,H,T) f32 or NULL, as d2s_attn_policy_fwd; no row statistics.
+ * policy (B,T) f32 or NULL: the policy softmax of d2s_attn_policy_fwd (mask p_j off the diagonal, eps/T on every entry).
+ * len (B) int32 or NULL: the variable-length form of d2s_attn_varlen_fwd (image b = its first len[b] tokens, out rows and
+ * cls_row columns >= len[b] written as zeros); policy and len are never both given.  scale > 0; B == 0 is a no-op. */
+int d2s_attn_long_fwd(const void* qkv, const float* policy, const int* len, int B, int T, int H, int hd, float scale, float eps,
+                      void* out, float* cls_row, d2s_stream_t stream);
 
 /* Backward of d2s_attn_policy_fwd (bf16, hd == 64, T <= 208): Attention.forward's core under autograd, differentiable in qkv AND
  * in the keep policy (dynamic_vit.py:195-214, :218-231; default_dynamic_vit.py:185-199, :203-213), flash style -- scores and
