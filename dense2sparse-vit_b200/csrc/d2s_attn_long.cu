@@ -106,8 +106,6 @@ attn_long_fwd_kernel(const __grid_constant__ CUtensorMap map, const float* __res
   __syncthreads();
   tc_fence_after();
   const uint32_t tmem = bars->tmem_base;
-  pdl_wait();
-  pdl_trigger();
 
   const int w = warp_uniform(warp);
   if (w == kLongTmaWarp) {
@@ -487,9 +485,8 @@ int launch_long(const CUtensorMap& map, const float* policy, const int* lens, in
   cudaError_t e = opt_in_smem(opt, kern, (int)kLongSmem);
   D2S_REQUIRE(e == cudaSuccess, D2S_ERR_CUDA, "attn_long_fwd: cudaFuncSetAttribute: %s", cudaGetErrorString(e));
   const int grid = units < 2 * kNumSMs ? units : 2 * kNumSMs;
-  e = launch_pdl(kern, dim3(grid), dim3(kLongThreads), kLongSmem, stream, map, policy, lens, units, shp, scale, eps,
-                 (__nv_bfloat16*)out, cls_row, (const __nv_bfloat16*)qkv);
-  D2S_REQUIRE(e == cudaSuccess, D2S_ERR_CUDA, "attn_long_fwd: launch: %s", cudaGetErrorString(e));
+  kern<<<grid, kLongThreads, kLongSmem, stream>>>(map, policy, lens, units, shp, scale, eps, (__nv_bfloat16*)out, cls_row,
+                                                 (const __nv_bfloat16*)qkv);
   count_launch();
   return check_launch("d2s_attn_long_fwd(tcgen05)");
 }

@@ -611,16 +611,12 @@ static int launch_attn_simt(const void* qkv, const float* policy, int B, int T, 
   return check_launch(lens ? "d2s_attn_varlen_fwd(simt)" : "d2s_attn_policy_fwd(simt)");
 }
 
-int attn_simt_dispatch(const void* qkv, const float* policy, int dtype, int B, int T, int H, int hd, float scale,
-                       float eps, void* out, float* cls_row, cudaStream_t stream, const int* lens) {
+int attn_simt_dispatch(const void* qkv, const float* policy, int B, int T, int H, int hd, float scale, float eps, void* out,
+                       float* cls_row, cudaStream_t stream, const int* lens) {
   D2S_REQUIRE(hd == 64 || hd == 32, D2S_ERR_ARG, "attn(simt): hd=%d unsupported (32 or 64)", hd);
   D2S_REQUIRE(T >= 1 && T <= 32 * kAttnEPL, D2S_ERR_ARG, "attn(simt): T=%d outside [1,%d]", T, 32 * kAttnEPL);
-  if (dtype == D2S_F32) {
-    return hd == 64 ? launch_attn_simt<float, 64>(qkv, policy, B, T, H, scale, eps, out, cls_row, stream, lens)
-                    : launch_attn_simt<float, 32>(qkv, policy, B, T, H, scale, eps, out, cls_row, stream, lens);
-  }
-  return hd == 64 ? launch_attn_simt<__nv_bfloat16, 64>(qkv, policy, B, T, H, scale, eps, out, cls_row, stream, lens)
-                  : launch_attn_simt<__nv_bfloat16, 32>(qkv, policy, B, T, H, scale, eps, out, cls_row, stream, lens);
+  return hd == 64 ? launch_attn_simt<float, 64>(qkv, policy, B, T, H, scale, eps, out, cls_row, stream, lens)
+                  : launch_attn_simt<float, 32>(qkv, policy, B, T, H, scale, eps, out, cls_row, stream, lens);
 }
 
 }  // namespace d2s

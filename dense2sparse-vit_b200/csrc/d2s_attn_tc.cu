@@ -22,11 +22,11 @@ extern "C" int d2s_attn_policy_fwd(const void* qkv, const float* policy, int dty
               "attn_policy_fwd: qkv/out/stats must be 16-byte aligned");
   D2S_REQUIRE(scale > 0.0f, D2S_ERR_ARG, "attn_policy_fwd: scale must be positive (got %g)", (double)scale);
   cudaStream_t stream = (cudaStream_t)stream_;
-  if (dtype == D2S_F32 || force_simt()) {
+  if (dtype == D2S_F32) {
     D2S_REQUIRE(stats == nullptr, D2S_ERR_ARG, "attn_policy_fwd: row statistics are written by the bf16 tcgen05 kernel only");
     D2S_REQUIRE((long long)B * H <= 65535, D2S_ERR_ARG, "attn_policy_fwd(simt): B*H=%lld exceeds 65535", (long long)B * H);
     if (B == 0) return D2S_OK;
-    return attn_simt_dispatch(qkv, policy, dtype, B, T, H, hd, scale, eps, out, cls_row, stream);
+    return attn_simt_dispatch(qkv, policy, B, T, H, hd, scale, eps, out, cls_row, stream);
   }
   D2S_REQUIRE(hd == kTcHD, D2S_ERR_ARG, "attn_policy_fwd(bf16): head dim %d unsupported by the tcgen05 kernel (64 only)", hd);
   D2S_REQUIRE(T <= 256, D2S_ERR_ARG, "attn_policy_fwd(bf16): T=%d exceeds 256", T);
@@ -40,8 +40,6 @@ extern "C" int d2s_attn_policy_fwd(const void* qkv, const float* policy, int dty
     return policy ? launch_tc<1, true, 4>(map_a, map_b, policy, units, T, H, Tkp, scale, eps, out, cls_row, stats, qkv, stream)
                   : launch_tc<1, false, 4>(map_a, map_b, policy, units, T, H, Tkp, scale, eps, out, cls_row, stats, qkv, stream);
   }
-  static const bool pol8 = []() { const char* e = getenv("D2S_ATTN_POL_SW"); return !(e && e[0] == '4'); }();
-  if (policy && !pol8) return launch_tc<2, true, 4>(map_a, map_b, policy, units, T, H, Tkp, scale, eps, out, cls_row, stats, qkv, stream);
   return policy ? launch_tc<2, true, 8>(map_a, map_b, policy, units, T, H, Tkp, scale, eps, out, cls_row, stats, qkv, stream)
                 : launch_tc<2, false, 8>(map_a, map_b, policy, units, T, H, Tkp, scale, eps, out, cls_row, stats, qkv, stream);
 }

@@ -120,8 +120,6 @@ attn_tc_fwd_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_const
   __syncthreads();
   tc_fence_after();
   const uint32_t tmem = bars->tmem_base;
-  pdl_wait();       // set-up above overlaps the previous kernel's tail (d2s_common.cuh, launch_pdl); qkv / policy are read below
-  pdl_trigger();
 
   if (warp_uniform(warp) == kSW) {
     {
@@ -602,17 +600,9 @@ attn_tc_fwd_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_const
   }
 }
 
-int attn_simt_dispatch(const void* qkv, const float* policy, int dtype, int B, int T, int H, int hd, float scale,
-                       float eps, void* out, float* cls_row, cudaStream_t stream, const int* lens = nullptr);
-
-static bool force_simt() {
-  static int v = -1;
-  if (v < 0) {
-    const char* e = getenv("D2S_ATTN_FORCE_SIMT");
-    v = (e && e[0] == '1') ? 1 : 0;
-  }
-  return v == 1;
-}
+// the fp32 attention forward (SIMT kernel, d2s_attn_simt.cu)
+int attn_simt_dispatch(const void* qkv, const float* policy, int B, int T, int H, int hd, float scale, float eps, void* out,
+                       float* cls_row, cudaStream_t stream, const int* lens = nullptr);
 
 // cuTensorMapEncodeTiled through the runtime's driver entry point (no link-time dependency on libcuda)
 typedef CUresult (*EncodeFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
@@ -674,9 +664,8 @@ static int launch_tc(const CUtensorMap& map_a, const CUtensorMap& map_b, const f
   cudaError_t e = opt_in_smem(opt, kern, 113 * 1024);
   D2S_REQUIRE(e == cudaSuccess, D2S_ERR_CUDA, "attn_policy_fwd: cudaFuncSetAttribute: %s", cudaGetErrorString(e));
   const int grid = units < per_sm * kNumSMs ? units : per_sm * kNumSMs;
-  e = launch_pdl(kern, dim3(grid), dim3(tc_threads(kSW)), smem, stream, map_a, map_b, policy, units, T, H, Tkp, kbufs, scale, eps,
-                 (__nv_bfloat16*)out, cls_row, stats, (const __nv_bfloat16*)qkv, lens);
-  D2S_REQUIRE(e == cudaSuccess, D2S_ERR_CUDA, "attn_policy_fwd: launch: %s", cudaGetErrorString(e));
+  kern<<<grid, tc_threads(kSW), smem, stream>>>(map_a, map_b, policy, units, T, H, Tkp, kbufs, scale, eps, (__nv_bfloat16*)out,
+                                                 cls_row, stats, (const __nv_bfloat16*)qkv, lens);
   count_launch();
   return check_launch(kVar ? "d2s_attn_varlen_fwd(tcgen05)" : "d2s_attn_policy_fwd(tcgen05)");
 }

@@ -17,10 +17,10 @@ extern "C" int d2s_attn_varlen_fwd(const void* qkv, const int* lens, int dtype, 
   D2S_REQUIRE(aligned16(qkv) && aligned16(out), D2S_ERR_ALIGN, "attn_varlen_fwd: qkv/out must be 16-byte aligned");
   D2S_REQUIRE(scale > 0.0f, D2S_ERR_ARG, "attn_varlen_fwd: scale must be positive (got %g)", (double)scale);
   cudaStream_t stream = (cudaStream_t)stream_;
-  if (dtype == D2S_F32 || force_simt()) {
+  if (dtype == D2S_F32) {
     D2S_REQUIRE((long long)B * H <= 65535, D2S_ERR_ARG, "attn_varlen_fwd(simt): B*H=%lld exceeds 65535", (long long)B * H);
     if (B == 0) return D2S_OK;
-    return attn_simt_dispatch(qkv, nullptr, dtype, B, Tmax, H, hd, scale, 0.0f, out, cls_row, stream, lens);
+    return attn_simt_dispatch(qkv, nullptr, B, Tmax, H, hd, scale, 0.0f, out, cls_row, stream, lens);
   }
   D2S_REQUIRE(hd == kTcHD, D2S_ERR_ARG, "attn_varlen_fwd(bf16): head dim %d unsupported by the tcgen05 kernel (64 only)", hd);
   if (B == 0) return D2S_OK;

@@ -42,42 +42,6 @@ static inline cudaError_t opt_in_smem(SmemOptIn& st, K kern, int bytes) {
   return e;
 }
 
-// ---- programmatic dependent launch (PDL) ------------------------------------------------------------------------------
-// A kernel launched through launch_pdl() may start while the previous kernel of the stream is still draining (its CTAs become
-// resident as SMs free up): barrier initialisation, TMEM allocation and the launch latency overlap the predecessor's tail.  Such
-// a kernel MUST execute pdl_wait() before it reads anything a predecessor may have written (it blocks until the preceding grid
-// has completed and its writes are visible) and calls pdl_trigger() to let ITS successor start early.  Both are no-ops when the
-// launch carried no PDL attribute or the predecessor is not a kernel.  Captured into CUDA graphs as programmatic dependency edges.
-// OFF unless D2S_PDL=1: on the inference step (attention -> proj+LN -> MLP chains between library GEMMs, which neither trigger nor
-// wait) and on the training step the same-box A/B shows no difference beyond noise (8.492 / 8.449 ms off, 8.498 / 8.469 ms on;
-// training 19.28 / 19.24 off, 19.25 / 19.10 on): what PDL can overlap here is only barrier set-up and the TMEM allocation -- a
-// dependent kernel's first tile needs the whole previous grid's output -- while the time lost at kernel boundaries is the row-tile
-// quantisation of the last wave (DESIGN.md section 9), which an early launch does not touch.
-static inline bool pdl_enabled() {
-  static int v = -1;
-  if (v < 0) {
-    const char* e = getenv("D2S_PDL");
-    v = (e && e[0] == '1') ? 1 : 0;
-  }
-  return v == 1;
-}
-template <typename... KArgs, typename... Args>
-static inline cudaError_t launch_pdl(void (*kern)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st, Args&&... args) {
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = grid;
-  cfg.blockDim = block;
-  cfg.dynamicSmemBytes = smem;
-  cfg.stream = st;
-  cudaLaunchAttribute at[1];
-  at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  at[0].val.programmaticStreamSerializationAllowed = pdl_enabled() ? 1 : 0;
-  cfg.attrs = at;
-  cfg.numAttrs = 1;
-  return cudaLaunchKernelEx(&cfg, kern, static_cast<KArgs>(args)...);
-}
-__device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
-__device__ __forceinline__ void pdl_trigger() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
-
 static inline bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; }
 static inline int  ceil_div(int a, int b) { return (a + b - 1) / b; }
 static inline size_t elem_size(int dtype) { return dtype == D2S_BF16 ? 2 : 4; }

@@ -88,7 +88,6 @@ struct GpParams {
   float eps;
   int M, N, K, act, want_ln;
   long long* trace;             // D2S_GEMM_TRACE: device buffer for per-warp clock64 phase totals (profiling only)
-  int dbg;                      // profiling switches (D2S_GEMM_DEBUG): 1 no output stores, 2 no epilogue body, 8 no operand loads
   int ares;                     // MODE_ACT192, K <= 384: the row tile's A rows stay resident across its column tiles
   int groups;                   // MODE_ACT*: a row tile's column tiles are split into `groups` work units (last-wave quantisation); 1 otherwise
   // MODE_ACT192 + ares: LayerNorm of the INPUT rows applied on the fly (A is the raw residual stream, in_stats its per-row (mean, rstd))
@@ -142,8 +141,6 @@ gemm_pair_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constan
     asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(&bars->tmem_base)), "n"(512) : "memory");
     asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
   }
-  pdl_wait();       // everything above overlaps the previous kernel's tail; nothing below may run before its writes are visible
-  pdl_trigger();
   if (MODE == kGpModeLn) {
     for (int i = tid; i < p.N; i += kThreads) {
       bias_s[i] = p.bias ? __bfloat162float(p.bias[i]) : 0.f;
@@ -204,7 +201,6 @@ gemm_pair_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constan
             const uint32_t s = it % STAGES, n = it / STAGES;
             mbar_wait(smem_u32(&bars->empty[s]), (n & 1) ^ 1);
             const uint32_t full_local = smem_u32(&bars->full[s]);
-            if (p.dbg & 8) { if (rank == 0) mbar_expect_tx(full_local, 0); continue; }
             if (rank == 0) mbar_expect_tx(full_local, 2 * kStage);       // both CTAs' boxes land on the leader's barrier
             const uint32_t full_leader = mapa(full_local, 0);
             const uint32_t dst = smem_u32(ring + s * kStage);
@@ -320,7 +316,6 @@ gemm_pair_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constan
           GP_TRACE(1)
 #pragma unroll
           for (int c = 0; c < 2; ++c) {
-            if (p.dbg & 2) break;
             uint32_t v[32];
             tmem_ld32_nowait(taddr + c * 32, v);
             tmem_ld_wait();
@@ -358,7 +353,7 @@ gemm_pair_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constan
           if (lane == 0) mbar_arrive_cluster(mapa(smem_u32(&bars->tmem_empty[as]), 0));
           asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
           asm volatile("bar.sync %0, 128;" ::"r"(1 + part) : "memory");
-          if (issuer && !(p.dbg & 1)) {
+          if (issuer) {
             tma_store_2d(&map_o, smem_u32(blk), col0, row0);
             asm volatile("cp.async.bulk.commit_group;" ::: "memory");
           }
@@ -562,11 +557,6 @@ gemm_pair_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constan
   }
 }
 
-static int gp_debug() {
-  const char* e = getenv("D2S_GEMM_DEBUG");
-  return e ? atoi(e) : 0;
-}
-
 static long long* gp_trace() {
   const char* e = getenv("D2S_GEMM_TRACE");
   return e ? reinterpret_cast<long long*>(strtoull(e, nullptr, 10)) : nullptr;
@@ -600,8 +590,7 @@ static int gp_launch(const CUtensorMap& ma, const CUtensorMap& mw, const CUtenso
   const int pair_tiles = (p.M + 2 * kGpBM - 1) / (2 * kGpBM);
   const int units = pair_tiles * (MODE == kGpModeLn ? 1 : p.groups);
   const int pairs = units < kNumSMs / 2 ? units : kNumSMs / 2;
-  e = launch_pdl(gemm_pair_kernel<MODE, NSUB, ACT>, dim3(2 * pairs), dim3((2 + 4 * Cfg::PARTS) * 32), smem, stream, ma, mw, mo, p);
-  D2S_REQUIRE(e == cudaSuccess, D2S_ERR_CUDA, "%s: launch: %s", what, cudaGetErrorString(e));
+  gemm_pair_kernel<MODE, NSUB, ACT><<<2 * pairs, (2 + 4 * Cfg::PARTS) * 32, smem, stream>>>(ma, mw, mo, p);
   count_launch();
   return check_launch(what);
 }
@@ -625,22 +614,18 @@ static int gp_linear_act(const char* what, const void* a, const float* in_stats,
   if ((rc = gp_map_2d(&ma, a, K, M, kGpBK, kGpBM, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, what))) return rc;
   if ((rc = gp_map_2d(&mw, w, K, N, kGpBK, t192 ? 96 : 128, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, what))) return rc;
   if ((rc = gp_map_2d(&mo, out, N, M, 64, kGpBM, CU_TENSOR_MAP_L2_PROMOTION_NONE, what))) return rc;
-  static const bool ares_on = []() { const char* e = getenv("D2S_GEMM_ARES"); return !(e && e[0] == '0'); }();
   // Split a row tile's column tiles into G work units when that shortens the last wave: time per CTA pair ~
   // ceil(row tiles * G / pairs) units of (column tiles per unit + 0.25) -- each unit (re)loads the A rows, partly exposed.
   const int n_tiles = N / (t192 ? 192 : 256), pair_tiles = (M + 2 * kGpBM - 1) / (2 * kGpBM), np = kNumSMs / 2;
   int groups = 1;
-  {
-    static const bool grp_on = []() { const char* e = getenv("D2S_GEMM_GROUPS"); return !(e && e[0] == '0'); }();
-    double best = (double)((pair_tiles + np - 1) / np) * (n_tiles + 0.25);
-    for (int g = 2; g <= n_tiles && grp_on; ++g) {
-      if (n_tiles % g) continue;
-      const double r = (double)((pair_tiles * g + np - 1) / np) * (n_tiles / g + 0.25);
-      if (r < best * 0.99) { best = r; groups = g; }
-    }
+  double best = (double)((pair_tiles + np - 1) / np) * (n_tiles + 0.25);
+  for (int g = 2; g <= n_tiles; ++g) {
+    if (n_tiles % g) continue;
+    const double r = (double)((pair_tiles * g + np - 1) / np) * (n_tiles / g + 0.25);
+    if (r < best * 0.99) { best = r; groups = g; }
   }
   GpParams p{(const __nv_bfloat16*)bias, nullptr, nullptr, nullptr, nullptr, nullptr, (__nv_bfloat16*)pre, nullptr, 0.f, M, N, K, act, 0,
-             gp_trace(), gp_debug(), (t192 && K <= 6 * kGpBK && (ares_on || in_stats)) ? 1 : 0, groups,
+             gp_trace(), (t192 && K <= 6 * kGpBK) ? 1 : 0, groups,
              reinterpret_cast<const float2*>(in_stats), (const __nv_bfloat16*)in_gamma, (const __nv_bfloat16*)in_beta};
   D2S_REQUIRE(!in_stats || p.ares, D2S_ERR_ARG, "%s: the on-the-fly input LayerNorm needs N %% 192 == 0 (N %% 256 != 0) and K <= %d", what,
               6 * kGpBK);
@@ -671,7 +656,7 @@ static int gp_linear_residual(const char* what, const void* a, const void* w, co
   if ((rc = gp_map_2d(&mw, w, K, N, kGpBK, 96, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, what))) return rc;
   GpParams p{(const __nv_bfloat16*)bias, (const __nv_bfloat16*)gamma, (const __nv_bfloat16*)beta, (const __nv_bfloat16*)x,
              (__nv_bfloat16*)out_sum, (__nv_bfloat16*)out_norm, nullptr, reinterpret_cast<float2*>(stats), eps, M, N, K, 0,
-             (out_norm || stats) ? 1 : 0, gp_trace(), gp_debug(), 0, 1, nullptr, nullptr, nullptr};
+             (out_norm || stats) ? 1 : 0, gp_trace(), 0, 1, nullptr, nullptr, nullptr};
   if (N != 192) return gp_launch<kGpModeLn, 2, 0>(ma, mw, ma, p, (cudaStream_t)stream, what);      // 384, or 768 as two halves
   return gp_launch<kGpModeLn, 1, 0>(ma, mw, ma, p, (cudaStream_t)stream, what);
 }

@@ -19,42 +19,28 @@
 //
 //   warp 0      TMA producer: H tile (once per row tile) and W1 k-blocks      warp 2   TMA producer: W2 chunks
 //   warp 1      TMEM allocation; G1 issue (leader CTA only)                   warp 3   G2 issue (leader CTA only)
-//   warps 4-11  E1: GELU of the hidden chunks (two groups of four warps; -DMP_E1W=16: four groups of 32 columns under setmaxnreg,
-//               measured slower -- the stage is bound by the sub-partitions' issue / MUFU slots, not by per-warp latency)
+//   warps 4-11  E1: GELU of the hidden chunks (two groups of four warps, 64 columns each)
 //   warps 12-15 output: residual add + LayerNorm of the finished row tile, overlapped with the next tile's GEMMs
-// Build options for experiments: -DMP_W1 / -DMP_W2 (weight ring depths, default 5 / 3), -DMP_E1W (8 | 16), -DMP_NO_GELU (the activation
-// stage without its arithmetic: 412 -> 399 us at T = 197, i.e. the GELU is not what bounds the kernel), -DD2S_GEMM_TRACE_BUILD
-// (clock64 totals of the issuers' barrier waits into MpParams::trace, a device buffer named by the D2S_GEMM_TRACE environment variable).
+// Measured alternatives, removed:
+//   * 16 E1 warps (four groups of 32 columns under setmaxnreg): slower -- the stage is bound by the sub-partitions' issue / MUFU
+//     slots, not by per-warp latency.
+//   * The activation stage without its arithmetic: 412 -> 399 us at T = 197, i.e. the GELU is not what bounds the kernel.
+// -DD2S_GEMM_TRACE_BUILD (profiling builds): clock64 totals of the issuers' barrier waits into MpParams::trace, a device buffer
+// named by the D2S_GEMM_TRACE environment variable.
 #include <stdlib.h>
 #include "d2s_tc.cuh"
-
-// -DMP_NO_GELU (profiling builds only): the activation stage without its arithmetic, to see what the GELU costs the pipeline
-#ifdef MP_NO_GELU
-#define MP_GELU(x) (x)
-#else
-#define MP_GELU(x) gelu_erf_pair(x)
-#endif
 
 namespace d2s {
 
 constexpr int kMpBM = 128, kMpD = 384, kMpCH = 128, kMpKB = kMpD / 64;
-#ifndef MP_W1
-#define MP_W1 5
-#endif
-#ifndef MP_W2
-#define MP_W2 3
-#endif
-constexpr int kMpW1Slots = MP_W1, kMpW2Slots = MP_W2;
+constexpr int kMpW1Slots = 5, kMpW2Slots = 3;   // weight ring depths
 constexpr uint32_t kMpA1Blk = 128 * 128;        // 16 KB: 128 rows x 64 bf16 of H
 constexpr uint32_t kMpW1Blk = 64 * 128;         //  8 KB: this CTA's 64 of the 128 W1 rows of a chunk, one k-block
 constexpr uint32_t kMpW2Blk = 96 * 128;         // 12 KB: this CTA's 96 of the 192 W2 rows of one N-half, 64 of the chunk's 128 hidden columns
 constexpr uint32_t kMpPBlk = 128 * 128;         // 16 KB: 128 rows x 64 bf16; P_j is two of them
-#ifndef MP_E1W
-#define MP_E1W 8
-#endif
-constexpr int kMpE1Warps = MP_E1W, kMpOutWarps = 4, kMpThreads = (4 + kMpE1Warps + kMpOutWarps) * 32;
+constexpr int kMpE1Warps = 8, kMpOutWarps = 4, kMpThreads = (4 + kMpE1Warps + kMpOutWarps) * 32;
 constexpr int kMpE1Parts = kMpE1Warps / 4;          // E1 warps per TMEM lane quadrant
-constexpr int kMpE1Cols = kMpCH / kMpE1Parts;       // hidden columns of a chunk per E1 warp (64 or 32)
+constexpr int kMpE1Cols = kMpCH / kMpE1Parts;       // hidden columns of a chunk per E1 warp
 constexpr uint32_t kMpAccCols = 384, kMpSCols = 128;
 
 // clock64 totals of the issuing warps' waits (profiling builds only: D2S_NVCC_EXTRA=-DD2S_GEMM_TRACE_BUILD)
@@ -116,11 +102,7 @@ __device__ __noinline__ void mp_normalize_block(unsigned char* hb, int r, int ch
 // kLnIn: the LayerNorm of the input is applied on the fly (MpParams::in_stats); a separate instantiation, so that the plain form
 // compiles exactly as it did before the option existed
 template <bool kLnIn>
-#if MP_E1W == 8
 __global__ void __cluster_dims__(2, 1, 1) __maxnreg__(128)
-#else
-__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kMpThreads, 1)
-#endif
 mlp_pair_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant__ CUtensorMap map_w1,
                 const __grid_constant__ CUtensorMap map_w2, const MpParams p) {
   constexpr int TN = kMpD;
@@ -166,8 +148,6 @@ mlp_pair_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant
     asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(&bars->tmem_base)), "n"(512) : "memory");
     asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
   }
-  pdl_wait();       // barrier set-up and the TMEM allocation overlap the previous kernel's tail (d2s_common.cuh, launch_pdl)
-  pdl_trigger();
   for (int i = tid; i < p.HID; i += kMpThreads) b1_s[i] = p.b1 ? __bfloat162float(p.b1[i]) : 0.f;
   for (int i = tid; i < TN; i += kMpThreads) {
     b2_s[i] = p.b2 ? __bfloat162float(p.b2[i]) : 0.f;
@@ -181,16 +161,7 @@ mlp_pair_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant
   tc_fence_after();
   const uint32_t tmem = bars->tmem_base;
 
-#if MP_E1W == 16
-  // 24 warps: the launch gives every thread 80 registers; the control warps hand some back to the output warps (setmaxnreg works
-  // per warpgroup = 4 aligned warps, which is how the roles are laid out).  4*32*48 + 16*32*80 + 4*32*112 = 768 * 80.
-  // (ptxas sizes a role's registers by the setmaxnreg that DOMINATES its code, so each sits at the top of its role's branch)
-#endif
-
   if (warp_u < 4) {
-#if MP_E1W == 16
-  asm volatile("setmaxnreg.dec.sync.aligned.u32 48;");
-#endif
   if (warp == 0) {
     if (lane == 0) {
       // ============================ TMA producer: H tile + W1 k-blocks (both CTAs) ============================
@@ -350,7 +321,7 @@ mlp_pair_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant
         for (int q = 0; q < 16; ++q) {
           const float2 bq = *reinterpret_cast<const float2*>(&b1_s[j * kMpCH + part * kMpE1Cols + 2 * q]);
           float g0, g1;
-          f2_unpack(MP_GELU(f2_add(f2_pack(__uint_as_float(va[2 * q]), __uint_as_float(va[2 * q + 1])), f2_pack(bq.x, bq.y))), g0, g1);
+          f2_unpack(gelu_erf_pair(f2_add(f2_pack(__uint_as_float(va[2 * q]), __uint_as_float(va[2 * q + 1])), f2_pack(bq.x, bq.y))), g0, g1);
           o[q] = pack_bf16x2(g0, g1);
         }
         if (kMpE1Cols == 64) {
@@ -358,7 +329,7 @@ mlp_pair_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant
           for (int q = 0; q < 16; ++q) {
             const float2 bq = *reinterpret_cast<const float2*>(&b1_s[j * kMpCH + part * kMpE1Cols + 32 + 2 * q]);
             float g0, g1;
-            f2_unpack(MP_GELU(f2_add(f2_pack(__uint_as_float(vb[2 * q]), __uint_as_float(vb[2 * q + 1])), f2_pack(bq.x, bq.y))), g0, g1);
+            f2_unpack(gelu_erf_pair(f2_add(f2_pack(__uint_as_float(vb[2 * q]), __uint_as_float(vb[2 * q + 1])), f2_pack(bq.x, bq.y))), g0, g1);
             o[(kMpE1Cols == 64 ? 16 : 0) + q] = pack_bf16x2(g0, g1);
           }
         }
@@ -377,9 +348,6 @@ mlp_pair_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant
     // every tile was spent here with the tensor pipe idle).  Global memory is touched in coalesced 64-byte row segments
     // through a 2 KB per-warp transposition buffer.  x' is not kept in registers: pass 2 re-reads it (L2-hot) once the row's
     // mean and variance are known.  Only pass 1 holds the accumulator, so G2 of the next tile waits for little.
-#if MP_E1W == 16
-    asm volatile("setmaxnreg.inc.sync.aligned.u32 112;");
-#endif
     const int quad = warp & 3;
     const int ow = warp - 4 - kMpE1Warps;       // 0..3
     const uint32_t lane_addr = tmem + ((uint32_t)(quad * 32) << 16);
@@ -605,9 +573,8 @@ static int mp_launch(const char* what, const void* h, const float* in_stats, con
   D2S_REQUIRE(e == cudaSuccess, D2S_ERR_CUDA, "mlp_residual_ln: cudaFuncSetAttribute: %s", cudaGetErrorString(e));
   const int pair_tiles = (M + 2 * kMpBM - 1) / (2 * kMpBM);
   const int pairs = pair_tiles < kNumSMs / 2 ? pair_tiles : kNumSMs / 2;
-  e = in_stats ? launch_pdl(mlp_pair_kernel<true>, dim3(2 * pairs), dim3(kMpThreads), smem, (cudaStream_t)stream, ma, mw1, mw2, p)
-               : launch_pdl(mlp_pair_kernel<false>, dim3(2 * pairs), dim3(kMpThreads), smem, (cudaStream_t)stream, ma, mw1, mw2, p);
-  D2S_REQUIRE(e == cudaSuccess, D2S_ERR_CUDA, "mlp_residual_ln: launch: %s", cudaGetErrorString(e));
+  if (in_stats) mlp_pair_kernel<true><<<2 * pairs, kMpThreads, smem, (cudaStream_t)stream>>>(ma, mw1, mw2, p);
+  else          mlp_pair_kernel<false><<<2 * pairs, kMpThreads, smem, (cudaStream_t)stream>>>(ma, mw1, mw2, p);
   count_launch();
   return check_launch(what);
 }

@@ -78,10 +78,7 @@ __device__ __forceinline__ float act_apply(float x, int act) {
 template <typename T_> struct ActFast { static constexpr bool value = false; };
 template <> struct ActFast<__nv_bfloat16> { static constexpr bool value = true; };
 
-#ifndef D2S_POOL_THREADS
-#define D2S_POOL_THREADS 256
-#endif
-constexpr int kPoolThreads = D2S_POOL_THREADS;
+constexpr int kPoolThreads = 256;
 
 // grid = B; thread = (16-byte vector column v, token group g); groups stride the tokens
 template <typename T_>

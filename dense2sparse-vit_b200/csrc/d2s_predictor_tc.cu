@@ -70,7 +70,6 @@ struct PfParams {
   int64_t* kept;
   float* prev_kept;
   int B, N, K;
-  int dbg;                          // profiling switches (D2S_PF_DEBUG): 1 no epilogue arithmetic
 };
 
 // bf16(GELU(bf16(x))) for a pair, as the separate Linear -> GELU modules round
@@ -261,7 +260,7 @@ predictor_a_tail_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_
         // ---- E2: second Linear + per-image bias -> GELU -> u, in place over the tile (A operand of the third Linear) ----
         const int u = step, i = u / nt, t = u - i * nt;
         const uint32_t s = u & 1, ph = (u >> 1) & 1, pb = i & 1;
-        const bool quad_active = t * 128 + quad * 32 < N && !(p.dbg & 1);   // rows past N: nothing to compute (their u rows stay stale)
+        const bool quad_active = t * 128 + quad * 32 < N;   // rows past N: nothing to compute (their u rows stay stale)
         if (t == 0) mbar_wait(smem_u32(&bars->pi_full[pb]), (i >> 1) & 1);
         mbar_wait(smem_u32(&bars->b_full[s]), ph);
         tc_fence_after();
@@ -302,7 +301,7 @@ predictor_a_tail_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_
         const int img = (int)blockIdx.x + i * (int)gridDim.x;
         const uint32_t kb = i & 1;
         const int n = t * 128 + r;
-        const bool quad_active = t * 128 + quad * 32 < N && !(p.dbg & 1);
+        const bool quad_active = t * 128 + quad * 32 < N;
         if (t == 0) mbar_wait(smem_u32(&bars->key_empty[kb]), ((i >> 1) & 1) ^ 1);
         mbar_wait(smem_u32(&bars->c_full), u & 1);
         tc_fence_after();
@@ -349,11 +348,6 @@ predictor_a_tail_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_
     tc_fence_after();
     asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "n"(512) : "memory");
   }
-}
-
-static int pf_debug() {
-  const char* e = getenv("D2S_PF_DEBUG");
-  return e ? atoi(e) : 0;
 }
 
 static int pf_map(CUtensorMap* map, const void* base, int rank, const cuuint64_t* gdim, const cuuint64_t* gstr,
@@ -405,7 +399,7 @@ extern "C" int d2s_predictor_a_tail_bf16(const void* local, int ld, long long lb
     const cuuint32_t box[2] = {64, (cuuint32_t)kPfQ};
     if ((rc = pf_map(&mw3, w3, 2, gdim, gstr, box, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, what))) return rc;
   }
-  PfParams p{(const __nv_bfloat16*)per_image, (const __nv_bfloat16*)b3, w4, b4, prev, logp, kept, prev_kept, B, N, K, pf_debug()};
+  PfParams p{(const __nv_bfloat16*)per_image, (const __nv_bfloat16*)b3, w4, b4, prev, logp, kept, prev_kept, B, N, K};
   const size_t smem = 1024 + (size_t)3 * kPfW2Bytes + 3 * kPfW3Bytes + 2 * kPfSlot + sizeof(PfSmall);
   D2S_REQUIRE(smem <= 227 * 1024, D2S_ERR_ARG, "%s: needs %zu B of shared memory", what, smem);
   static SmemOptIn opt;

@@ -20,20 +20,19 @@ import torch.nn.functional as F
 
 from . import ops
 
-_FUSED_FC1 = os.environ.get("D2S_FUSED_FC1", "1") != "0"   # A/B switch for the tcgen05 fc1+GELU GEMM
-_TRAIN_ATTN = os.environ.get("D2S_TRAIN_ATTN", "1") != "0"    # A/B switch for ops.attention_train (bf16 training attention)
-_FROZEN_BF16 = os.environ.get("D2S_FROZEN_BF16", "1") != "0"   # A/B switch: cached bf16 copy of a frozen teacher under bf16 autocast
-_FUSED_ADD_LN_TRAIN = os.environ.get("D2S_FUSED_ADD_LN_TRAIN", "1") != "0"   # A/B switch: residual adds folded into LayerNorm fwd/bwd
-_FUSED_MLP = os.environ.get("D2S_FUSED_MLP", "1") != "0"      # A/B switch for the one-kernel MLP (ops.mlp_residual_ln)
-_FUSED_PAIR = os.environ.get("D2S_FUSED_PAIR", "1") != "0"  # A/B switch for the CTA-pair GEMMs (fc1 pair; proj/fc2 + add + LN)
-_LAZY_PRED = os.environ.get("D2S_LAZY_PRED", "1") != "0"    # A/B switch: the predictors' input norm applied inside their first GEMM (row statistics)
-_LAZY_NORM1 = os.environ.get("D2S_LAZY_NORM1", "1") != "0"  # A/B switch: norm1 applied inside the qkv GEMM from the MLP kernel's row statistics
-_LAZY_NORM2 = os.environ.get("D2S_LAZY_NORM2", "1") != "0"  # A/B switch: norm2 applied inside the one-kernel MLP from per-row statistics (no normalised copy)
-_QKV_PAIR = os.environ.get("D2S_QKV_PAIR", "1") != "0"     # A/B switch: inference qkv projection on the CTA-pair tcgen05 GEMM (else the library GEMM)
-_PRED_FUSED = os.environ.get("D2S_PRED_FUSED", "1") != "0"  # A/B switch: second half of the Variant A predictor + selection as one tcgen05 kernel (inference, D = 384)
-_POOL_TRAIN = os.environ.get("D2S_POOL_TRAIN", "1") != "0"  # A/B switch: the predictors' local/global split as one kernel each way
+# Test hooks.  Each is True in use; a test sets one to False to run the unfused reference path it compares the fused path
+# against (tests/test_gpu_models.py::test_fused_block_kernels_at_deit_s_width, ::test_training_fusions_match_the_unfused_training_path,
+# ::test_frozen_teacher_under_autocast_runs_on_a_cached_bf16_copy; tests/test_gpu_parity.py::test_predictor_a_tail_matches_the_unfused_path,
+# ::test_lazy_norms_are_invisible_at_model_level; the kernel on/off comparisons in tests/test_gpu_long_attn.py).
+_FUSED_PAIR = True           # the CTA-pair GEMMs (qkv, fc1 pair; proj/fc2 + add + LN)
+_FUSED_MLP = True            # the one-kernel MLP (ops.mlp_residual_ln)
+_FUSED_ADD_LN_TRAIN = True   # residual adds folded into LayerNorm fwd/bwd
+_FROZEN_BF16 = True          # cached bf16 copy of a frozen teacher under bf16 autocast
+_PRED_FUSED = True           # second half of the Variant A predictor + selection as one tcgen05 kernel (inference, D = 384)
+_LAZY_NORM1 = True           # norm1 applied inside the qkv GEMM from the MLP kernel's row statistics
+_LAZY_NORM2 = True           # norm2 applied inside the one-kernel MLP from per-row statistics (no normalised copy)
+_LONG_ATTN = True            # bf16 inference attention beyond 256 tokens on the key-blocked kernel
 _THRESHOLD_INFERENCE = os.environ.get("D2S_THRESHOLD_INFERENCE", "0") == "1"   # opt-in: what dynamic_vit.py:935-949 intends
-_LONG_ATTN = os.environ.get("D2S_LONG_ATTN", "1") != "0"    # A/B switch: bf16 inference attention beyond 256 tokens on the key-blocked kernel
 INIT_N = 14 * 14  # the reference hard-codes 196 spatial tokens (dynamic_vit.py:828, default_dynamic_vit.py:446)
 
 
@@ -56,7 +55,7 @@ def _ln_rows_ok(x):
 
 def _attn_kernel_ok(qkv, H):
     """Shapes of the fused attention kernels: bf16 -> tcgen05 kernel (hd 64), fp32 -> SIMT kernel (hd 32 / 64), T <= 256; and bf16,
-    hd 64, 256 < T <= 2048 -> the key-blocked tcgen05 kernel (d2s_attn_long_fwd) unless D2S_LONG_ATTN=0."""
+    hd 64, 256 < T <= 2048 -> the key-blocked tcgen05 kernel (d2s_attn_long_fwd)."""
     hd = qkv.shape[-1] // 3 // H
     if qkv.shape[-1] != 3 * H * hd:
         return False
@@ -112,7 +111,7 @@ def patch_embed_forward(m, img):
 
 def _qkv_pair_ok(lin, x):
     """The qkv projection runs on the CTA-pair tcgen05 GEMM with 192-column tiles and resident input rows: inference, bf16, D <= 384."""
-    return (_QKV_PAIR and _FUSED_PAIR and x.is_cuda and x.dtype == torch.bfloat16 and lin.weight.dtype == torch.bfloat16
+    return (_FUSED_PAIR and x.is_cuda and x.dtype == torch.bfloat16 and lin.weight.dtype == torch.bfloat16
             and not _needs_grad(x, lin.weight, lin.bias) and lin.in_features % 64 == 0 and lin.in_features <= 384
             and lin.out_features % 192 == 0 and lin.out_features % 256 != 0)
 
@@ -144,7 +143,7 @@ def attention_pre_proj(m, x, policy=None, return_cls_attn=False, lens=None):
                                f"take (bf16 with head dim 64 and T <= 2048, or fp32 with head dim 32 / 64 and T <= 256); got {tuple(qkv.shape)} {qkv.dtype}")
         o, cls_attn = ops.attention_core(qkv, H, scale=m.scale, want_cls_row=return_cls_attn, lengths=lens)
         return o, (cls_attn.to(qkv.dtype) if cls_attn is not None else None)
-    if _needs_grad(qkv, policy) and qkv.is_cuda and qkv.dtype == torch.bfloat16 and T <= 256 and _TRAIN_ATTN:
+    if _needs_grad(qkv, policy) and qkv.is_cuda and qkv.dtype == torch.bfloat16 and T <= 256:
         # training, bf16: the tcgen05 flash forward / backward pair on the packed tensor (T <= 208, hd 64), else per-head GEMMs
         # on a head-major copy around the padded-row policy softmax
         o, cls_attn = ops.attention_train(qkv, H, policy=policy, scale=m.scale, want_cls_row=return_cls_attn)
@@ -205,7 +204,7 @@ def _mlp_is_plain(m, h):
 def mlp_hidden(m, h):
     """act(fc1(h)) of Mlp.forward (dynamic_vit.py:159-175) for inference: the tcgen05 GEMM with the exact-erf GELU in its
     epilogue when the shapes allow, else cuBLAS + the in-place d2s GELU kernel."""
-    if (_FUSED_FC1 and _FUSED_PAIR and h.dtype == torch.bfloat16 and m.fc1.weight.dtype == torch.bfloat16 and m.fc1.out_features % 256 == 0
+    if (_FUSED_PAIR and h.dtype == torch.bfloat16 and m.fc1.weight.dtype == torch.bfloat16 and m.fc1.out_features % 256 == 0
             and m.fc1.out_features <= 4096 and m.fc1.in_features % 64 == 0):
         return ops.linear_act(h, m.fc1.weight, m.fc1.bias, ops.ACT_GELU)
     u = m.fc1(h)
@@ -523,7 +522,7 @@ def predictor_a_hidden(m, x, policy, normed=None, row0=0):
     h = _seq_forward(m.in_conv, x, row0=row0) if normed is None else _seq_forward(list(m.in_conv)[1:], normed)
     B, N, C = h.shape
     half = C // 2
-    if _POOL_TRAIN and ops.pool_concat_train_ok(h) and policy is not None and policy.is_cuda:
+    if ops.pool_concat_train_ok(h) and policy is not None and policy.is_cuda:
         h = ops.pool_concat_train(h, policy)          # slice, multiply, sum, divide, expand, cat: one kernel each way
     else:
         pooled = (h[:, :, half:] * policy).sum(dim=1, keepdim=True) / torch.sum(policy, dim=1, keepdim=True)
@@ -616,7 +615,7 @@ def predictor_b_hidden(m, x, normed=None):
     h = _seq_forward(m.in_conv, x) if normed is None else m.in_conv[2](m.in_conv[1](normed))
     B, N, C = h.shape
     half = C // 2
-    if _POOL_TRAIN and ops.pool_concat_train_ok(h) and torch.is_grad_enabled() and h.requires_grad:
+    if ops.pool_concat_train_ok(h) and torch.is_grad_enabled() and h.requires_grad:
         h = ops.pool_concat_train(h)
     else:
         pooled = torch.mean(h[:, :, half:], dim=1, keepdim=True)
@@ -790,7 +789,7 @@ def variant_a_forward(model, img):
                 if (ln is not None and _predictor_a_fusable(pred) and st._probe().is_cuda and _d2s_float(st._probe())
                         and not _needs_grad(st.x, st.y, ln.weight)):
                     # residual add folded into the predictor's LayerNorm over x[:, 1:]; fused predictor body
-                    x, hn = st.normed(ln, row0=1, lazy=_LAZY_PRED and _LAZY_NORM1 and _predictor_a_gemm_ok(pred, st._probe()))
+                    x, hn = st.normed(ln, row0=1, lazy=_LAZY_NORM1 and _predictor_a_gemm_ok(pred, st._probe()))
                     _, keep_policy, prev_f32 = predictor_a_select(pred, hn, prev_f32, k)
                     prev_decision = None                 # materialised on demand below
                 else:
@@ -984,8 +983,8 @@ def _frozen_bf16_shadow(model, img):
     changes (load_state_dict, .to(), in-place edits through the tensor itself); invalidate_frozen_copies() drops it explicitly.
     Numerics: torch autocast keeps the fp32 residual stream and fp32 LayerNorm / softmax of an fp32 module; the copy computes
     like `model.to(bfloat16)` (bf16 residual stream).  Teacher logits / tokens / CLS rows agree with the per-call-cast path to
-    bf16 accuracy (3e-2 of the tensor's max, pinned by tests/test_gpu_models.py::test_frozen_teacher_under_autocast_...);
-    D2S_FROZEN_BF16=0 keeps torch's autocast numerics.  Returns None when this does not apply."""
+    bf16 accuracy (3e-2 of the tensor's max, pinned by tests/test_gpu_models.py::test_frozen_teacher_under_autocast_...).
+    Returns None when this does not apply."""
     if not (_FROZEN_BF16 and img.is_cuda and not model.training and torch.is_autocast_enabled("cuda")
             and torch.get_autocast_dtype("cuda") == torch.bfloat16):
         return None
@@ -993,7 +992,7 @@ def _frozen_bf16_shadow(model, img):
     if not params or any(p.requires_grad or p.dtype != torch.float32 or not p.is_cuda for p in params):
         return None
     # storage + version counter of every parameter and buffer.  Edits that bypass the version counter (`p.data.copy_()`, an EMA
-    # teacher updated through .data) are NOT seen: call invalidate_frozen_copies(model) after those, or set D2S_FROZEN_BF16=0.
+    # teacher updated through .data) are NOT seen: call invalidate_frozen_copies(model) after those.
     fp = hash(tuple((p.data_ptr(), p._version) for p in params + list(model.buffers())))
     hit = _SHADOWS.get(model)
     if hit is None or hit[0] != fp:

@@ -364,9 +364,9 @@ def softmax_with_policy(attn, policy, eps=1e-6):
     return _SoftmaxPolicy.apply(attn, policy, eps)
 
 
-_FUSED_WGRAD = os.environ.get("D2S_FUSED_WGRAD", "1") != "0"   # A/B switch for ops.linear_train (d2s bias gradient)
-_FUSED_GELU_BWD = os.environ.get("D2S_FUSED_GELU_BWD", "1") != "0"   # A/B switch: fc1 -> GELU as one autograd node
-_FUSED_GELU_FWD = os.environ.get("D2S_FUSED_GELU_FWD", "1") != "0"   # A/B switch: its forward as one tcgen05 GEMM (GELU + pre-activation out)
+# Test hook: True in use; tests/test_gpu_models.py::test_training_fusions_match_the_unfused_training_path sets it to False to run
+# linear_train on torch's own Linear, the reference it compares the fused training path against.
+_FUSED_WGRAD = True   # ops.linear_train (d2s bias gradient)
 
 
 def colsum(dy):
@@ -423,35 +423,6 @@ def _grad_slot(p):
     return g, e
 
 
-# Weight / bias gradients that land in gradient slots are consumed only by the optimizer, while dx is what the rest of the backward
-# waits for: with D2S_WGRAD_STREAM=1 they are enqueued on a side stream (forked after dy is ready) and fill the launch / tail gaps
-# of the dx chain; whoever owns the step joins the stream before the gradients are read (join_wgrad_stream(), called by
-# runner.TrainStepRunner after backward).  The operands are kept alive until the join, so the allocator cannot hand their memory
-# to the main stream while the side stream still reads it.
-_WGRAD_STREAM = os.environ.get("D2S_WGRAD_STREAM", "0") == "1"
-_wgrad_side = {}          # device index -> (stream, [operand references])
-
-
-def _wgrad_ctx(t):
-    """(stream context, refs list) for slot-bound parameter gradients of tensors on t's device; the side stream has been made to
-    wait for the current one (dy is ready)."""
-    dev = t.device
-    ent = _wgrad_side.get(dev.index)
-    if ent is None:
-        ent = _wgrad_side[dev.index] = (torch.cuda.Stream(device=dev), [])
-    ent[0].wait_stream(torch.cuda.current_stream(dev))
-    return ent
-
-
-def join_wgrad_stream(device=None):
-    """Make the current stream wait for every parameter-gradient kernel enqueued on the side stream (no-op when unused)."""
-    for idx, (stream, refs) in _wgrad_side.items():
-        if device is None or device.index == idx:
-            if refs:
-                torch.cuda.current_stream(torch.device("cuda", idx)).wait_stream(stream)
-                refs.clear()
-
-
 def _wgrad_into(p, dy, x, b_p=None):
     """dW = dy^T x landed in `p`'s gradient slot -- and, when `b_p` has a slot too, its bias gradient (column sums of dy) right
     behind it; returns (weight done, bias done).  False: the caller returns that gradient to autograd."""
@@ -460,24 +431,15 @@ def _wgrad_into(p, dy, x, b_p=None):
     w_ok = slot is not None and _MM_OUT
     if not w_ok and bslot is None:
         return False, False
-
-    def run():
-        if w_ok:
-            if e[1]:
-                torch.mm(dy.t(), x, out_dtype=torch.float32, out=slot)
-                e[1] = False
-            else:
-                slot.add_(torch.mm(dy.t(), x, out_dtype=torch.float32))
-        if bslot is not None:
-            _call("d2s_colsum_acc_bf16", _ptr(dy), dy.shape[0], dy.shape[1], _ptr(bslot), _stream(dy))
-            be[1] = False
-    if _WGRAD_STREAM and dy.is_cuda:
-        stream, refs = _wgrad_ctx(dy)
-        refs.append((dy, x))
-        with torch.cuda.stream(stream):
-            run()
-    else:
-        run()
+    if w_ok:
+        if e[1]:
+            torch.mm(dy.t(), x, out_dtype=torch.float32, out=slot)
+            e[1] = False
+        else:
+            slot.add_(torch.mm(dy.t(), x, out_dtype=torch.float32))
+    if bslot is not None:
+        _call("d2s_colsum_acc_bf16", _ptr(dy), dy.shape[0], dy.shape[1], _ptr(bslot), _stream(dy))
+        be[1] = False
     return w_ok, bslot is not None
 
 
@@ -574,7 +536,7 @@ def _probe_mm_out():
         return False
 
 
-_MM_OUT = _MM_OUT_DTYPE and _probe_mm_out() and os.environ.get("D2S_DIRECT_GRADS", "1") != "0"
+_MM_OUT = _MM_OUT_DTYPE and _probe_mm_out()
 
 
 class _LinearTrain(torch.autograd.Function):
@@ -639,7 +601,7 @@ class _LinearGeluTrain(torch.autograd.Function):
     def forward(ctx, x, w, b):
         xb, wb = x.to(torch.bfloat16), _bf16_of(w)
         bb = _bf16_of(b)
-        if _FUSED_GELU_FWD and wb.shape[0] % 256 == 0 and wb.shape[0] <= 4096 and wb.shape[1] % 64 == 0:
+        if wb.shape[0] % 256 == 0 and wb.shape[0] <= 4096 and wb.shape[1] % 64 == 0:
             # one tcgen05 GEMM writes both the Linear's output (kept for GELU') and its GELU: torch's separate GELU pass
             # (read + write of the (M, 4D) hidden tensor) disappears
             a, u = linear_act(xb, wb, bb, ACT_GELU, want_pre=True)
@@ -683,7 +645,7 @@ def _linear_train_ok(lin, x):
 def linear_gelu_train(lin, act, x):
     """`act(lin(x))` under autograd: one node with the fused GELU-backward + bias-gradient kernel when `act` is the exact-erf
     nn.GELU and the bf16 training path applies, else `act(linear_train(lin, x))`."""
-    if (_FUSED_GELU_BWD and _linear_train_ok(lin, x) and isinstance(act, torch.nn.GELU)
+    if (_linear_train_ok(lin, x) and isinstance(act, torch.nn.GELU)
             and getattr(act, "approximate", "none") == "none" and lin.out_features <= 8192):
         return _LinearGeluTrain.apply(x, lin.weight, lin.bias)
     return act(linear_train(lin, x))
@@ -796,7 +758,6 @@ class _AttentionFlash(torch.autograd.Function):
         return dqkv, gpol, None, None, None, None
 
 
-_FLASH_TRAIN = os.environ.get("D2S_FLASH_TRAIN", "1") != "0"   # A/B switch: tcgen05 flash forward/backward for training attention
 FLASH_MAX_T = 208
 
 
@@ -809,7 +770,7 @@ def attention_train(qkv, num_heads, policy=None, scale=None, eps=1e-6, want_cls_
         raise RuntimeError("attention_train: bf16 and T <= 256 only (other cases use softmax_with_policy around torch matmuls)")
     hd = qkv.shape[-1] // 3 // num_heads
     scale = hd ** -0.5 if scale is None else scale
-    if _FLASH_TRAIN and hd == 64 and qkv.shape[1] <= FLASH_MAX_T and scale > 0:
+    if hd == 64 and qkv.shape[1] <= FLASH_MAX_T and scale > 0:
         return _AttentionFlash.apply(qkv, policy, num_heads, float(scale), float(eps), bool(want_cls_row))
     return _AttentionTrain.apply(qkv, policy, num_heads, float(scale), float(eps), bool(want_cls_row))
 

@@ -103,7 +103,7 @@ class InferenceRunner:
             # One captured forward PER staging buffer: the step reads the images where the copy stream put them, instead of
             # moving them into static_in first (a 2 x (B,3,H,W) device-to-device pass per step, ~1 % of the step).
             self._slot_graphs = None
-            if self.graph is not None and os.environ.get("D2S_E2E_SLOT_GRAPHS", "1") != "0":
+            if self.graph is not None:
                 self._slot_graphs = []
                 with torch.no_grad():
                     for k in range(2):
@@ -338,7 +338,6 @@ class TrainStepRunner:
             self.grads.zero()
         self.loss = self.step_fn(self.static_x, self.static_y)
         self.loss.backward()
-        ops.join_wgrad_stream()                      # parameter gradients enqueued on the side stream (D2S_WGRAD_STREAM=1)
         if self.grads is not None:
             self.grads.all_reduce()
         self.opt.step()

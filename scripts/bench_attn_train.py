@@ -51,13 +51,12 @@ def main():
         o2 = ref_attention(q2[:nb], H, None if p2 is None else p2[:nb])
         (o2 * go[:nb].float()).sum().backward()
         row = {"B": B, "T": T, "policy": with_pol}
-        for name, flag in (("flash", True), ("gemm", False)):
-            ops._FLASH_TRAIN = flag
+        for name, fn in (("flash", ops._AttentionFlash.apply), ("gemm", ops._AttentionTrain.apply)):
             q1 = qkv.clone().requires_grad_(True)
             p1 = None if pol is None else pol.clone().requires_grad_(True)
 
             def fwd():
-                return ops.attention_train(q1, H, policy=p1)[0]
+                return fn(q1, p1, H, float(hd ** -0.5), 1e-6, False)[0]
 
             o1 = fwd()
             (o1.float() * go.float()).sum().backward()
@@ -83,7 +82,6 @@ def main():
                 e1.record()
                 torch.cuda.synchronize()
                 row[f"{name}_{what}_us"] = 100.0 * e0.elapsed_time(e1)
-        ops._FLASH_TRAIN = True
         hbm = B * T * H * hd * 2 * (4 + 8)                  # fwd: q,k,v in + o out; bwd: q,k,v,o,do in + dq,dk,dv out
         row["flash_fwd+bwd_gbs"] = hbm / row["flash_fwd+bwd_us"] / 1e3
         rows.append(row)

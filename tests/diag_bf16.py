@@ -59,13 +59,12 @@ def main(names):
         print(f"torch eager bf16 (oracle on GPU)  {err(lt, truth)}")
         with torch.no_grad():
             print(f"d2s bf16 fused                    {err(m16(x16), truth)}")
-            for flags in (("_FUSED_MLP",), ("_FUSED_MLP", "_FUSED_PAIR"), ("_FUSED_MLP", "_FUSED_PAIR", "_FUSED_FC1")):
+            for flags in (("_FUSED_MLP",), ("_FUSED_MLP", "_FUSED_PAIR")):
                 for f in flags:
                     setattr(pkg.engine, f, False)
                 print(f"d2s bf16 without {'+'.join(flags):<30} {err(m16(x16), truth)}")
                 for f in flags:
                     setattr(pkg.engine, f, True)
-            os.environ["D2S_ATTN_FORCE_SIMT"] = "0"
 
 
 if __name__ == "__main__":

@@ -101,6 +101,20 @@ def test_product_never_imports_oracle():
             assert not re.search(r"^\s*(from|import)\s+oracle\b", src, flags=re.M), f"{fn} imports the oracle"
 
 
+def test_package_reads_only_its_documented_environment_variables():
+    """The D2S_* variables the package reads: a semantic opt-in, input validation, and the profiling-build hooks.  Every other
+    configuration is fixed in the code, so what runs does not depend on the environment."""
+    pkg = os.path.join(ROOT, "dense2sparse-vit_b200")
+    names = set()
+    for sub in (pkg, os.path.join(pkg, "csrc")):
+        for fn in os.listdir(sub):
+            if fn.endswith((".py", ".cu", ".cuh")):
+                src = open(os.path.join(sub, fn)).read()
+                names |= set(re.findall(r"(?:os\.environ(?:\.get)?\s*[\(\[]|getenv\s*\()\s*[\"'](\w+)[\"']", src))
+    assert {n for n in names if n.startswith("D2S_")} == {"D2S_THRESHOLD_INFERENCE", "D2S_CHECK_INDICES", "D2S_NVCC_EXTRA",
+                                                           "D2S_GEMM_TRACE"}
+
+
 def test_shard_range_partitions(d2s):
     sr = d2s.runner.shard_range
     for gb, w in [(1024, 1), (1024, 8), (1000, 8), (7, 8), (0, 4)]:

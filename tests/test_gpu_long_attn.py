@@ -65,7 +65,7 @@ def test_long_attention_argument_errors_precede_any_launch(d2s):
 
 
 def test_engine_routes_long_bf16_attention_behind_its_switch(d2s, monkeypatch):
-    """The fused path takes bf16, head dim 64, 256 < T <= 2048 unless D2S_LONG_ATTN=0; fp32 above 256 keeps the torch path."""
+    """The fused path takes bf16, head dim 64, 256 < T <= 2048 unless engine._LONG_ATTN is False; fp32 above 256 keeps the torch path."""
     ok = d2s.engine._attn_kernel_ok
     bf = torch.empty(1, 577, 3 * 6 * 64, dtype=torch.bfloat16)
     assert ok(bf, 6) and ok(torch.empty(1, 2048, 3 * 6 * 64, dtype=torch.bfloat16), 6)
@@ -262,7 +262,7 @@ KEEP_ALL = [576 / 196 + 1e-4] * 3      # int(196 r) = 576: every token of a 384-
 @pytest.mark.parametrize("kind,ratios", [("teacher", None), ("a", KEEP_ALL), ("a", RATIOS), ("b", RATIOS)])
 def test_models_at_384_pixels_bf16_graph(d2s, cuda_dev, monkeypatch, kind, ratios):
     """DeiT-S/16 at 384 px (T = 577) in bf16 through the CUDA-graph runner, B = 64, with the key-blocked attention kernel and with
-    D2S_LONG_ATTN off (torch matmuls around the policy softmax), each against the fp32 GPU path on identical (bf16-representable)
+    engine._LONG_ATTN off (torch matmuls around the policy softmax), each against the fp32 GPU path on identical (bf16-representable)
     weights and images -- the rule of test_bench_config_bf16_graph_at_batch_1024:
       * no token can change sides (the teacher; Variant A keeping all 576 tokens): logits within 1e-2 relative (L2), largest
         deviation 3e-2 of max |logit|;

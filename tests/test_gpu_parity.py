@@ -1234,7 +1234,7 @@ def test_mlp_kernel_applies_its_input_layernorm_from_row_statistics(ops, B, T, r
 
 
 def test_lazy_norms_are_invisible_at_model_level(d2s, monkeypatch):
-    """engine: norm2 handed to the one-kernel MLP and norm1 to the qkv GEMM as row statistics (D2S_LAZY_NORM2 / D2S_LAZY_NORM1)
+    """engine: norm2 handed to the one-kernel MLP and norm1 to the qkv GEMM as row statistics (engine._LAZY_NORM2 / _LAZY_NORM1)
     against the same forward with the normalised copies: identical logits and kept sets (the kernels are bit-identical; the
     CLS-only last MLP normalises its rows itself)."""
     torch.manual_seed(3)
