@@ -25,7 +25,8 @@
 // columns and keeps them in registers: the residual rows are fetched with coalesced loads while the MMAs still run and
 // transposed to one-row-per-lane through a 4 KB per-warp buffer; pass 1 reads the accumulator, forms x' and the fp32
 // sum / sum of squares and releases TMEM (the next tile's MMAs start here); x' goes out through the same per-warp
-// transposition as coalesced 128-byte lines; pass 2 normalises the registers and writes h the same way.  No
+// transposition as coalesced 128-byte lines; pass 2 normalises the registers and writes h the same way.  (A row far off zero
+// gets two-pass statistics from its freshly written x' lines instead of the one-pass sums: see the statistics below.)  No
 // CTA-wide barrier and no tile-sized staging buffer: shared memory goes to a 4-deep operand ring instead (a 96 KB
 // residual tile left only 3 stages = 48 KB of A in flight per SM, too little to cover HBM latency at K = 1536).
 // The separate add+LayerNorm kernel (8 bytes of traffic per element) and the GEMM's own output round trip disappear.
@@ -94,6 +95,26 @@ struct GpParams {
   const float2* in_stats;
   const __nv_bfloat16 *in_gamma, *in_beta;
 };
+
+// Sum of (x - m)^2 over `nblk` 64-column blocks of one bf16 row, `stride` elements apart (the rare two-pass statistics of a
+// row far off zero; out of line, so that the epilogue keeps its registers)
+__device__ __noinline__ float bf16_sq_dev_blocks(const __nv_bfloat16* x, int nblk, int stride, float m) {
+  const uint64_t nm = f2_bcast(-m);
+  uint64_t acc0 = f2_bcast(0.f), acc1 = f2_bcast(0.f);
+  for (int b = 0; b < nblk; ++b)
+#pragma unroll 2
+    for (int k = 0; k < 8; ++k) {
+      const uint4 t = ld_cg16(x + (size_t)b * stride + k * 8);
+      const uint64_t d0 = f2_add(f2_pack(bf16_lo(t.x), bf16_hi(t.x)), nm), d1 = f2_add(f2_pack(bf16_lo(t.y), bf16_hi(t.y)), nm);
+      const uint64_t d2 = f2_add(f2_pack(bf16_lo(t.z), bf16_hi(t.z)), nm), d3 = f2_add(f2_pack(bf16_lo(t.w), bf16_hi(t.w)), nm);
+      acc0 = f2_fma(d2, d2, f2_fma(d0, d0, acc0));
+      acc1 = f2_fma(d3, d3, f2_fma(d1, d1, acc1));
+    }
+  float a0, a1, b0, b1;
+  f2_unpack(acc0, a0, a1);
+  f2_unpack(acc1, b0, b1);
+  return (a0 + a1) + (b0 + b1);
+}
 
 template <int MODE, int NSUB_, int ACT>
 __global__ void __cluster_dims__(2, 1, 1) __maxnreg__((GpCfg<MODE, NSUB_>::MAXREG))
@@ -476,12 +497,28 @@ gemm_pair_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constan
 #pragma unroll
           for (int k = 0; k < PARTS; ++k) { const float2 t = red_s[k * 128 + r]; sum += t.x; sq += t.y; }
           const float inv_n = 1.0f / (float)ldn;
-          const float mean = sum * inv_n;
+          float mean = sum * inv_n;
           const float var = fmaxf(sq * inv_n - mean * mean, 0.f);
-          const float rstd = rsqrtf(var + p.eps);
-          const uint64_t sc = f2_bcast(rstd), sh = f2_bcast(-mean * rstd);
+          float rstd = rsqrtf(var + p.eps);
           const uint32_t sel_lo = sel_s[0], sel_hi = sel_s[1];
-          asm volatile("bar.sync %0, %1;" ::"r"(1 + quad), "n"(32 * PARTS) : "memory");     // red_s may be rewritten by the next tile
+          asm volatile("bar.sync %0, %1;" ::"r"(1 + quad), "n"(32 * PARTS) : "memory");     // red_s may be rewritten
+          // E[x^2] - mean^2 is exact enough while 8 mean^2 <= var (the sum of squares is then at most 1.125 x the squared
+          // deviations).  A row farther off zero would lose log2(1 + mean^2 / var) bits to the cancellation: it gets two-pass
+          // statistics instead, from the x' this warp has just written (every lane re-reads its own row, its part's columns).
+          // The warps of a lane quadrant hold the same rows and the same sums, so they all take this branch or none.
+          const bool far = row0 + lane < p.M && 8.f * mean * mean > var;
+          if (far) mean = fmaf(fmaf(-mean, (float)ldn, sum), inv_n, mean);     // sum / N: exact when representable (constant rows)
+          if (__any_sync(0xffffffffu, far)) {
+            red_s[part * 128 + r].x = far ? bf16_sq_dev_blocks(p.out_sum + (size_t)(row0 + lane) * ldn + part * 64, n_tiles * BPT,
+                                                               PARTS * 64, mean) : 0.f;
+            asm volatile("bar.sync %0, %1;" ::"r"(1 + quad), "n"(32 * PARTS) : "memory");
+            float m2 = 0.f;
+#pragma unroll
+            for (int k = 0; k < PARTS; ++k) m2 += red_s[k * 128 + r].x;
+            asm volatile("bar.sync %0, %1;" ::"r"(1 + quad), "n"(32 * PARTS) : "memory");
+            if (far) rstd = rsqrtf(m2 * inv_n + p.eps);
+          }
+          const uint64_t sc = f2_bcast(rstd), sh = f2_bcast(-mean * rstd);
           if (p.stats != nullptr && part == 0 && row0 + lane < p.M) p.stats[row0 + lane] = make_float2(mean, rstd);
           GP_TRACE(4)
           if (p.out_norm != nullptr) {
@@ -521,6 +558,7 @@ gemm_pair_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constan
 #pragma unroll
             for (int i = 0; i < 8; ++i) {
               const float m_i = __shfl_sync(0xffffffffu, mean, 4 * i + crow), r_i = __shfl_sync(0xffffffffu, rstd, 4 * i + crow);
+              const float sh_i = -m_i * r_i;
               if (4 * i < rows_left) {
 #pragma unroll
                 for (int bi = 0; bi < BPT; ++bi) {
@@ -533,7 +571,8 @@ gemm_pair_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constan
                   for (int q = 0; q < 4; ++q) {
                     const float2 g = *reinterpret_cast<const float2*>(&gamma_s[col + 2 * q]);
                     const float2 bt = *reinterpret_cast<const float2*>(&beta_s[col + 2 * q]);
-                    o[q] = pack_bf16x2(fmaf((bf16_lo(w[q]) - m_i) * r_i, g.x, bt.x), fmaf((bf16_hi(w[q]) - m_i) * r_i, g.y, bt.y));
+                    // the form of the last half (and of every bf16 LayerNorm producer): fma(fma(x, rstd, -mean rstd), gamma, beta)
+                    o[q] = pack_bf16x2(fmaf(fmaf(bf16_lo(w[q]), r_i, sh_i), g.x, bt.x), fmaf(fmaf(bf16_hi(w[q]), r_i, sh_i), g.y, bt.y));
                   }
                   *reinterpret_cast<uint4*>(p.out_norm + off) = make_uint4(o[0], o[1], o[2], o[3]);
                 }
@@ -582,7 +621,8 @@ static int gp_launch(const CUtensorMap& ma, const CUtensorMap& mw, const CUtenso
   using Cfg = GpCfg<MODE, NSUB>;
   constexpr uint32_t kStage = kGpABytes + NSUB * (Cfg::UN / 2) * 128;
   const size_t smem = 1024 + (size_t)Cfg::STAGES * kStage + (size_t)Cfg::BLOCKS * kGpBlkBytes + sizeof(GpBars) +
-                      (MODE == kGpModeLn ? (size_t)3 * p.N * 4 + 4 * 128 * sizeof(float2) + 16 : (size_t)p.N * 4 + (size_t)p.K * 4);
+                      (MODE == kGpModeLn ? (size_t)3 * p.N * 4 + 4 * 128 * sizeof(float2) + 16
+                                          : (size_t)p.N * 4 + (p.in_stats ? (size_t)p.K * 4 : 0));   // gbin_s: in_stats only
   D2S_REQUIRE(smem <= 227 * 1024, D2S_ERR_ARG, "%s: needs %zu B of shared memory", what, smem);
   static SmemOptIn opt;
   cudaError_t e = opt_in_smem(opt, gemm_pair_kernel<MODE, NSUB, ACT>, 227 * 1024);

@@ -99,6 +99,28 @@ __device__ __noinline__ void mp_normalize_block(unsigned char* hb, int r, int ch
   }
 }
 
+// Two-pass (mean, rstd) of one bf16 row of n elements whose fp32 sum s and one-pass mean are known: the rare statistics of a row far
+// off zero.  The mean is s / n with one correction step (exact when representable: a constant row gets var = 0).  Out of line, so
+// that the output warps keep their registers.
+__device__ __noinline__ float2 bf16_row_stats_two_pass(const __nv_bfloat16* x, int n, float s, float mean1, float eps) {
+  const float inv_n = 1.0f / (float)n;
+  const float m = fmaf(fmaf(-mean1, (float)n, s), inv_n, mean1);
+  const uint64_t nm = f2_bcast(-m);
+  uint64_t acc0 = f2_bcast(0.f), acc1 = f2_bcast(0.f);
+#pragma unroll 2
+  for (int k = 0; k < n; k += 8) {
+    const uint4 t = ld_cg16(x + k);
+    const uint64_t d0 = f2_add(f2_pack(bf16_lo(t.x), bf16_hi(t.x)), nm), d1 = f2_add(f2_pack(bf16_lo(t.y), bf16_hi(t.y)), nm);
+    const uint64_t d2 = f2_add(f2_pack(bf16_lo(t.z), bf16_hi(t.z)), nm), d3 = f2_add(f2_pack(bf16_lo(t.w), bf16_hi(t.w)), nm);
+    acc0 = f2_fma(d2, d2, f2_fma(d0, d0, acc0));
+    acc1 = f2_fma(d3, d3, f2_fma(d1, d1, acc1));
+  }
+  float a0, a1, b0, b1;
+  f2_unpack(acc0, a0, a1);
+  f2_unpack(acc1, b0, b1);
+  return make_float2(m, rsqrtf(((a0 + a1) + (b0 + b1)) * inv_n + eps));
+}
+
 // kLnIn: the LayerNorm of the input is applied on the fly (MpParams::in_stats); a separate instantiation, so that the plain form
 // compiles exactly as it did before the option existed
 template <bool kLnIn>
@@ -452,9 +474,17 @@ mlp_pair_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant
         float s0, s1, q0, q1;
         f2_unpack(acc_s, s0, s1);
         f2_unpack(acc_q, q0, q1);
-        const float mean = (s0 + s1) * (1.0f / TN);
+        float mean = (s0 + s1) * (1.0f / TN);
         const float var = fmaxf((q0 + q1) * (1.0f / TN) - mean * mean, 0.f);
-        const float rstd = rsqrtf(var + p.eps);
+        float rstd = rsqrtf(var + p.eps);
+        // E[x^2] - mean^2 is exact enough while 8 mean^2 <= var (the sum of squares is then at most 1.125 x the squared
+        // deviations).  A row farther off zero would lose log2(1 + mean^2 / var) bits to the cancellation: it gets two-pass
+        // statistics instead, from the x' row this warp has just written (L2-hot; the thread re-reads its own row).
+        if (row0 + lane < p.M && 8.f * mean * mean > var) {
+          const float2 st = bf16_row_stats_two_pass(p.out_sum + (size_t)(row0 + lane) * TN, TN, s0 + s1, mean, p.eps);
+          mean = st.x;
+          rstd = st.y;
+        }
         if (p.out_stats != nullptr && row0 + lane < p.M) p.out_stats[row0 + lane] = make_float2(mean, rstd);   // (this thread's row)
         if (!p.want_ln) continue;
         const uint64_t sc = f2_bcast(rstd), sh = f2_bcast(-mean * rstd);

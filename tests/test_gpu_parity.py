@@ -1228,7 +1228,7 @@ def test_mlp_kernel_applies_its_input_layernorm_from_row_statistics(ops, B, T, r
     assert torch.equal(xs1, xs0) and st.shape == (B * T, 2)
     xf = xs1.float().reshape(B * T, D)
     torch.testing.assert_close(st[:, 0], xf.mean(-1), rtol=1e-4, atol=1e-4)
-    torch.testing.assert_close(st[:, 1], torch.rsqrt(xf.var(-1, unbiased=False) + 1e-6), rtol=1e-3, atol=1e-4)
+    torch.testing.assert_close(st[:, 1], torch.rsqrt(xf.var(-1, unbiased=False) + 1e-6), rtol=1e-4, atol=1e-4)
     out = ops.mlp_residual_ln(None, W1, b1, W2, b2, xs1, g1, bt1, 1e-6, norm_row0=row0, in_stats=st, in_ln_weight=g2, in_ln_bias=bt2)
     assert torch.equal(out[0], ref[0]) and torch.equal(out[1], ref[1])
 
