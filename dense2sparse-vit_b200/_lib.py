@@ -81,6 +81,8 @@ SIGNATURES = {
     "d2s_pool_concat_varlen_inplace": [_p, _p, _i, _i, _i, _i, _p],
     "d2s_attn_varlen_fwd": [_p, _p, _i, _i, _i, _i, _i, _f, _p, _p, _p],
     "d2s_attn_long_fwd": [_p, _p, _p, _i, _i, _i, _i, _f, _f, _p, _p, _p],
+    "d2s_attn_long_fwd_stats": [_p, _p, _i, _i, _i, _i, _f, _f, _p, _p, _p, _p],
+    "d2s_attn_long_bwd": [_p, _p, _p, _p, _p, _p, _p, _i, _i, _i, _i, _f, _p, _p, _p, _p],
     "d2s_gather_layernorm_varlen": [_p, _p, _p, _p, _p, _i, _i, _i, _i, _i, _f, _p, _p, _p],
     "d2s_gather_layernorm_stats_varlen": [_p, _p, _p, _i, _i, _i, _i, _f, _p, _p, _p],
 }

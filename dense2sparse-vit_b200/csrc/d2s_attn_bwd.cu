@@ -417,6 +417,16 @@ static size_t bwd_smem_bytes(int knt, int Tp) {
          256 * 4 + sizeof(BwdBars);
 }
 
+// the delta pre-pass of both training backwards (d2s_attn_policy_bwd, d2s_attn_long_bwd): stats[..][3] = gout_i . out_i (+ g_cls . P_0)
+int launch_attn_bwd_prep(const void* out, const void* gout, const float* cls_row, const float* g_cls, int B, int T, int H,
+                         float* stats, cudaStream_t stream) {
+  const long long rows = (long long)B * T * H;
+  attn_bwd_prep_kernel<<<(unsigned)((rows + 31) / 32), 256, 0, stream>>>((const __nv_bfloat16*)out, (const __nv_bfloat16*)gout,
+                                                                          cls_row, g_cls, rows, T, H, stats);
+  count_launch();
+  return check_launch("attn_bwd_prep");
+}
+
 template <int kNT, bool kPol>
 static int launch_bwd(const CUtensorMap* maps, const float* policy, const float* stats, const float* g_cls, int units, int T, int H,
                       int Tp, float scale, void* dqkv, float* gpolicy, cudaStream_t stream) {
@@ -469,11 +479,7 @@ extern "C" int d2s_attn_policy_bwd(const void* qkv, const float* policy, const v
                       CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
     D2S_REQUIRE(cr == CUDA_SUCCESS, D2S_ERR_CUDA, "attn_policy_bwd: cuTensorMapEncodeTiled failed (%d)", (int)cr);
   }
-  const long long rows = (long long)B * T * H;
-  attn_bwd_prep_kernel<<<(unsigned)((rows + 31) / 32), 256, 0, stream>>>((const __nv_bfloat16*)out, (const __nv_bfloat16*)gout,
-                                                                          cls_row, g_cls, rows, T, H, stats);
-  count_launch();
-  int rc = check_launch("d2s_attn_policy_bwd(prep)");
+  const int rc = launch_attn_bwd_prep(out, gout, cls_row, g_cls, B, T, H, stats, stream);
   if (rc != D2S_OK) return rc;
   const int units = B * H;
   if (T <= kTileRows)

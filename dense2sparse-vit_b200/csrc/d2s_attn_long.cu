@@ -19,6 +19,8 @@
 // one test of the finished row sums (beyond 2^100, inf or NaN) after the last block; a failed row is redone from the packed qkv in
 // global memory in fp32 over all keys.  A masked key far above every kept one raises m' by whole binades at the end (exact: O, the
 // sum and the CLS values are multiplied by the same power of two).
+// d2s_attn_long_fwd_stats (training) is the same kernel with kStats: each row also stores the (m', 1/den, c/den) that produced it,
+// which d2s_attn_long_bwd (d2s_attn_long_bwd.cu) recomputes the probabilities from.
 #undef D2S_ATTN_TRACE_BUILD   // the clock64 phase traces instrument the T <= 256 kernels only
 #include "d2s_attn_tc.cuh"
 
@@ -60,12 +62,14 @@ __device__ __forceinline__ int long_len(const int* __restrict__ lens, int b, int
 __device__ __forceinline__ int block_chunks(int Tv, int jb) { return min(8, (Tv - jb * 128 + 15) >> 4); }
 
 // kPol: policy given (eps terms, masked exponentials, colsum(V)).  kVar: variable-length form (lens, no policy).
-template <bool kPol, bool kVar>
+// kStats: also write the row statistics (m', 1/den, c/den, 0) of d2s_attn_policy_fwd that produced out (training forward).
+template <bool kPol, bool kVar, bool kStats = false>
 __global__ void __launch_bounds__(kLongThreads, 2)
 attn_long_fwd_kernel(const __grid_constant__ CUtensorMap map, const float* __restrict__ policy, const int* __restrict__ lens,
                      int num_units, LongShape shp, float scale, float eps, __nv_bfloat16* __restrict__ out,
-                     float* __restrict__ cls_row, const __nv_bfloat16* __restrict__ qkv) {
+                     float* __restrict__ cls_row, const __nv_bfloat16* __restrict__ qkv, float* __restrict__ stats) {
   static_assert(!(kVar && kPol), "the variable-length form takes no policy");
+  static_assert(!(kVar && kStats), "training has no variable-length form");
   extern __shared__ unsigned char smem_dyn[];
   const uint32_t raw = smem_u32(smem_dyn);
   unsigned char* tiles = smem_dyn + ((1024u - (raw & 1023u)) & 1023u);   // SWIZZLE_128B atoms are address based
@@ -452,6 +456,11 @@ attn_long_fwd_kernel(const __grid_constant__ CUtensorMap map, const float* __res
         }
         f = 1.0f;
       }
+      if (kStats && warp_active && i < Tv) {
+        // after the rare-path redo and the whole-binade raise: the m' and den that produced this row of out
+        const float inv = 1.0f / den;
+        reinterpret_cast<float4*>(stats)[((size_t)b * H + h) * T + i] = make_float4(mxk, inv, c_eps_row * inv, 0.0f);
+      }
       if (cls_dst != nullptr && qt == 0 && warp == 0) {
         // CLS row (query 0 = lane 0 of warp 0): probabilities of row 0, Attention.forward's second output
         __syncwarp();
@@ -477,16 +486,16 @@ attn_long_fwd_kernel(const __grid_constant__ CUtensorMap map, const float* __res
   }
 }
 
-template <bool kPol, bool kVar>
+template <bool kPol, bool kVar, bool kStats = false>
 int launch_long(const CUtensorMap& map, const float* policy, const int* lens, int units, LongShape shp, float scale, float eps,
-                void* out, float* cls_row, const void* qkv, cudaStream_t stream) {
-  auto kern = attn_long_fwd_kernel<kPol, kVar>;
+                void* out, float* cls_row, const void* qkv, cudaStream_t stream, float* stats = nullptr) {
+  auto kern = attn_long_fwd_kernel<kPol, kVar, kStats>;
   static SmemOptIn opt;  // one per instantiation
   cudaError_t e = opt_in_smem(opt, kern, (int)kLongSmem);
   D2S_REQUIRE(e == cudaSuccess, D2S_ERR_CUDA, "attn_long_fwd: cudaFuncSetAttribute: %s", cudaGetErrorString(e));
   const int grid = units < 2 * kNumSMs ? units : 2 * kNumSMs;
   kern<<<grid, kLongThreads, kLongSmem, stream>>>(map, policy, lens, units, shp, scale, eps, (__nv_bfloat16*)out, cls_row,
-                                                 (const __nv_bfloat16*)qkv);
+                                                 (const __nv_bfloat16*)qkv, stats);
   count_launch();
   return check_launch("d2s_attn_long_fwd(tcgen05)");
 }
@@ -496,9 +505,10 @@ int launch_long(const CUtensorMap& map, const float* policy, const int* lens, in
 
 using namespace d2s;
 
-extern "C" int d2s_attn_long_fwd(const void* qkv, const float* policy, const int* len, int B, int T, int H, int hd, float scale,
-                                 float eps, void* out, float* cls_row, d2s_stream_t stream_) {
+static int attn_long_fwd(const void* qkv, const float* policy, const int* len, int B, int T, int H, int hd, float scale, float eps,
+                         void* out, float* cls_row, float* stats, d2s_stream_t stream_) {
   D2S_REQUIRE(qkv && out, D2S_ERR_ARG, "attn_long_fwd: null pointer");
+  D2S_REQUIRE(aligned16(stats), D2S_ERR_ALIGN, "attn_long_fwd: stats must be 16-byte aligned");
   D2S_REQUIRE(hd == kTcHD, D2S_ERR_ARG, "attn_long_fwd: head dim %d unsupported (64 only)", hd);
   D2S_REQUIRE(B >= 0 && H >= 1 && T >= 1 && T <= kLongMaxT, D2S_ERR_ARG, "attn_long_fwd: bad shape B=%d T=%d H=%d (1 <= T <= %d)",
               B, T, H, kLongMaxT);
@@ -523,7 +533,21 @@ extern "C" int d2s_attn_long_fwd(const void* qkv, const float* policy, const int
   cudaStream_t stream = (cudaStream_t)stream_;
   const LongShape shp{T, H, nqt};
   const int units = B * H * nqt;
+  if (stats)
+    return policy ? launch_long<true, false, true>(map, policy, nullptr, units, shp, scale, eps, out, cls_row, qkv, stream, stats)
+                  : launch_long<false, false, true>(map, nullptr, nullptr, units, shp, scale, eps, out, cls_row, qkv, stream, stats);
   if (len) return launch_long<false, true>(map, nullptr, len, units, shp, scale, 0.0f, out, cls_row, qkv, stream);
   if (policy) return launch_long<true, false>(map, policy, nullptr, units, shp, scale, eps, out, cls_row, qkv, stream);
   return launch_long<false, false>(map, nullptr, nullptr, units, shp, scale, eps, out, cls_row, qkv, stream);
+}
+
+extern "C" int d2s_attn_long_fwd(const void* qkv, const float* policy, const int* len, int B, int T, int H, int hd, float scale,
+                                 float eps, void* out, float* cls_row, d2s_stream_t stream) {
+  return attn_long_fwd(qkv, policy, len, B, T, H, hd, scale, eps, out, cls_row, nullptr, stream);
+}
+
+extern "C" int d2s_attn_long_fwd_stats(const void* qkv, const float* policy, int B, int T, int H, int hd, float scale, float eps,
+                                       void* out, float* cls_row, float* stats, d2s_stream_t stream) {
+  D2S_REQUIRE(stats, D2S_ERR_ARG, "attn_long_fwd_stats: null stats");
+  return attn_long_fwd(qkv, policy, nullptr, B, T, H, hd, scale, eps, out, cls_row, stats, stream);
 }

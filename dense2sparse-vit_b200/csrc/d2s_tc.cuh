@@ -319,6 +319,10 @@ static inline void bind_primary_context() {
   }
 }
 
+// d2s_attn_bwd.cu: launches the delta pre-pass of the training attention backwards (stats[..][3] = gout_i . out_i + g_cls . P_0)
+int launch_attn_bwd_prep(const void* out, const void* gout, const float* cls_row, const float* g_cls, int B, int T, int H,
+                         float* stats, cudaStream_t stream);
+
 static inline GgEncodeFn gg_encode_fn() {
   bind_primary_context();
   static GgEncodeFn fn = nullptr;

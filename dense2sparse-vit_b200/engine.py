@@ -31,7 +31,7 @@ _FROZEN_BF16 = True          # cached bf16 copy of a frozen teacher under bf16 a
 _PRED_FUSED = True           # second half of the Variant A predictor + selection as one tcgen05 kernel (inference, D = 384)
 _LAZY_NORM1 = True           # norm1 applied inside the qkv GEMM from the MLP kernel's row statistics
 _LAZY_NORM2 = True           # norm2 applied inside the one-kernel MLP from per-row statistics (no normalised copy)
-_LONG_ATTN = True            # bf16 inference attention beyond 256 tokens on the key-blocked kernel
+_LONG_ATTN = True            # bf16 attention beyond 256 tokens on the key-blocked kernels (inference, and training fwd + bwd)
 _THRESHOLD_INFERENCE = os.environ.get("D2S_THRESHOLD_INFERENCE", "0") == "1"   # opt-in: what dynamic_vit.py:935-949 intends
 INIT_N = 14 * 14  # the reference hard-codes 196 spatial tokens (dynamic_vit.py:828, default_dynamic_vit.py:446)
 
@@ -62,6 +62,18 @@ def _attn_kernel_ok(qkv, H):
     if qkv.shape[1] > 256:
         return _LONG_ATTN and qkv.dtype == torch.bfloat16 and hd == 64 and qkv.shape[1] <= ops.LONG_ATTN_MAX_T
     return (qkv.dtype == torch.bfloat16 and hd == 64) or (qkv.dtype == torch.float32 and hd in (32, 64))
+
+
+def _attn_train_kernel_ok(qkv, H):
+    """Shapes the training branch hands to ops.attention_train: bf16 with T <= 256 (tcgen05 flash kernels at hd 64, T <= 208,
+    else head-major GEMMs around the padded-row softmax), and bf16, hd 64, 256 < T <= 2048 (the key-blocked forward with row
+    statistics + d2s_attn_long_bwd) unless _LONG_ATTN is off."""
+    if qkv.dtype != torch.bfloat16:
+        return False
+    if qkv.shape[1] <= 256:
+        return True
+    hd = qkv.shape[-1] // 3 // H
+    return _LONG_ATTN and qkv.shape[-1] == 3 * H * hd and hd == 64 and qkv.shape[1] <= ops.LONG_ATTN_MAX_T
 
 
 def _softmax_policy_torch(attn, policy, eps=1e-6):
@@ -143,9 +155,9 @@ def attention_pre_proj(m, x, policy=None, return_cls_attn=False, lens=None):
                                f"take (bf16 with head dim 64 and T <= 2048, or fp32 with head dim 32 / 64 and T <= 256); got {tuple(qkv.shape)} {qkv.dtype}")
         o, cls_attn = ops.attention_core(qkv, H, scale=m.scale, want_cls_row=return_cls_attn, lengths=lens)
         return o, (cls_attn.to(qkv.dtype) if cls_attn is not None else None)
-    if _needs_grad(qkv, policy) and qkv.is_cuda and qkv.dtype == torch.bfloat16 and T <= 256:
-        # training, bf16: the tcgen05 flash forward / backward pair on the packed tensor (T <= 208, hd 64), else per-head GEMMs
-        # on a head-major copy around the padded-row policy softmax
+    if _needs_grad(qkv, policy) and qkv.is_cuda and _attn_train_kernel_ok(qkv, H):
+        # training, bf16: the tcgen05 flash forward / backward pair on the packed tensor (T <= 208, hd 64; key-blocked beyond 256
+        # tokens), else per-head GEMMs on a head-major copy around the padded-row policy softmax
         o, cls_attn = ops.attention_train(qkv, H, policy=policy, scale=m.scale, want_cls_row=return_cls_attn)
     elif _needs_grad(qkv, policy) or not qkv.is_cuda or not _attn_kernel_ok(qkv, H):
         q, k, v = qkv.reshape(B, T, 3, H, C // H).permute(2, 0, 3, 1, 4).unbind(0)

@@ -721,9 +721,10 @@ class _AttentionTrain(torch.autograd.Function):
 
 class _AttentionFlash(torch.autograd.Function):
     """Training attention as two tcgen05 kernels on the packed qkv tensor, differentiable in qkv and in the keep policy:
-    forward = the inference kernel, which also writes per-row softmax statistics (`d2s_attn_policy_fwd` with `stats`);
-    backward = `d2s_attn_policy_bwd`, which recomputes scores and probabilities on chip.  Saves qkv, the output and
-    (B,H,T,4) floats; no (B,H,T,T) tensor, no head-major copies, no library GEMM."""
+    forward = the inference kernel, which also writes per-row softmax statistics (`d2s_attn_policy_fwd` with `stats`, or for
+    T > FLASH_MAX_T the key-blocked `d2s_attn_long_fwd_stats`); backward = `d2s_attn_policy_bwd` (or the key-blocked
+    `d2s_attn_long_bwd` with a (B,H,T,64) fp32 dQ workspace), which recomputes scores and probabilities on chip.  Saves qkv,
+    the output and (B,H,T,4) floats; no (B,H,T,T) tensor, no head-major copies, no library GEMM."""
 
     @staticmethod
     def forward(ctx, qkv, policy, H, scale, eps, want_cls):
@@ -735,7 +736,11 @@ class _AttentionFlash(torch.autograd.Function):
         out = torch.empty(B, T, D, dtype=qkv.dtype, device=dev)
         cls_row = torch.empty(B, H, T, dtype=torch.float32, device=dev) if want_cls else None
         stats = torch.empty(B, H, T, 4, dtype=torch.float32, device=dev)
-        _call("d2s_attn_policy_fwd", _ptr(qkv), _ptr(pol), BF16, B, T, H, D // H, float(scale), float(eps), _ptr(out),
+        if T > FLASH_MAX_T:
+            _call("d2s_attn_long_fwd_stats", _ptr(qkv), _ptr(pol), B, T, H, D // H, float(scale), float(eps), _ptr(out),
+                  _ptr(cls_row), _ptr(stats), _stream(qkv))
+        else:
+            _call("d2s_attn_policy_fwd", _ptr(qkv), _ptr(pol), BF16, B, T, H, D // H, float(scale), float(eps), _ptr(out),
                   _ptr(cls_row), _ptr(stats), _stream(qkv))
         none = torch.empty(0, device=dev)
         ctx.save_for_backward(qkv, out, stats, pol if pol is not None else none, cls_row if want_cls else none)
@@ -751,8 +756,13 @@ class _AttentionFlash(torch.autograd.Function):
         gc = _f32c(g_cls) if (want_cls and g_cls is not None) else None
         dqkv = torch.empty_like(qkv)
         gpol = torch.zeros(B, T, dtype=torch.float32, device=qkv.device) if has_pol else None
-        _call("d2s_attn_policy_bwd", _ptr(qkv), _ptr(pol) if has_pol else None, _ptr(out), _ptr(g),
-                  _ptr(cls_row) if want_cls else None, _ptr(gc), _ptr(stats), B, T, H, hd, scale, _ptr(dqkv), _ptr(gpol), _stream(qkv))
+        args = (_ptr(qkv), _ptr(pol) if has_pol else None, _ptr(out), _ptr(g), _ptr(cls_row) if want_cls else None, _ptr(gc),
+                _ptr(stats), B, T, H, hd, scale, _ptr(dqkv), _ptr(gpol))
+        if T > FLASH_MAX_T:
+            ws = torch.empty(B, H, T, hd, dtype=torch.float32, device=qkv.device)
+            _call("d2s_attn_long_bwd", *args, _ptr(ws), _stream(qkv))
+        else:
+            _call("d2s_attn_policy_bwd", *args, _stream(qkv))
         if has_pol:
             gpol = gpol.reshape(pol_meta[0]).to(pol_meta[1])
         return dqkv, gpol, None, None, None, None
@@ -763,14 +773,20 @@ FLASH_MAX_T = 208
 
 def attention_train(qkv, num_heads, policy=None, scale=None, eps=1e-6, want_cls_row=False):
     """Differentiable attention core of Attention.forward (vit_models/dynamic_vit.py:216-231) on the packed qkv (B,T,3*H*hd):
-    returns (out (B,T,H*hd), cls_row (B,H,T) | None).  bf16 CUDA tensors, T <= 256.  hd == 64 and T <= 208 (every DeiT shape
-    at 224 px) run the tcgen05 flash kernels; the rest keeps the head-major GEMMs around the padded-row softmax kernels."""
+    returns (out (B,T,H*hd), cls_row (B,H,T) | None).  bf16 CUDA tensors, T <= 256, or hd == 64 and T <= LONG_ATTN_MAX_T.
+    hd == 64 and T <= 208 (every DeiT shape at 224 px) run the tcgen05 flash kernels, hd == 64 and T > 256 (384 / 512-px
+    inputs) their key-blocked forms (d2s_attn_long_fwd_stats, d2s_attn_long_bwd); the rest keeps the head-major GEMMs around
+    the padded-row softmax kernels."""
     _check_cuda(qkv, policy)
-    if qkv.dtype != torch.bfloat16 or qkv.shape[1] > 256:
-        raise RuntimeError("attention_train: bf16 and T <= 256 only (other cases use softmax_with_policy around torch matmuls)")
+    T = qkv.shape[1]
     hd = qkv.shape[-1] // 3 // num_heads
+    if qkv.dtype != torch.bfloat16 or (T > 256 and (hd != 64 or T > LONG_ATTN_MAX_T)):
+        raise RuntimeError(f"attention_train: bf16 with T <= 256, or bf16 with head dim 64 and T <= {LONG_ATTN_MAX_T}; got "
+                           f"{qkv.dtype}, T = {T}, head dim {hd} (other cases use softmax_with_policy around torch matmuls)")
     scale = hd ** -0.5 if scale is None else scale
-    if hd == 64 and qkv.shape[1] <= FLASH_MAX_T and scale > 0:
+    if T > 256 and not scale > 0:
+        raise ValueError(f"attention_train: scale must be positive beyond 256 tokens (got {scale})")
+    if hd == 64 and (T <= FLASH_MAX_T or T > 256) and scale > 0:
         return _AttentionFlash.apply(qkv, policy, num_heads, float(scale), float(eps), bool(want_cls_row))
     return _AttentionTrain.apply(qkv, policy, num_heads, float(scale), float(eps), bool(want_cls_row))
 

@@ -237,12 +237,20 @@ int d2s_attn_policy_fwd(const void* qkv, const float* policy, int dtype, int B, 
 /* d2s_attn_long_fwd: the same attention core (dynamic_vit.py:195-214 softmax_with_policy, :218-234 Attention.forward) for
  * sequences beyond 256 tokens (384 / 512-pixel inputs): bf16 only, hd == 64, 1 <= T <= 2048, key-blocked tcgen05/TMEM kernel
  * (128-row query tiles x 128-column key blocks, K / V streamed, no (B,H,T,T) tensor, no global scratch).
- * qkv (B,T,3,H,64), out (B,T,H*64), cls_row (B,H,T) f32 or NULL, as d2s_attn_policy_fwd; no row statistics.
+ * qkv (B,T,3,H,64), out (B,T,H*64), cls_row (B,H,T) f32 or NULL, as d2s_attn_policy_fwd; no row statistics (see
+ * d2s_attn_long_fwd_stats).
  * policy (B,T) f32 or NULL: the policy softmax of d2s_attn_policy_fwd (mask p_j off the diagonal, eps/T on every entry).
  * len (B) int32 or NULL: the variable-length form of d2s_attn_varlen_fwd (image b = its first len[b] tokens, out rows and
  * cls_row columns >= len[b] written as zeros); policy and len are never both given.  scale > 0; B == 0 is a no-op. */
 int d2s_attn_long_fwd(const void* qkv, const float* policy, const int* len, int B, int T, int H, int hd, float scale, float eps,
                       void* out, float* cls_row, d2s_stream_t stream);
+/* d2s_attn_long_fwd_stats: the training forward beyond 256 tokens -- d2s_attn_long_fwd without len (no variable-length form),
+ * which also writes stats (B,H,T,4) f32, 16-byte aligned, with the meaning of d2s_attn_policy_fwd's: per query row
+ * (m', 1/den, c/den, unused), P_ij = 2^(k2 s_ij - m') m_ij / den + c/den, for the m' and den that produced out (rows redone
+ * in fp32 and rows whose reference was raised by whole binades included).  out and cls_row are bit-identical to
+ * d2s_attn_long_fwd's.  bf16, hd == 64, 1 <= T <= 2048, policy (B,T) f32 or NULL, scale > 0; B == 0 is a no-op. */
+int d2s_attn_long_fwd_stats(const void* qkv, const float* policy, int B, int T, int H, int hd, float scale, float eps, void* out,
+                            float* cls_row, float* stats, d2s_stream_t stream);
 
 /* Backward of d2s_attn_policy_fwd (bf16, hd == 64, T <= 208): Attention.forward's core under autograd, differentiable in qkv AND
  * in the keep policy (dynamic_vit.py:195-214, :218-231; default_dynamic_vit.py:185-199, :203-213), flash style -- scores and
@@ -255,6 +263,16 @@ int d2s_attn_long_fwd(const void* qkv, const float* policy, const int* len, int 
 int d2s_attn_policy_bwd(const void* qkv, const float* policy, const void* out, const void* gout, const float* cls_row,
                         const float* g_cls, float* stats, int B, int T, int H, int hd, float scale, void* dqkv,
                         float* gpolicy, d2s_stream_t stream);
+/* d2s_attn_long_bwd: the backward of d2s_attn_long_fwd_stats (and of d2s_attn_policy_fwd with stats) for 1 <= T <= 2048, with
+ * the arguments and semantics of d2s_attn_policy_bwd: bf16, hd == 64, scale > 0, policy / gpolicy both NULL or both given,
+ * g_cls only with cls_row; B == 0 is a no-op.  Key-blocked tcgen05/TMEM kernel (128-key tiles x 128-query blocks, one
+ * (image, head) per CTA): no (B,H,T,T) tensor is read or written.
+ *   workspace: (B,H,T,64) f32 (B*H*T*64 floats), 16-byte aligned, caller-provided scratch for the dQ partial sums of the key
+ *   tiles (read only where written first; its contents on return are unspecified).
+ * dqkv is bitwise reproducible from run to run; gpolicy is accumulated across heads with fp32 atomics, as in d2s_attn_policy_bwd. */
+int d2s_attn_long_bwd(const void* qkv, const float* policy, const void* out, const void* gout, const float* cls_row,
+                      const float* g_cls, float* stats, int B, int T, int H, int hd, float scale, void* dqkv, float* gpolicy,
+                      float* workspace, d2s_stream_t stream);
 
 /* ---- predictor body (inference path of PredictorLG.forward, default_dynamic_vit.py:324-330; dynamic_vit.py:538-546)
  * d2s_pool_act: z (B,N,C) = in_conv's Linear output; local (B,N,C/2) = act(z[:,:,:C/2]);
