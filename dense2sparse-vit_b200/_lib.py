@@ -36,10 +36,6 @@ SIGNATURES = {
     "d2s_ptopk_bwd": [_p, _p, _i, _i, _i, _p, _p],
     "d2s_softmax_policy_fwd": [_p, _p, _i, _i, _i, _i, _f, _p, _p, _p],
     "d2s_softmax_policy_bwd": [_p, _p, _p, _p, _i, _i, _i, _i, _f, _p, _p, _p],
-    "d2s_softmax_policy_fwd_ld": [_p, _p, _i, _i, _i, _i, _i, _f, _p, _p, _p],
-    "d2s_softmax_policy_bwd_ld": [_p, _p, _p, _p, _i, _i, _i, _i, _i, _f, _p, _p, _p],
-    "d2s_split_heads_bf16": [_p, _i, _i, _i, _i, _i, _i, _p, _p],
-    "d2s_merge_heads_bf16": [_p, _i, _i, _i, _i, _i, _i, _p, _p],
     "d2s_colsum_bf16": [_p, ctypes.c_longlong, _i, _p, _p],
     "d2s_gelu_bwd_colsum_bf16": [_p, _p, ctypes.c_longlong, _i, _p, _p, _p],
     "d2s_colsum_acc_bf16": [_p, ctypes.c_longlong, _i, _p, _p],

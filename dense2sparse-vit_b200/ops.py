@@ -659,66 +659,6 @@ def linear_train(lin, x):
     return lin(x)
 
 
-class _AttentionTrain(torch.autograd.Function):
-    """Training attention on the packed qkv tensor, differentiable in qkv and in the keep policy.
-
-    One d2s relayout pass turns the packed (B,T,3,H,hd) tensor into head-major (3,B,H,Tp,hd) with Tp = round_up(T, 8) zero
-    padded, so that the six batched GEMMs of forward + backward run over B*H matrices whose every dimension and leading
-    dimension is a multiple of 8 (T = 197 otherwise sends cuBLAS to unaligned legacy kernels and torch to permute copies),
-    and the d2s policy-softmax kernels move 16-byte vectors.  dq/dk/dv are merged straight into the packed qkv gradient
-    (no cat).  Saves q/k/v head-major, the scaled scores, the probabilities and the (row max, denominator) pairs."""
-
-    @staticmethod
-    def forward(ctx, qkv, policy, H, scale, eps, want_cls):
-        qkv = qkv.contiguous()
-        B, T, C3 = qkv.shape
-        D = C3 // 3
-        hd = D // H
-        Tp = (T + 7) // 8 * 8
-        dev, dt = qkv.device, qkv.dtype
-        qkvh = torch.empty(3, B * H, Tp, hd, dtype=dt, device=dev)
-        _call("d2s_split_heads_bf16", _ptr(qkv), B, T, Tp, 3, H, hd, _ptr(qkvh), _stream(qkv))
-        S = torch.empty(B * H, Tp, Tp, dtype=dt, device=dev)
-        torch.baddbmm(S, qkvh[0], qkvh[1].transpose(1, 2), beta=0, alpha=scale, out=S)
-        pol = _f32c(policy.reshape(B, T)) if policy is not None else None
-        P = torch.empty_like(S)
-        stats = torch.empty(B, H, T, 2, dtype=torch.float32, device=dev)
-        _call("d2s_softmax_policy_fwd_ld", _ptr(S), _ptr(pol), B, H, T, Tp, Tp, float(eps), _ptr(P), _ptr(stats), _stream(S))
-        Oh = torch.bmm(P, qkvh[2])                                                    # (B*H, Tp, hd)
-        O = torch.empty(B, T, D, dtype=dt, device=dev)
-        _call("d2s_merge_heads_bf16", _ptr(Oh), B, T, Tp, 1, H, hd, _ptr(O), _stream(Oh))
-        cls_attn = P.view(B, H, Tp, Tp)[:, :, 0, :T].clone() if want_cls else None
-        ctx.save_for_backward(qkvh, S, P, stats, pol if pol is not None else torch.empty(0, device=dev))
-        ctx.meta = (B, T, Tp, H, hd, float(scale), float(eps), pol is not None,
-                    None if policy is None else (policy.shape, policy.dtype))
-        return O, cls_attn
-
-    @staticmethod
-    def backward(ctx, gO, g_cls):
-        qkvh, S, P, stats, pol = ctx.saved_tensors
-        B, T, Tp, H, hd, scale, eps, has_pol, pol_meta = ctx.meta
-        polp = pol if has_pol else None
-        dev, dt = S.device, S.dtype
-        g = gO.to(dt).contiguous()
-        gOh = torch.empty(B * H, Tp, hd, dtype=dt, device=dev)
-        _call("d2s_split_heads_bf16", _ptr(g), B, T, Tp, 1, H, hd, _ptr(gOh), _stream(g))
-        dqkvh = torch.empty(3, B * H, Tp, hd, dtype=dt, device=dev)
-        torch.bmm(P.transpose(1, 2), gOh, out=dqkvh[2])                               # dV = P^T dO
-        dP = torch.bmm(gOh, qkvh[2].transpose(1, 2))                                  # dP = dO V^T  (padding rows are zero)
-        if g_cls is not None:
-            dP.view(B, H, Tp, Tp)[:, :, 0, :T] += g_cls.to(dt)
-        gpol = torch.zeros(B, T, dtype=torch.float32, device=dev) if has_pol else None
-        _call("d2s_softmax_policy_bwd_ld", _ptr(S), _ptr(polp), _ptr(dP), _ptr(stats), B, H, T, Tp, Tp, eps, _ptr(dP),
-                  _ptr(gpol), _stream(S))
-        torch.baddbmm(dqkvh[0], dP, qkvh[1], beta=0, alpha=scale, out=dqkvh[0])                    # dQ = scale dS K
-        torch.baddbmm(dqkvh[1], dP.transpose(1, 2), qkvh[0], beta=0, alpha=scale, out=dqkvh[1])    # dK = scale dS^T Q
-        dqkv = torch.empty(B, T, 3 * H * hd, dtype=dt, device=dev)
-        _call("d2s_merge_heads_bf16", _ptr(dqkvh), B, T, Tp, 3, H, hd, _ptr(dqkv), _stream(dqkvh))
-        if has_pol:
-            gpol = gpol.reshape(pol_meta[0]).to(pol_meta[1])
-        return dqkv, gpol, None, None, None, None
-
-
 class _AttentionFlash(torch.autograd.Function):
     """Training attention as two tcgen05 kernels on the packed qkv tensor, differentiable in qkv and in the keep policy:
     forward = the inference kernel, which also writes per-row softmax statistics (`d2s_attn_policy_fwd` with `stats`, or for
@@ -768,27 +708,28 @@ class _AttentionFlash(torch.autograd.Function):
         return dqkv, gpol, None, None, None, None
 
 
-FLASH_MAX_T = 208
+FLASH_MAX_T = 208        # _AttentionFlash runs d2s_attn_policy_fwd / _bwd up to this T, the key-blocked pair above it
+
+
+def attention_train_ok(qkv, num_heads, scale=None):
+    """Inputs attention_train takes: bf16 packed qkv (B,T,3*H*64), 1 <= T <= LONG_ATTN_MAX_T, and a positive scale (`scale`, or
+    64^-0.5 when None).  Shapes and dtype only: the caller checks the device."""
+    return (qkv.dim() == 3 and qkv.dtype == torch.bfloat16 and qkv.shape[-1] == 3 * num_heads * 64
+            and 1 <= qkv.shape[1] <= LONG_ATTN_MAX_T and (scale is None or scale > 0))
 
 
 def attention_train(qkv, num_heads, policy=None, scale=None, eps=1e-6, want_cls_row=False):
-    """Differentiable attention core of Attention.forward (vit_models/dynamic_vit.py:216-231) on the packed qkv (B,T,3*H*hd):
-    returns (out (B,T,H*hd), cls_row (B,H,T) | None).  bf16 CUDA tensors, T <= 256, or hd == 64 and T <= LONG_ATTN_MAX_T.
-    hd == 64 and T <= 208 (every DeiT shape at 224 px) run the tcgen05 flash kernels, hd == 64 and T > 256 (384 / 512-px
-    inputs) their key-blocked forms (d2s_attn_long_fwd_stats, d2s_attn_long_bwd); the rest keeps the head-major GEMMs around
-    the padded-row softmax kernels."""
+    """Differentiable attention core of Attention.forward (vit_models/dynamic_vit.py:216-231) on the packed qkv (B,T,3*H*64):
+    returns (out (B,T,H*64), cls_row (B,H,T) | None), for the inputs attention_train_ok admits, on CUDA.  T <= FLASH_MAX_T
+    (every DeiT shape at 224 px) runs the tcgen05 flash kernels, longer sequences their key-blocked forms
+    (d2s_attn_long_fwd_stats, d2s_attn_long_bwd)."""
     _check_cuda(qkv, policy)
-    T = qkv.shape[1]
-    hd = qkv.shape[-1] // 3 // num_heads
-    if qkv.dtype != torch.bfloat16 or (T > 256 and (hd != 64 or T > LONG_ATTN_MAX_T)):
-        raise RuntimeError(f"attention_train: bf16 with T <= 256, or bf16 with head dim 64 and T <= {LONG_ATTN_MAX_T}; got "
-                           f"{qkv.dtype}, T = {T}, head dim {hd} (other cases use softmax_with_policy around torch matmuls)")
-    scale = hd ** -0.5 if scale is None else scale
-    if T > 256 and not scale > 0:
-        raise ValueError(f"attention_train: scale must be positive beyond 256 tokens (got {scale})")
-    if hd == 64 and (T <= FLASH_MAX_T or T > 256) and scale > 0:
-        return _AttentionFlash.apply(qkv, policy, num_heads, float(scale), float(eps), bool(want_cls_row))
-    return _AttentionTrain.apply(qkv, policy, num_heads, float(scale), float(eps), bool(want_cls_row))
+    if not attention_train_ok(qkv, num_heads, scale):
+        raise RuntimeError(f"attention_train: bf16 packed qkv with head dim 64, 1 <= T <= {LONG_ATTN_MAX_T} and a positive scale; "
+                           f"got {qkv.dtype} {tuple(qkv.shape)}, {num_heads} heads, scale {scale} (other cases use "
+                           "softmax_with_policy around torch matmuls)")
+    scale = 64 ** -0.5 if scale is None else scale
+    return _AttentionFlash.apply(qkv, policy, num_heads, float(scale), float(eps), bool(want_cls_row))
 
 
 def attention_core(qkv, num_heads, policy=None, scale=None, eps=1e-6, want_cls_row=False, lengths=None):

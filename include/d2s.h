@@ -173,23 +173,6 @@ int d2s_softmax_policy_bwd(const void* attn, const float* policy, const void* go
                            int dtype, int B, int H, int T, float eps,
                            void* gattn, float* gpolicy, d2s_stream_t stream);
 
-/* Padded-row variants used by the training attention (ops.attention_train): bf16 only, tensors are (B,H,T,ld) with
- * ld % 8 == 0, T <= ld <= 256, so every row is 16-byte aligned and moved with 16-byte accesses; padding columns of `out`
- * / `gattn` are written as zeros.  gattn may alias gout.  `rows` >= T is the row count of the buffers (rows T..rows-1 of
- * `out` are zero-filled by the forward so the padded tensor can be a GEMM operand; the backward leaves them untouched).
- * The backward omits the gradient through the subtracted row max (sum_j dS_ij = O(eps) * g ~ 1e-6 relative, below bf16
- * resolution; d2s_softmax_policy_bwd keeps it for the fp32 parity runs). */
-int d2s_softmax_policy_fwd_ld(const void* attn, const float* policy, int B, int H, int T, int rows, int ld, float eps,
-                              void* out, float* stats, d2s_stream_t stream);
-int d2s_softmax_policy_bwd_ld(const void* attn, const float* policy, const void* gout, const float* stats, int B, int H,
-                              int T, int rows, int ld, float eps, void* gattn, float* gpolicy, d2s_stream_t stream);
-
-/* Head-major relayout for the training attention (dynamic_vit.py:218-221), bf16: token-major packed (B,T,G,H,hd)
- * (G = 3: qkv Linear output; G = 1: attention output / its gradient) <-> head-major (G,B,H,Tp,hd), Tp >= T; split writes
- * the padding rows T..Tp-1 as zeros, merge drops them.  hd % 8 == 0. */
-int d2s_split_heads_bf16(const void* src, int B, int T, int Tp, int G, int H, int hd, void* dst, d2s_stream_t stream);
-int d2s_merge_heads_bf16(const void* src, int B, int T, int Tp, int G, int H, int hd, void* dst, d2s_stream_t stream);
-
 /* Column sums of a bf16 matrix in fp32: out[n] = sum_m dy[m, n] (out is overwritten): the bias gradient of an nn.Linear
  * under autograd (dynamic_vit.py:159-236).  N % 8 == 0, N <= 8192. */
 int d2s_colsum_bf16(const void* dy, long long M, int N, float* out, d2s_stream_t stream);

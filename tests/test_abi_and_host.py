@@ -56,7 +56,7 @@ def test_argument_errors_precede_any_launch(d2s):
     assert lib.d2s_attn_policy_fwd(p, None, 1, 1, 8, 2, 48, 0.1, 1e-6, p, None, None, None) == 1
     assert b"head dim" in lib.d2s_last_error()
     assert lib.d2s_softmax_policy_fwd(p, None, 0, 1, 1, 5000, 1e-6, p, None, None) == 1
-    # the tcgen05 GEMM family and the training-attention helpers: shape / alignment contracts
+    # the tcgen05 GEMM family: shape / alignment contracts
     assert lib.d2s_linear_residual_ln_bf16(p, p, p, p, p, p, 1e-6, 256, 576, 384, p, p, None) == 1 and b"N in {192, 384, 768}" in lib.d2s_last_error()
     assert lib.d2s_linear_residual_ln_bf16(p, p, p, p, None, None, 1e-6, 256, 384, 384, p, p, None) == 1 and b"gamma" in lib.d2s_last_error()
     assert lib.d2s_linear_residual_ln_bf16(p, p, p, p, p, p, 1e-6, 256, 384, 100, p, p, None) == 1 and b"K %" in lib.d2s_last_error()
@@ -66,14 +66,9 @@ def test_argument_errors_precede_any_launch(d2s):
     assert lib.d2s_mlp_residual_ln_bf16(p, p, p, p, p, p, p, p, 1e-6, 256, 384, 1000, 1, 0, p, p, None) == 1 and b"HID" in lib.d2s_last_error()
     assert lib.d2s_mlp_residual_ln_bf16(None, p, p, p, p, p, p, p, 1e-6, 256, 384, 1536, 1, 0, p, p, None) == 1 and b"null" in lib.d2s_last_error()
     assert lib.d2s_mlp_residual_ln_bf16(p, p, p, p, p, p, p, p, 1e-6, 256, 384, 1536, 197, 1, p, p, None) == 1 and b"norm_row0" in lib.d2s_last_error()
-    assert lib.d2s_softmax_policy_fwd_ld(p, None, 1, 1, 197, 200, 197, 1e-6, p, None, None) == 1 and b"ld" in lib.d2s_last_error()
-    assert lib.d2s_softmax_policy_bwd_ld(p, None, p, p, 1, 1, 300, 304, 304, 1e-6, p, None, None) == 1 and b"T=300" in lib.d2s_last_error()
-    assert lib.d2s_split_heads_bf16(p, 1, 197, 100, 3, 6, 64, p, None) == 1 and b"Tp=100" in lib.d2s_last_error()
-    assert lib.d2s_merge_heads_bf16(p, 1, 197, 200, 3, 6, 60, p, None) == 1 and b"hd=60" in lib.d2s_last_error()
     assert d2s._lib.launch_count() == before
     # empty batches are a no-op, not an error
     assert lib.d2s_mlp_residual_ln_bf16(p, p, p, p, p, p, p, p, 1e-6, 0, 384, 1536, 1, 0, p, p, None) == 0
-    assert lib.d2s_split_heads_bf16(p, 0, 197, 200, 3, 6, 64, p, None) == 0
     assert lib.d2s_assemble_layernorm(p, p, p, p, p, 1, 2, 196, 380, 1e-6, p, p, None) == 1 and b"D=380" in lib.d2s_last_error()
     assert lib.d2s_assemble_layernorm(p, None, p, p, p, 1, 2, 196, 384, 1e-6, p, p, None) == 1
     assert lib.d2s_colsum_bf16(p, 16, 12, p, None) == 1 and b"N=12" in lib.d2s_last_error()

@@ -4,6 +4,7 @@ formula, against the T <= 208 flash kernels where both run, at the edges of the 
 DeiT-S-width models at 384 and 512 pixels."""
 import copy
 import ctypes
+import types
 
 import pytest
 import torch
@@ -18,12 +19,13 @@ def _stream():
     return torch.cuda.current_stream().cuda_stream
 
 
-def _ref(qkv, H, policy=None, eps=1e-6, scale=0.125):
-    """Attention.forward's core (dynamic_vit.py:195-214 softmax_with_policy, :218-234) in float64, differentiable in qkv and
-    policy: (out (B,T,H*64), cls_row (B,H,T), probabilities (B,H,T,T))."""
-    B, T, _ = qkv.shape
-    q, k, v = qkv.view(B, T, 3, H, 64).permute(2, 0, 3, 1, 4).unbind(0)
-    s = (q @ k.transpose(-1, -2)) * scale
+def _ref(qkv, H, policy=None, eps=1e-6):
+    """Attention.forward's core (dynamic_vit.py:195-214 softmax_with_policy, :218-234) in float64 with scale hd^-0.5, differentiable
+    in qkv and policy: (out (B,T,H*hd), cls_row (B,H,T), probabilities (B,H,T,T))."""
+    B, T, C3 = qkv.shape
+    hd = C3 // 3 // H
+    q, k, v = qkv.view(B, T, 3, H, hd).permute(2, 0, 3, 1, 4).unbind(0)
+    s = (q @ k.transpose(-1, -2)) * hd ** -0.5
     if policy is None:
         p = torch.softmax(s, dim=-1)
     else:
@@ -32,7 +34,7 @@ def _ref(qkv, H, policy=None, eps=1e-6, scale=0.125):
         mask = pol + (1.0 - pol) * eye
         e = (s - s.amax(-1, keepdim=True)).exp() * mask
         p = (e + eps / T) / (e.sum(-1, keepdim=True) + eps)
-    return (p @ v).transpose(1, 2).reshape(B, T, H * 64), p[:, :, 0, :], p
+    return (p @ v).transpose(1, 2).reshape(B, T, H * hd), p[:, :, 0, :], p
 
 
 def _policy(B, T, g, kind):
@@ -119,23 +121,34 @@ def test_long_attention_training_argument_errors_precede_any_launch(d2s):
 
 
 def test_engine_routes_long_bf16_training_attention_behind_its_switch(d2s, monkeypatch):
-    """The training branch takes bf16 at T <= 256 (as before) and bf16, head dim 64, 256 < T <= 2048; _LONG_ATTN = False sends
-    everything above 256 tokens back to torch matmuls around the policy softmax."""
-    ok = d2s.engine._attn_train_kernel_ok
+    """The training branch takes bf16 with head dim 64 and 1 <= T <= 2048 (ops.attention_train_ok: the flash pair up to 208 tokens,
+    the key-blocked pair beyond); _LONG_ATTN = False sends everything above 208 tokens back to torch matmuls around the policy
+    softmax, as every other dtype, head dim and non-positive scale goes there."""
+    train_ok = d2s.ops.attention_train_ok
     bf = lambda T, hd=64: torch.empty(1, T, 3 * 6 * hd, dtype=torch.bfloat16)     # noqa: E731
-    assert ok(bf(577), 6) and ok(bf(2048), 6) and ok(bf(197), 6) and ok(bf(257), 6)
+    assert train_ok(bf(1), 6) and train_ok(bf(197), 6) and train_ok(bf(2048), 6) and train_ok(bf(197), 6, 0.125)
+    assert not train_ok(bf(2049), 6) and not train_ok(torch.empty(1, 0, 3 * 6 * 64, dtype=torch.bfloat16), 6)
+    assert not train_ok(bf(197, 48), 6) and not train_ok(bf(197, 32), 6) and not train_ok(bf(197), 4)
+    assert not train_ok(torch.empty(1, 197, 3 * 6 * 64, dtype=torch.float32), 6)
+    assert not train_ok(torch.empty(1, 197, 3 * 6 * 64, dtype=torch.float16), 6)
+    assert not train_ok(bf(197), 6, 0.0) and not train_ok(bf(577), 6, -0.125) and not train_ok(bf(197), 6, float("nan"))
+    ok = d2s.engine._attn_train_kernel_ok
+    assert ok(bf(577), 6) and ok(bf(2048), 6) and ok(bf(197), 6) and ok(bf(208), 6) and ok(bf(209), 6) and ok(bf(256), 6)
+    assert ok(bf(257), 6) and ok(bf(197), 6, 0.125)
     assert not ok(bf(2049), 6)
     assert not ok(torch.empty(1, 577, 3 * 6 * 64, dtype=torch.float32), 6)
     assert not ok(torch.empty(1, 197, 3 * 6 * 64, dtype=torch.float32), 6)
     assert not ok(bf(577, 48), 6)
-    assert ok(bf(197, 48), 6)                                                        # T <= 256 keeps its head-major GEMM path
+    assert not ok(bf(197, 48), 6)                                                    # head dim 48 goes to torch
+    assert not ok(bf(197), 6, 0.0) and not ok(bf(577), 6, -0.125)                    # so does a non-positive scale
     monkeypatch.setattr(d2s.engine, "_LONG_ATTN", False)
-    assert not ok(bf(577), 6) and not ok(bf(257), 6) and ok(bf(256), 6) and ok(bf(197), 6)
+    assert not ok(bf(577), 6) and not ok(bf(257), 6) and not ok(bf(256), 6) and not ok(bf(209), 6)
+    assert ok(bf(208), 6) and ok(bf(197), 6)
 
 
 # ----------------------------------------------------------------------------------------------------------------- kernels
 @pytest.mark.gpu
-@pytest.mark.parametrize("T", [257, 577, 1025])
+@pytest.mark.parametrize("T", [209, 256, 257, 577, 1025])
 @pytest.mark.parametrize("with_policy", [False, True])
 def test_long_row_statistics(d2s, cuda_dev, T, with_policy):
     """stats of d2s_attn_long_fwd_stats reproduce the float64 probabilities through P = 2^(k2 s - m') m / den + c / den, and out /
@@ -178,16 +191,20 @@ def _check_stats(lib, qkv, H, pol):
     torch.testing.assert_close(e * st[..., 1:2] + st[..., 2:3], ref, rtol=2e-4, atol=1e-7)
 
 
-def _train_vs_f64(d2s, qkv, H, pol, seed):
-    """ops.attention_train forward + backward (a loss on out and on the CLS rows) against float64 autograd of the reference formula
-    on the same bf16 inputs, at the bounds of test_gpu_parity.py::test_attention_train_fwd_bwd_vs_oracle_autograd."""
-    B, T, _ = qkv.shape
+def _train_vs_f64(d2s, qkv, H, pol, seed, attend=None, dpol_tol=1e-3):
+    """attend(qkv, H, policy) -> (out, cls_row), ops.attention_train by default: forward + backward (a loss on out and on the CLS
+    rows) against float64 autograd of the reference formula on the same bf16 inputs, at the bounds of
+    test_gpu_parity.py::test_attention_train_fwd_bwd_vs_oracle_autograd."""
+    B, T, C3 = qkv.shape
     g = torch.Generator(device="cuda").manual_seed(seed)
-    go = (torch.randn(B, T, H * 64, device="cuda", generator=g) * 0.5).bfloat16()
+    go = (torch.randn(B, T, C3 // 3, device="cuda", generator=g) * 0.5).bfloat16()
     gc = torch.randn(B, H, T, device="cuda", generator=g) * 0.5
     q1 = qkv.clone().requires_grad_(True)
     p1 = pol.clone().requires_grad_(True) if pol is not None else None
-    o1, c1 = d2s.ops.attention_train(q1, H, policy=p1, want_cls_row=True)
+    if attend is None:
+        o1, c1 = d2s.ops.attention_train(q1, H, policy=p1, want_cls_row=True)
+    else:
+        o1, c1 = attend(q1, H, p1)
     (o1.float() * go.float()).sum().add((c1.float() * gc).sum()).backward()
     q2 = qkv.double().requires_grad_(True)
     p2 = pol.double().requires_grad_(True) if pol is not None else None
@@ -201,11 +218,11 @@ def _train_vs_f64(d2s, qkv, H, pol, seed):
     if pol is not None:
         gp1, gp2 = p1.grad.double(), p2.grad
         assert bool(torch.isfinite(gp1).all())
-        assert float((gp1 - gp2).abs().max()) <= 1e-3 * float(gp2.abs().max()) + 1e-5
+        assert float((gp1 - gp2).abs().max()) <= dpol_tol * float(gp2.abs().max()) + 1e-5
 
 
 @pytest.mark.gpu
-@pytest.mark.parametrize("T", [257, 300, 577, 785, 1025, 2048])
+@pytest.mark.parametrize("T", [209, 256, 257, 300, 577, 785, 1025, 2048])
 @pytest.mark.parametrize("H", [6, 12])
 @pytest.mark.parametrize("pol_kind", ["none", "binary", "fraction"])
 def test_long_attention_train_matches_float64_autograd(d2s, cuda_dev, T, H, pol_kind):
@@ -215,6 +232,25 @@ def test_long_attention_train_matches_float64_autograd(d2s, cuda_dev, T, H, pol_
     n0 = d2s._lib.launch_count()
     _train_vs_f64(d2s, qkv, H, _policy(B, T, g, pol_kind), 6100 + T)
     assert d2s._lib.launch_count() > n0
+
+
+@pytest.mark.gpu
+@pytest.mark.parametrize("hd", [32, 48])
+def test_bf16_training_at_other_head_dims_runs_the_torch_branch(d2s, cuda_dev, monkeypatch, hd):
+    """bf16 training at a head dim the tcgen05 pairs do not take goes through engine.attention_pre_proj's torch branch (matmuls around
+    ops.softmax_with_policy), never ops.attention_train, and matches float64 autograd of the reference formula.  The stand-in
+    module's qkv projection returns the packed tensor under test, so its gradient is observed directly; x carries the shape only
+    (fp32, so no qkv GEMM takes it).  d policy is held to 3e-2: this branch rounds the scores, the probabilities and dP to bf16."""
+    B, T, H = 2, 197, 6
+    g = torch.Generator(device="cuda").manual_seed(6500 + hd)
+    qkv = (torch.randn(B, T, 3 * H * hd, device="cuda", generator=g) * 0.7).bfloat16()
+    x = torch.empty(B, T, H * hd, device="cuda")
+    monkeypatch.setattr(d2s.ops, "attention_train", lambda *a, **k: pytest.fail("head dim %d reached ops.attention_train" % hd))
+
+    def attend(q, H, policy):
+        m = types.SimpleNamespace(num_heads=H, scale=hd ** -0.5, qkv=lambda _: q)
+        return d2s.engine.attention_pre_proj(m, x, policy=policy, return_cls_attn=True)
+    _train_vs_f64(d2s, qkv, H, _policy(B, T, g, "fraction"), 6600 + hd, attend=attend, dpol_tol=3e-2)
 
 
 @pytest.mark.gpu
@@ -299,7 +335,7 @@ class _Guarded:
 
 
 @pytest.mark.gpu
-@pytest.mark.parametrize("T", [257, 300, 577, 1025])
+@pytest.mark.parametrize("T", [226, 257, 300, 577, 1025])
 @pytest.mark.parametrize("H,pol", [(1, True), (6, False), (6, True)])
 def test_long_attention_train_stays_in_bounds(d2s, cuda_dev, T, H, pol):
     """Odd B, T with a nearly empty last tile: no write outside any output or the workspace, NaN behind every input never reaches a
